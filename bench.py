@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — AutoInt train samples/s on synthetic Criteo-shape batches (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype f32|bf16] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype f32|bf16] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): AutoInt (InteractingLayer layer_num=3, unit 16, 2 heads)
 + DNN tower 624->256->128, 39 fields, 1M-row fp32 tables (d=16), batch 8192 per GPU,
@@ -16,6 +16,9 @@ with the largest share of the step; `kernels` lists every phase with its algorit
 bytes/FLOPs.  `cpu_baseline` / `--impl reference`: the op-for-op torch-CPU restatement of the
 reference TF graph (oracle/oracle_torch.py — TensorFlow is not installable offline) on the
 box's host cores.
+
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (see timed_outputs), so that two
+builds can be compared output for output: the inputs depend on the arguments alone (seeded on the device).
 """
 from __future__ import annotations
 
@@ -323,6 +326,24 @@ def _finish(world, dist):
         os._exit(0)
 
 
+DUMP_MAX_ROWS = 1 << 19      # 32 MiB of fp32 table rows: a dump stays under 64 MB
+
+
+def timed_outputs(tr):
+    """What the trainer's last step computed, as float32 / float64 host arrays: the loss, the clipped predictions,
+    every dense parameter after the update, and the embedding rows the step updated (`table_rows`: arena row indices,
+    this rank's own rows when sharded; `table`: their values), a fixed seeded sample if there are more than
+    DUMP_MAX_ROWS of them.  Collective when sharded: every rank calls it."""
+    import torch
+    rows = tr._touched_rows()
+    if rows.numel() > DUMP_MAX_ROWS:
+        g = torch.Generator(device=rows.device).manual_seed(SEED)
+        rows = rows[torch.randperm(rows.numel(), device=rows.device, generator=g)[:DUMP_MAX_ROWS]].sort().values
+    out = {"loss": tr.loss, "pred": tr.p_raw.float().clamp(1e-6, 1.0), "table_rows": rows.double(), "table": tr.table[rows]}
+    out.update({f"dense_{k}": v for k, v in tr.P.items()})
+    return {k: (v if v.dtype == torch.float64 else v.float()).cpu().numpy() for k, v in out.items()}
+
+
 def run_own(args):
     import numpy as np
     import torch
@@ -395,6 +416,8 @@ def run_own(args):
     ms = e0.elapsed_time(e1)
     clk = clocks.stop() if rank == 0 else None
     loss_dev = float(tr.loss.item())
+    # taken now: the end-to-end loop below trains the same trainer further
+    dump = timed_outputs(tr) if args.dump_outputs else None
 
     # ---- end to end: pinned host inputs, H2D + step + loss D2H every step
     ids_host = ids_dev.cpu().pin_memory()
@@ -573,6 +596,10 @@ def run_own(args):
         "clocks": clk, "roofline": roof, "embed_roofline": embed, "kernels": kernels,
         "cpu_baseline": cpu, "loss": loss_dev, "loss_e2e_last": last, "other_configs": other,
     }
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     print(json.dumps(out), flush=True)
     _finish(world, dist)
 
@@ -591,7 +618,13 @@ def main():
                          "(headline, default), cfg3 = DIN, cfg4 = multi_head AUTOINT 200 M rows / 8 GPUs, cfg5 = VideoDnn")
     ap.add_argument("--ids", default="uniform", choices=["uniform", "zipf"],
                     help="id distribution of the synthetic batches (headline: uniform; zipf = skewed secondary workload)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (headline workload only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "own" or args.config != "cfg2"):
+        ap.error("--dump-outputs needs the headline workload (--impl own, --config cfg2)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
