@@ -33,7 +33,8 @@ extern "C" {
 
 #define RS_ABI_VERSION 5   /* 4: + rs_interacting_path; saved buffer grows by the per-head softmax statistics.
                               5: + deferred parameter-gradient reductions (rs_logit_head_reduce, rs_interacting_bwd_reduce),
-                                 rs_peer_all_to_all_i32, rs_embed_keys_from_rows */
+                                 rs_peer_all_to_all_i32, rs_embed_keys_from_rows;
+                                 + rs_idmap_insert / _lookup / _rebuild (additions only, same version) */
 
 enum rs_dtype { RS_F32 = 0, RS_BF16 = 1 };
 
@@ -276,6 +277,53 @@ int rs_route_ids_padded_spread(const int64_t* ids, int64_t n, int F, const int64
  * its adjoint out[index[i], :] = src[i, :] (index < 0 skipped). */
 int rs_permute_rows(const void* src, void* out, const int32_t* index, int64_t n,
                     int d, int dtype, int scatter, void* stream);
+
+/* ------------------------------------------ K9 collision-free id map ----
+ * Replaces TensorNet's per-shard sign -> row hash tables, which the reference
+ * reaches through tn.feature_column.category_column + tn.layers.EmbeddingFeatures
+ * (rank/ctr/base_model.py:203-217, staytime/VideoDnn.py:217-244,
+ * rough_rank/model.py:89-115): every distinct (field, id) gets its own arena row
+ * the first time a training step sees it, instead of row_base + id mod rows.
+ *
+ * Map of `n_fields` fields (field f: capacity R_f rows starting at arena row
+ * row_base_f):
+ *   slots       16-byte {int64 key; int32 row; int32 pad} slots, field f owns
+ *               S_f = next_pow2(2 R_f) of them from slot_base_f; key -1 = empty,
+ *               row -1 = the key got no row (its field was full).  16-B aligned.
+ *   key_of_row  int64[total rows]: the id that owns each arena row (-1 = unused).
+ *   counters    int64[2][n_fields]: rows used per field, then overflowed lookups.
+ *   geom        int64[n_fields][4] = {row_base_f, R_f, slot_base_f, S_f - 1}, 16-B aligned.
+ * Lookup i reads ids[i] of field field_of_col[i % F] (int32[F]); ids < 0 are padding.
+ * The slot of an id is splitmix64(id) & (S_f - 1), probed linearly (at most S_f
+ * probes; no thread ever waits for another).
+ *
+ * rs_idmap_insert gives every new key a row (row_base_f + the counter's next value)
+ * and writes that row's whole optimizer record: w[0:d] (row stride w_ld) from the
+ * init rule below, s0 / s1 (nullable; s_width floats at row stride s_ld) set to
+ * s*_init.  Once R_f rows are used, new keys of the field get no row.
+ * Init rule: pair p = k/2 of w draws r = mix64(base + G (p+1)), base =
+ * mix64(mix64(seed + G (f+1)) ^ id), G = 0x9E3779B97F4A7C15; u1 = ((r >> 40) + 1) 2^-24,
+ * u2 = ((r mod 2^32) >> 8) 2^-24; w[2p] = scale (sqrt(-2 ln u1) cos(2 pi u2)),
+ * w[2p+1] = scale (sqrt(-2 ln u1) sin(2 pi u2)) in fp32 (logf, sincospif).
+ * A row's initial value depends on (seed, field, id) only.
+ *
+ * rs_idmap_lookup writes rows_out[i] (int64 arena row, -1 for padding, unseen or
+ * overflowed keys).  after_insert = 1 (the call follows rs_idmap_insert on the same
+ * ids): lookups of keys without a row are counted in counters[1][f], and the row
+ * counters are clamped to R_f.  after_insert = 0 (inference): the map is not changed.
+ *
+ * rs_idmap_rebuild clears all `n_slots` slots (cudaMemsetAsync) and re-inserts
+ * key_of_row[row_base_f + j] for j < counters[0][f] with its row; key_of_row past
+ * the counters is set to -1.  Used to restore a map from a checkpoint or to roll it
+ * back to earlier counters.  max_rows = max R_f. */
+int rs_idmap_insert(void* slots, int64_t* key_of_row, int64_t* counters, const int64_t* geom, int n_fields,
+                    const int64_t* ids, int64_t n, int F, const int32_t* field_of_col, uint64_t seed, float scale,
+                    float* w, int64_t w_ld, int d, float* s0, int64_t s0_ld, int s0_width, float s0_init,
+                    float* s1, int64_t s1_ld, int s1_width, float s1_init, void* stream);
+int rs_idmap_lookup(const void* slots, int64_t* counters, const int64_t* geom, int n_fields, const int64_t* ids,
+                    int64_t n, int F, const int32_t* field_of_col, int64_t* rows_out, int after_insert, void* stream);
+int rs_idmap_rebuild(void* slots, int64_t n_slots, int64_t* key_of_row, const int64_t* counters, const int64_t* geom,
+                     int n_fields, int64_t max_rows, void* stream);
 
 /* ------------------------------------------------- K4 InteractingLayer ----
  * InteractingLayer.call (InteractingLayer.py:37-61; duplicate at

@@ -217,16 +217,19 @@ def create_autoint_sub_model(slot_zip_user_embs, dense_inputs_map, deep_hidden_u
 
 
 def AUTOINT(linear_features, dense_features, training, dnn_hidden_units=(32, 16), *, bucket_size=100_000,
-            device="cuda:0", seed=0, embedding_cls=None, group=None):
+            device="cuda:0", seed=0, embedding_cls=None, group=None, id_map="mod"):
     """AUTOINT(linear_features, dense_features, training, dnn_hidden_units=(32,16)) -> ModelResult{model, sub_model,
     model_predict} — rank/multi_head/multidnn.py:214-259.  8-d embeddings (combiner mean, tn.core.Adam lr 5e-5,
     :222,235) of the sorted, de-duplicated slots (:215-218) feed create_autoint_sub_model in `linear_features` order
     (:239).  Keyword-only extras stand in for the missing `src.*` Config: bucket_size (rows per slot table), device,
-    seed; embedding_cls / group select the row-sharded multi-GPU embedding (api.sharded_embedding)."""
+    seed; embedding_cls / group select the row-sharded multi-GPU embedding (api.sharded_embedding); id_map="hash" gives
+    every distinct slot id its own row (api.embedding.EmbeddingFeatures)."""
     features = sorted(set(linear_features))                                   # :215-218
     cols = [embedding_column(category_column(s, bucket_size), dimension=8, combiner="mean") for s in features]
     E = embedding_cls or EmbeddingFeatures
     kw = {"group": group} if embedding_cls is not None else {}      # None = the default process group
+    if id_map != "mod":
+        kw["id_map"] = id_map
     emb = E(cols, Adam(5e-5, 0.9, 0.999, 1e-8), "linear", device=device, seed=seed, **kw)
     sub_model = create_autoint_sub_model([(s, None) for s in linear_features], {k: None for k in dense_features},
                                          dnn_hidden_units, training, device=device)

@@ -5,7 +5,11 @@
 TensorNet itself is not vendored by the reference: table storage, the `bucket_size` semantics (ids
 are reduced mod bucket_size here) and the exact update rules are this repo's documented choices
 (SURVEY.md §8c, DESIGN.md).  All tables of one EmbeddingFeatures layer live in ONE fp32 arena so a
-batch is served by a single gather launch and a single sorted-segment update launch."""
+batch is served by a single gather launch and a single sorted-segment update launch.
+
+`id_map="hash"` replaces the modulo rule by a collision-free map (recommendsystem_b200.idmap): every distinct
+(column, id) gets its own row of the column's `bucket_size` rows, as TensorNet's hash tables give every feature sign
+its own row."""
 from __future__ import annotations
 
 from dataclasses import dataclass
@@ -15,6 +19,7 @@ import numpy as np
 import torch
 
 from .. import cabi, ops
+from ..idmap import IdMap, check_id_map
 
 
 @dataclass
@@ -67,10 +72,17 @@ class EmbeddingFeatures:
     ([B, T, d], mask [B, T]) for `combiner=None, seq_max_len=T` sequence columns.
 
     `backward(grads)` applies the fused sorted-segment sparse optimizer to the rows the last
-    forward touched (the reference's server-side push); `grads` maps column key -> d(loss)/d(output)."""
+    forward touched (the reference's server-side push); `grads` maps column key -> d(loss)/d(output).
+
+    id_map="mod" (default): row = row_base[column] + id mod bucket_size.  id_map="hash": `bucket_size` is the
+    column's row capacity and each distinct id gets its own row the first time a call with gradients enabled
+    (training) sees it, initialised N(0, scale) as a function of (seed, column, id); calls under torch.no_grad()
+    (the nets' predict) give unseen ids zero vectors and change nothing.  Once a column's rows are used up, new ids
+    read as zero vectors and get no update, like padding (`idmap.stats()` counts them)."""
 
     def __init__(self, embedding_columns: List[EmbeddingColumn], sparse_opt, name="embedding", device="cuda:0",
-                 out_dtype=torch.float32, seed=0):
+                 out_dtype=torch.float32, seed=0, id_map="mod"):
+        self.id_map = check_id_map(id_map)
         self.cols = list(embedding_columns)
         self.opt = sparse_opt
         self.dev = torch.device(device)
@@ -84,6 +96,7 @@ class EmbeddingFeatures:
         self.rows = rows
         if not isinstance(sparse_opt, (Adam, AdaGrad)):
             raise TypeError("sparse_opt must be api.embedding.Adam or AdaGrad")
+        self.idmap = None
         total = self._alloc_tables(seed)
         self.row_bits = ops.row_bits(total)
         self._last = None
@@ -111,6 +124,11 @@ class EmbeddingFeatures:
         of rows the sort keys must address."""
         total = int(self.rows.sum())
         self._alloc_state(total)
+        if self.id_map == "hash":                       # rows are initialised when their id is first inserted
+            states = [(self.m, 0.0), (self.v, 0.0)] if isinstance(self.opt, Adam) else \
+                [(self.g2sum, float(self.opt.initial_g2sum))]
+            self.idmap = IdMap(self.rows, self.dev, seed, self._init_scale(), self.table, states)
+            return total
         gen = torch.Generator(device=self.dev).manual_seed(seed)
         chunk = 1 << 22
         for r0 in range(0, total, chunk):
@@ -128,7 +146,7 @@ class EmbeddingFeatures:
         if len(single) > 1:
             ids = torch.stack([inputs[self.cols[ci].categorical_column.key].reshape(-1) for ci in single], dim=1)
             ids = ids.to(self.dev, torch.int64).contiguous()
-            base, rows = self._geom(tuple(single))
+            ids, base, rows = self._lookup(ids, tuple(single))
             emb, keys, _ = ops.embed_gather(self.table, ids, base, rows, torch.float32, want_keys=True)
             for j, ci in enumerate(single):
                 out[self.cols[ci].key] = emb[:, j, :].to(self.out_dtype)
@@ -142,13 +160,12 @@ class EmbeddingFeatures:
             if ci in single:
                 continue
             raw = inputs[c.categorical_column.key]
-            base, rows = self._geom((ci,))
             if isinstance(raw, (tuple, list)):
                 # variable-length bag in CSR form (values int64 [nnz], offsets int64 [B+1]): the VarLenFeature /
                 # SparseTensor input of the reference (staytime/parse.py:22-23), combiner='mean' (VideoDnn.py:224-226)
                 if c.combiner is None:
                     raise ValueError("CSR (values, offsets) inputs are for combiner='mean' columns")
-                vals = raw[0].to(self.dev, torch.int64).contiguous()
+                vals, base, rows = self._lookup(raw[0].to(self.dev, torch.int64).contiguous(), (ci,))
                 offs = raw[1].to(self.dev, torch.int64).contiguous()
                 nb = offs.numel() - 1
                 emb = torch.empty(nb, self.d, dtype=torch.float32, device=self.dev)
@@ -164,7 +181,8 @@ class EmbeddingFeatures:
             if c.combiner is None:                               # sequence column -> ([B,T,d], mask)
                 T = c.seq_max_len or ids.shape[1]
                 seq = ids[:, :T].contiguous()
-                emb, keys, arows = ops.embed_gather(self.table, seq.reshape(-1, 1), base, rows, self.out_dtype,
+                lk, base, rows = self._lookup(seq.reshape(-1, 1), (ci,))
+                emb, keys, arows = ops.embed_gather(self.table, lk, base, rows, self.out_dtype,
                                                     want_keys=True, want_rows=True)
                 out[c.key] = (emb.view(seq.shape[0], T, self.d), (arows.view(seq.shape[0], T) >= 0))
                 plan.append((c.key, keys, 1.0, None))
@@ -172,7 +190,8 @@ class EmbeddingFeatures:
                 if ids.dim() == 1:
                     ids = ids[:, None]
                 B, bag = ids.shape
-                emb, keys, arows = ops.embed_gather(self.table, ids.reshape(-1, 1).contiguous(), base, rows,
+                lk, base, rows = self._lookup(ids.reshape(-1, 1).contiguous(), (ci,))
+                emb, keys, arows = ops.embed_gather(self.table, lk, base, rows,
                                                     torch.float32, want_keys=True, want_rows=True)
                 if bag == 1:
                     out[c.key] = emb.view(B, self.d).to(self.out_dtype)
@@ -187,8 +206,9 @@ class EmbeddingFeatures:
 
     # ---- state one train step changes (GraphedTrainStep undoes its warm-up steps with these) -----------
     def touched_rows(self, inputs: Dict[str, torch.Tensor]) -> torch.Tensor:
-        """Sorted unique arena rows a step on `inputs` reads and updates."""
-        rows = []
+        """Sorted unique arena rows a step on `inputs` reads and updates (hash mode: the rows of the ids already
+        mapped, and every row the step's inserts may hand out)."""
+        rows, lookups = [], []
         for ci, c in enumerate(self.cols):
             ids = inputs[c.categorical_column.key]
             if isinstance(ids, (tuple, list)):                   # CSR bag: (values, offsets)
@@ -197,14 +217,25 @@ class EmbeddingFeatures:
             if c.combiner is None and c.seq_max_len:
                 ids = inputs[c.categorical_column.key].to(self.dev, torch.int64)[:, :c.seq_max_len].reshape(-1)
             ids = ids[ids >= 0]
+            if self.idmap is not None:
+                r = self.idmap.resolve(ids.reshape(-1, 1).contiguous(), self.idmap.fields((ci,)), insert=False)
+                rows.append(r[r >= 0].reshape(-1))
+                lookups.append(ids.numel())
+                continue
             rows.append(int(self.base[ci]) + torch.remainder(ids, int(self.rows[ci])))
+        if self.idmap is not None:
+            rows.append(self.idmap.pending_rows(lookups))
         return torch.unique(torch.cat(rows)) if rows else torch.empty(0, dtype=torch.int64, device=self.dev)
 
     def snapshot(self, inputs):
         rows = self.touched_rows(inputs)
         if isinstance(self.opt, Adam):
-            return {"rows": rows, "arena": self.arena[rows].clone(), "scalars": self.scalars.clone()}
-        return {"rows": rows, "table": self.table[rows].clone(), "g2sum": self.g2sum[rows].clone()}
+            snap = {"rows": rows, "arena": self.arena[rows].clone(), "scalars": self.scalars.clone()}
+        else:
+            snap = {"rows": rows, "table": self.table[rows].clone(), "g2sum": self.g2sum[rows].clone()}
+        if self.idmap is not None:
+            snap["idmap"] = self.idmap.snapshot()
+        return snap
 
     def restore(self, snap):
         rows = snap["rows"]
@@ -214,6 +245,22 @@ class EmbeddingFeatures:
         else:
             self.table[rows] = snap["table"]
             self.g2sum[rows] = snap["g2sum"]
+        if "idmap" in snap:
+            self.idmap.restore(snap["idmap"])
+
+    def _lookup(self, ids, cols):
+        """(ids, row_base, rows) the gather kernels read for the columns `cols`: the raw ids with the modulo geometry,
+        or (hash mode) the mapped arena rows with an identity geometry (row_base 0, rows = arena rows)."""
+        if self.idmap is None:
+            return (ids, *self._geom(cols))
+        mapped = self.idmap.resolve(ids, self.idmap.fields(cols), insert=torch.is_grad_enabled())
+        key = ("identity", len(cols))
+        g = self._geom_cache.get(key)
+        if g is None:
+            g = (torch.zeros(len(cols), dtype=torch.int64, device=self.dev),
+                 torch.full((len(cols),), self.idmap.total_rows, dtype=torch.int64, device=self.dev))
+            self._geom_cache[key] = g
+        return (mapped, *g)
 
     def _geom(self, cols):
         """(row_base, rows) device tensors of a column group, created once (no host->device copy per call:

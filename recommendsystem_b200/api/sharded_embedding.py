@@ -41,7 +41,9 @@ class _Group:
 
 class ShardedEmbeddingFeatures(EmbeddingFeatures):
     def __init__(self, embedding_columns: List[EmbeddingColumn], sparse_opt, name="embedding", device="cuda:0",
-                 out_dtype=torch.float32, seed=0, group=None, capacity_factor=None):
+                 out_dtype=torch.float32, seed=0, group=None, capacity_factor=None, id_map="mod"):
+        if id_map != "mod":
+            raise NotImplementedError("ShardedEmbeddingFeatures supports id_map='mod' only (row-sharded id maps are not built)")
         if not dist.is_initialized():
             raise RuntimeError("ShardedEmbeddingFeatures needs torch.distributed (one process per GPU)")
         self.group = group

@@ -23,6 +23,7 @@ import numpy as np
 import torch
 
 from . import cabi, ops
+from .idmap import IdMap, check_id_map
 
 
 class PhaseTimer:
@@ -88,6 +89,9 @@ class AutoIntConfig:
     # bf16 / tcgen05 mode: the embedding lookup runs inside the InteractingLayer forward's tile loader and the
     # embedding-gradient push (multi-GPU) inside its backward's epilogue; False = separate gather / scatter kernels
     fuse_embedding: bool = True
+    # "mod": row = row_base[f] + id mod rows_per_field[f].  "hash": every distinct (field, id) gets its own row of the
+    # field's rows_per_field (a capacity) the first time a train step sees it (recommendsystem_b200.idmap)
+    id_map: str = "mod"
 
     def rows(self) -> List[int]:
         if isinstance(self.rows_per_field, int):
@@ -107,6 +111,8 @@ class AutoIntTrainer:
         if self.dev.type != "cuda":
             raise RuntimeError("AutoIntTrainer runs on a CUDA device only (no CPU fallback)")
         self.act_dtype = {"f32": torch.float32, "bf16": torch.bfloat16}[cfg.dtype]
+        if check_id_map(cfg.id_map) == "hash" and tables is not None:
+            raise ValueError("tables= initialises rows by position; with id_map='hash' rows are initialised per id")
         F, d, U, B = cfg.num_fields, cfg.embed_dim, cfg.unit_num, cfg.batch
         if cfg.layer_num > 1 and d != U:
             raise ValueError("layer_num > 1 needs embed_dim == unit_num (InteractingLayer.py:41-46)")
@@ -118,6 +124,7 @@ class AutoIntTrainer:
             raise ValueError("arena rows must fit int32")
         self.rows_t = torch.from_numpy(self.rows_host).to(self.dev)
         self.base_t = torch.from_numpy(self.base_host).to(self.dev)
+        self.idmap = None
         self._alloc_tables(tables)
 
         # ---- dense parameters: one flat fp32 buffer (+ grads, m, v, bf16 shadow) with views
@@ -147,6 +154,13 @@ class AutoIntTrainer:
         T = self.act_dtype
         e = lambda *shape, dtype=T: torch.empty(*shape, device=self.dev, dtype=dtype)
         self.ids = torch.zeros(B, F, dtype=torch.int64, device=self.dev)
+        if self.idmap is not None:
+            # hash mode: the step's first two launches map ids -> arena rows (static buffer), and every gather reads
+            # those rows through an identity geometry (row_base 0, rows = total rows: id mod rows = id)
+            self.ids_rows = torch.full((B, F), -1, dtype=torch.int64, device=self.dev)
+            self.id_fields = self.idmap.fields(range(F))
+            self.id_base_t = torch.zeros(F, dtype=torch.int64, device=self.dev)
+            self.id_rows_t = torch.full((F,), self.total_rows, dtype=torch.int64, device=self.dev)
         self.labels = torch.zeros(B, 1, device=self.dev)
         self.X = e(B, F, d)
         self.keys = torch.empty(B * F, dtype=torch.int64, device=self.dev)
@@ -190,7 +204,10 @@ class AutoIntTrainer:
         cfg, d = self.cfg, self.cfg.embed_dim
         gen = torch.Generator(device=self.dev).manual_seed(cfg.seed)
         self._alloc_arena(self.total_rows, d)
-        if tables is None:
+        if cfg.id_map == "hash":                         # a row is initialised when its id is first inserted
+            self.idmap = IdMap(self.rows_host, self.dev, cfg.seed, cfg.table_init_scale, self.table,
+                               [(self.table_m, 0.0), (self.table_v, 0.0)])
+        elif tables is None:
             chunk = 1 << 22                              # initialise through bounded temporaries
             for r0 in range(0, self.total_rows, chunk):
                 r1 = min(self.total_rows, r0 + chunk)
@@ -260,6 +277,9 @@ class AutoIntTrainer:
         ph = lambda name: _Phase(self.timer, name)
         main = torch.cuda.current_stream(self.dev)
         self._stamp("step_begin")
+        if self.idmap is not None:
+            with ph("idmap"):
+                self.idmap.resolve(self.ids, self.id_fields, insert=True, out=self.ids_rows)
         # Adam's step counter / bias corrections are read by the two optimizer kernels at the end of the step only:
         # advance them on the side stream now instead of between the backward and the sparse update
         self.side.wait_stream(main)
@@ -272,9 +292,10 @@ class AutoIntTrainer:
             # separate branch
             self._embed_forward(ph, st, T, gather=False)
             tabs, world, lbase_t, keys = self._lookup_args()
+            lk_ids, _, lk_rows = self._lookup_geom()
             with ph("interacting_fwd"):
-                cabi.call("rs_interacting_fwd_gather", tabs, self.table_ld, world, self.ids.data_ptr(), lbase_t.data_ptr(),
-                          self.rows_t.data_ptr(), self.X.data_ptr(), d, 0, keys, T, P["Wqkvr"].data_ptr(),
+                cabi.call("rs_interacting_fwd_gather", tabs, self.table_ld, world, lk_ids.data_ptr(), lbase_t.data_ptr(),
+                          lk_rows.data_ptr(), self.X.data_ptr(), d, 0, keys, T, P["Wqkvr"].data_ptr(),
                           P["bqkvr"].data_ptr(), P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps,
                           self.Z[:, self.n_deep:].data_ptr(), U, self.zw, self.saved.data_ptr(), B, F, d, U,
                           c.head_num, c.layer_num, int(c.use_res), st)
@@ -407,13 +428,20 @@ class AutoIntTrainer:
             self._stamp("side_sort_end")
 
     # ---- embedding halves of the step (overridden by the row-sharded multi-GPU trainer)
+    def _lookup_geom(self):
+        """(ids, row_base, rows) the embedding lookups read: the raw ids with the modulo geometry, or (hash mode) the
+        mapped arena rows with the identity geometry."""
+        if self.idmap is None:
+            return self.ids, self.base_t, self.rows_t
+        return self.ids_rows, self.id_base_t, self.id_rows_t
+
     def _lookup_args(self):
         """(address of the W table pointers, W, per-field local row base, sort-key buffer) of the fused lookup."""
         if not hasattr(self, "_tab1"):
             import ctypes
             self._tab1 = (ctypes.c_void_p * 1)(self.table.data_ptr())
         import ctypes
-        return ctypes.addressof(self._tab1), 1, self.base_t, self.keys.data_ptr()
+        return ctypes.addressof(self._tab1), 1, self._lookup_geom()[1], self.keys.data_ptr()
 
     def _scatter_args(self):
         """(address of the W receive-buffer pointers, W, rank, inverse, cap) of the fused gradient push; None on one GPU."""
@@ -437,9 +465,10 @@ class AutoIntTrainer:
         n = c.batch * c.num_fields
         if not gather:
             return
+        ids, base, rows = self._lookup_geom()
         with ph("embed_gather"):
-            cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, self.ids.data_ptr(),
-                      self.base_t.data_ptr(), self.rows_t.data_ptr(), n, c.num_fields, c.embed_dim, self.X.data_ptr(), T,
+            cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(),
+                      base.data_ptr(), rows.data_ptr(), n, c.num_fields, c.embed_dim, self.X.data_ptr(), T,
                       self.keys.data_ptr(), None, st)
 
     def _embed_backward(self, ph, st, T, main):
@@ -495,7 +524,12 @@ class AutoIntTrainer:
 
     # ---- capture: the warm-up launch must not train ---------------------------------------------------
     def _touched_rows(self) -> torch.Tensor:
-        """Arena rows the step on the CURRENT static id buffer updates (sorted unique int64)."""
+        """Arena rows the step on the CURRENT static id buffer updates (sorted unique int64); hash mode: the rows of
+        the ids already mapped and every row the step's insert may hand out."""
+        if self.idmap is not None:
+            rows = self.idmap.resolve(self.ids, self.id_fields, insert=False)
+            pending = self.idmap.pending_rows([self.cfg.batch] * self.cfg.num_fields)
+            return torch.unique(torch.cat([rows[rows >= 0], pending]))
         rows = self.base_t[None, :] + torch.remainder(self.ids, self.rows_t[None, :])
         return torch.unique(rows[self.ids >= 0])
 
@@ -508,6 +542,8 @@ class AutoIntTrainer:
                 "scalars": self.adam_scalars.clone()}
         if self.bf16:
             snap["WT16"] = {k: v.clone() for k, v in self.WT16.items()}
+        if self.idmap is not None:
+            snap["idmap"] = self.idmap.snapshot()
         return snap
 
     def _restore(self, snap):
@@ -516,6 +552,8 @@ class AutoIntTrainer:
         self.flat_bf16.copy_(snap["flat_bf16"]); self.adam_scalars.copy_(snap["scalars"])
         for k, v in snap.get("WT16", {}).items():
             self.WT16[k].copy_(v)
+        if "idmap" in snap:
+            self.idmap.restore(snap["idmap"])
 
     def capture(self):
         """Capture the step into a CUDA graph.  The warm-up launch (one real step on whatever the static id / label
@@ -605,7 +643,8 @@ class AutoIntTrainer:
 
     @torch.no_grad()
     def predict(self, ids: torch.Tensor) -> torch.Tensor:
-        """Forward only (clip(sigmoid) probabilities), eager launches."""
+        """Forward only (clip(sigmoid) probabilities), eager launches.  Hash mode: ids are looked up, never inserted
+        (unseen ids read as zero vectors)."""
         c = self.cfg
         F, d, U, B = c.num_fields, c.embed_dim, c.unit_num, c.batch
         assert ids.shape == (B, F)
@@ -613,8 +652,11 @@ class AutoIntTrainer:
         T = ops._DT[self.act_dtype]
         st = ops._stream()
         P = self.P
-        cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, self.ids.data_ptr(),
-                  self.base_t.data_ptr(), self.rows_t.data_ptr(), B * F, F, d, self.X.data_ptr(), T, None, None, st)
+        if self.idmap is not None:
+            self.idmap.resolve(self.ids, self.id_fields, insert=False, out=self.ids_rows)
+        ids, base, rows = self._lookup_geom()
+        cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(),
+                  base.data_ptr(), rows.data_ptr(), B * F, F, d, self.X.data_ptr(), T, None, None, st)
         cabi.call("rs_interacting_fwd", self.X.data_ptr(), d, 0, T, P["Wqkvr"].data_ptr(), P["bqkvr"].data_ptr(),
                   P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps, self.Z[:, self.n_deep:].data_ptr(), U,
                   self.zw, None, B, F, d, U, c.head_num, c.layer_num, int(c.use_res), 0, st)

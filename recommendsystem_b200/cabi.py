@@ -52,6 +52,10 @@ PROTOTYPES = {
     "rs_route_ids_padded": (_i, [_p, _i64, _i, _p, _p, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "rs_route_ids_padded_spread": (_i, [_p, _i64, _i, _p, _p, _i, _i, _p, _p, _p, _p, _p, _sz, _p]),
     "rs_permute_rows": (_i, [_p, _p, _p, _i64, _i, _i, _i, _p]),
+    "rs_idmap_insert": (_i, [_p, _p, _p, _p, _i, _p, _i64, _i, _p, _u64, _f, _p, _i64, _i, _p, _i64, _i, _f,
+                             _p, _i64, _i, _f, _p]),
+    "rs_idmap_lookup": (_i, [_p, _p, _p, _i, _p, _i64, _i, _p, _p, _i, _p]),
+    "rs_idmap_rebuild": (_i, [_p, _i64, _p, _p, _p, _i, _i64, _p]),
     "rs_interacting_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "rs_interacting_saved_bytes": (_sz, [_i, _i, _i, _i]),
     "rs_interacting_path": (_i, [_i, _i, _i, _i, _i, _i, _f]),

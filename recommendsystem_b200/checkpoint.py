@@ -9,6 +9,9 @@ sub-model whose Keras weight names are the serving contract (`rank/multi_head/au
     dense.npz                      fp32 master weights by name, `m/<name>`, `v/<name>`, `adam_scalars`
     tables.rank<r>of<W>.bin        that rank's arena as it lies in HBM: [n_local, 3, d] fp32 records
                                    [w | m | v] (DESIGN.md §2), field f at rows local_base[f]...
+    idmap.npz                      id_map="hash" trainers only (meta.json "id_map": "hash"): the ids owning the used
+                                   rows of every field (`key_of_row`, field after field), `rows_used`, `overflow`,
+                                   `rows_per_field`; loading copies the arena and rebuilds the map from it
 
 Every rank writes its own shard (device -> pinned host -> file in bounded chunks); rank 0 also
 writes meta.json and dense.npz (dense state is replicated).  Loading works for ANY world size:
@@ -108,6 +111,10 @@ def _world_rank(trainer) -> Tuple[int, int]:
     return int(getattr(trainer, "world", 1)), int(getattr(trainer, "rank", 0))
 
 
+def _id_map(trainer) -> str:
+    return "hash" if getattr(trainer, "idmap", None) is not None else "mod"
+
+
 def save_checkpoint(trainer, directory, step: int | None = None) -> Path:
     """Write `trainer`'s tables, sparse-Adam state, dense weights and dense-Adam state.  Collective
     for a ShardedAutoIntTrainer: every rank calls it; the caller barriers before reading."""
@@ -141,6 +148,10 @@ def save_checkpoint(trainer, directory, step: int | None = None) -> Path:
             dense["v/" + name] = trainer.flat_v[off:off + k].view(shape).cpu().numpy()
         dense["adam_scalars"] = trainer.adam_scalars.cpu().numpy()
         np.savez(directory / "dense.npz", **dense)
+        if _id_map(trainer) == "hash":
+            np.savez(directory / "idmap.npz", **trainer.idmap.state())
+        elif (directory / "idmap.npz").exists():           # left by an earlier hash-mode save into this directory
+            (directory / "idmap.npz").unlink()
         meta = {
             "format": FORMAT, "world": W, "embed_dim": int(d),
             "rows_per_field": [int(x) for x in trainer.rows_host],
@@ -148,6 +159,8 @@ def save_checkpoint(trainer, directory, step: int | None = None) -> Path:
             "dense_spec": [[nm, list(sh)] for nm, sh, _ in trainer.spec],
             "config": _cfg_dict(trainer.cfg), "step": step,
         }
+        if _id_map(trainer) == "hash":
+            meta["id_map"] = "hash"
         tmp = directory / "meta.json.tmp"
         tmp.write_text(json.dumps(meta, indent=1))
         os.replace(tmp, directory / "meta.json")
@@ -167,6 +180,9 @@ def load_checkpoint(trainer, directory, tables: bool = True, dense: bool = True)
     directory = Path(directory)
     meta = read_meta(directory)
     W, r = _world_rank(trainer)
+    if meta.get("id_map", "mod") != _id_map(trainer):
+        raise ValueError(f"checkpoint id_map={meta.get('id_map', 'mod')!r} does not match the trainer's "
+                         f"id_map={_id_map(trainer)!r}")
     if tables:
         if [int(x) for x in trainer.rows_host] != meta["rows_per_field"] or trainer.arena.shape[2] != meta["embed_dim"]:
             raise ValueError("checkpoint tables do not match the trainer's rows_per_field / embed_dim")
@@ -180,6 +196,9 @@ def load_checkpoint(trainer, directory, tables: bool = True, dense: bool = True)
                 arena[int(dst[0]): int(dst[-1]) + 1].copy_(t)
             else:
                 arena.index_copy_(0, torch.from_numpy(dst).to(trainer.dev), t)
+        if _id_map(trainer) == "hash":
+            with np.load(directory / "idmap.npz") as z:
+                trainer.idmap.load_state({k: z[k] for k in z.files})
     if dense:
         with np.load(directory / "dense.npz") as z:
             for name, shape, off in trainer.spec:

@@ -188,6 +188,35 @@ def route_ids_padded(ids, F, rows, local_base, world, capacity, send_rows=None, 
     return send_rows, inverse, counts, overflow
 
 
+def idmap_insert(slots, key_of_row, counters, geom, ids, field_of_col, seed, scale, w, states=()):
+    """rs_idmap_insert: new (field, id) keys of `ids` [..., F] get rows; their records are initialised.  `w` is an
+    fp32 [R, d] view with contiguous rows; `states` up to two (fp32 view [R] or [R, k], initial value) pairs."""
+    _need(ids.dtype == torch.int64 and ids.is_contiguous(), "ids must be contiguous int64")
+    _need(w.dtype == torch.float32 and w.dim() == 2 and w.stride(1) == 1, "w must be fp32 [R, d] with contiguous rows")
+    st = []
+    for t, v in states:
+        _need(t.dtype == torch.float32 and (t.dim() == 1 or t.stride(1) == 1), "optimizer state: fp32, contiguous rows")
+        st += [_ptr(t), t.stride(0), 1 if t.dim() == 1 else t.shape[1], float(v)]
+    st += [None, 0, 0, 0.0] * (2 - len(states))
+    call("rs_idmap_insert", _ptr(slots), _ptr(key_of_row), _ptr(counters), _ptr(geom), geom.shape[0], _ptr(ids),
+         ids.numel(), field_of_col.numel(), _ptr(field_of_col), int(seed) & 0xFFFFFFFFFFFFFFFF, float(scale), _ptr(w),
+         w.stride(0), w.shape[1], *st, _stream())
+
+
+def idmap_lookup(slots, counters, geom, ids, field_of_col, out=None, after_insert=False):
+    """rs_idmap_lookup: int64 arena rows of `ids` [..., F] (-1: padding, unseen or overflowed)."""
+    _need(ids.dtype == torch.int64 and ids.is_contiguous(), "ids must be contiguous int64")
+    out = torch.empty(ids.shape, dtype=torch.int64, device=ids.device) if out is None else out
+    call("rs_idmap_lookup", _ptr(slots), _ptr(counters), _ptr(geom), geom.shape[0], _ptr(ids), ids.numel(),
+         field_of_col.numel(), _ptr(field_of_col), _ptr(out), int(after_insert), _stream())
+    return out
+
+
+def idmap_rebuild(slots, key_of_row, counters, geom, max_rows):
+    call("rs_idmap_rebuild", _ptr(slots), slots.numel() // 2, _ptr(key_of_row), _ptr(counters), _ptr(geom),
+         geom.shape[0], int(max_rows), _stream())
+
+
 def permute_rows(src, index, scatter=False, out=None):
     n, d = index.numel(), src.shape[-1]
     out = torch.empty(n, d, dtype=src.dtype, device=src.device) if out is None else out

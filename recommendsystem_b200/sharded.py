@@ -111,6 +111,9 @@ class ShardedAutoIntTrainer(AutoIntTrainer):
     def __init__(self, cfg: AutoIntConfig, device, group=None, global_tables: torch.Tensor | None = None,
                  dense_init: dict | None = None, capacity_factor: float | None = None,
                  peer_gather: bool | None = None, capacity: int | None = None, peer_ids: bool | None = None):
+        if cfg.id_map != "mod":
+            # the owners would have to map the routed ids before the peers read rows by index: not built yet
+            raise NotImplementedError("ShardedAutoIntTrainer supports id_map='mod' only (row-sharded id maps are not built)")
         self.ex = Exchange(group)
         self.world, self.rank = self.ex.world, self.ex.rank
         self._global_tables = global_tables
