@@ -15,11 +15,10 @@ from __future__ import annotations
 from dataclasses import dataclass
 from typing import Dict, List, Optional
 
-import numpy as np
 import torch
 
 from .. import cabi, ops
-from ..idmap import IdMap, check_id_map
+from ..arena import Arena
 
 
 @dataclass
@@ -82,7 +81,7 @@ class EmbeddingFeatures:
 
     def __init__(self, embedding_columns: List[EmbeddingColumn], sparse_opt, name="embedding", device="cuda:0",
                  out_dtype=torch.float32, seed=0, id_map="mod"):
-        self.id_map = check_id_map(id_map)
+        self.id_map = id_map
         self.cols = list(embedding_columns)
         self.opt = sparse_opt
         self.dev = torch.device(device)
@@ -91,50 +90,24 @@ class EmbeddingFeatures:
             raise ValueError("one EmbeddingFeatures layer holds columns of a single dimension (one arena)")
         self.d = dims.pop()
         self.out_dtype = out_dtype
-        rows = np.asarray([c.categorical_column.bucket_size for c in self.cols], np.int64)
-        self.base = np.concatenate([[0], np.cumsum(rows)[:-1]]).astype(np.int64)
-        self.rows = rows
         if not isinstance(sparse_opt, (Adam, AdaGrad)):
             raise TypeError("sparse_opt must be api.embedding.Adam or AdaGrad")
-        self.idmap = None
-        total = self._alloc_tables(seed)
-        self.row_bits = ops.row_bits(total)
-        self._last = None
-        self._geom_cache = {}
-
-    def _init_scale(self):
-        return float(getattr(self.opt, "initial_scale", 0.1) if isinstance(self.opt, AdaGrad) else 0.1)
-
-    def _alloc_state(self, n_rows):
-        """Storage for `n_rows` table rows + optimizer state: Adam keeps one [w | m | v] record per row (DESIGN.md 2:
-        the sparse update touches ONE contiguous 12d-byte block per row instead of three far-apart ones)."""
-        if isinstance(self.opt, Adam):
-            self.arena = torch.zeros(n_rows, 3, self.d, device=self.dev)
-            self.table, self.m, self.v = self.arena[:, 0, :], self.arena[:, 1, :], self.arena[:, 2, :]
-            self.table_ld = 3 * self.d
+        scale = float(getattr(sparse_opt, "initial_scale", 0.1) if isinstance(sparse_opt, AdaGrad) else 0.1)
+        adagrad = None if isinstance(sparse_opt, Adam) else (sparse_opt.initial_g2sum, sparse_opt.per_element)
+        # every table of the layer in one arena (sharded layer: this rank's rows of it), N(0, scale) from `seed`
+        self.store = ar = Arena([c.categorical_column.bucket_size for c in self.cols], self.d, self.dev,
+                                shard=self._arena_shard(), adagrad=adagrad, id_map=id_map, seed=seed, scale=scale)
+        if ar.idmap is None:                    # (hash mode: a row is initialised when its id is first inserted)
+            ar.init_normal(seed, scale)
+        self.table, self.arena, self.m, self.v, self.g2sum = ar.w, ar.records, ar.m, ar.v, ar.g2sum
+        self.idmap, self.base, self.rows, self.table_ld, self.row_bits = ar.idmap, ar.base, ar.rows, ar.ld, ar.row_bits
+        if isinstance(sparse_opt, Adam):
             self.scalars = torch.zeros(4, device=self.dev)
-        else:
-            self.table = torch.zeros(n_rows, self.d, device=self.dev)
-            self.table_ld = self.d
-            shape = (n_rows, self.d) if self.opt.per_element else (n_rows,)
-            self.g2sum = torch.full(shape, float(self.opt.initial_g2sum), device=self.dev)
+        self._last = None
 
-    def _alloc_tables(self, seed) -> int:
-        """Allocate and initialise (N(0, scale), one generator stream over the rows in arena order); returns the number
-        of rows the sort keys must address."""
-        total = int(self.rows.sum())
-        self._alloc_state(total)
-        if self.id_map == "hash":                       # rows are initialised when their id is first inserted
-            states = [(self.m, 0.0), (self.v, 0.0)] if isinstance(self.opt, Adam) else \
-                [(self.g2sum, float(self.opt.initial_g2sum))]
-            self.idmap = IdMap(self.rows, self.dev, seed, self._init_scale(), self.table, states)
-            return total
-        gen = torch.Generator(device=self.dev).manual_seed(seed)
-        chunk = 1 << 22
-        for r0 in range(0, total, chunk):
-            r1 = min(total, r0 + chunk)
-            self.table[r0:r1] = torch.empty(r1 - r0, self.d, device=self.dev).normal_(0.0, self._init_scale(), generator=gen)
-        return total
+    def _arena_shard(self):
+        """(W, rank) of a row-sharded layer; None on one GPU."""
+        return None
 
     def __call__(self, inputs: Dict[str, torch.Tensor]):
         out, plan = {}, []
@@ -146,7 +119,7 @@ class EmbeddingFeatures:
         if len(single) > 1:
             ids = torch.stack([inputs[self.cols[ci].categorical_column.key].reshape(-1) for ci in single], dim=1)
             ids = ids.to(self.dev, torch.int64).contiguous()
-            ids, base, rows = self._lookup(ids, tuple(single))
+            ids, base, rows = self._lookup(ids, single)
             emb, keys, _ = ops.embed_gather(self.table, ids, base, rows, torch.float32, want_keys=True)
             for j, ci in enumerate(single):
                 out[self.cols[ci].key] = emb[:, j, :].to(self.out_dtype)
@@ -208,70 +181,32 @@ class EmbeddingFeatures:
     def touched_rows(self, inputs: Dict[str, torch.Tensor]) -> torch.Tensor:
         """Sorted unique arena rows a step on `inputs` reads and updates (hash mode: the rows of the ids already
         mapped, and every row the step's inserts may hand out)."""
-        rows, lookups = [], []
+        return self.store.touched_rows(list(self._column_ids(inputs)))
+
+    def _column_ids(self, inputs):
+        """(ids [N, 1], (column,)) of every column: the ids a step on `inputs` looks up (< 0 = padding)."""
         for ci, c in enumerate(self.cols):
             ids = inputs[c.categorical_column.key]
             if isinstance(ids, (tuple, list)):                   # CSR bag: (values, offsets)
                 ids = ids[0]
-            ids = ids.to(self.dev, torch.int64).reshape(-1)
-            if c.combiner is None and c.seq_max_len:
-                ids = inputs[c.categorical_column.key].to(self.dev, torch.int64)[:, :c.seq_max_len].reshape(-1)
-            ids = ids[ids >= 0]
-            if self.idmap is not None:
-                r = self.idmap.resolve(ids.reshape(-1, 1).contiguous(), self.idmap.fields((ci,)), insert=False)
-                rows.append(r[r >= 0].reshape(-1))
-                lookups.append(ids.numel())
-                continue
-            rows.append(int(self.base[ci]) + torch.remainder(ids, int(self.rows[ci])))
-        if self.idmap is not None:
-            rows.append(self.idmap.pending_rows(lookups))
-        return torch.unique(torch.cat(rows)) if rows else torch.empty(0, dtype=torch.int64, device=self.dev)
+            elif c.combiner is None and c.seq_max_len:
+                ids = ids[:, :c.seq_max_len]
+            yield ids.to(self.dev, torch.int64).reshape(-1, 1), (ci,)
 
     def snapshot(self, inputs):
-        rows = self.touched_rows(inputs)
-        if isinstance(self.opt, Adam):
-            snap = {"rows": rows, "arena": self.arena[rows].clone(), "scalars": self.scalars.clone()}
-        else:
-            snap = {"rows": rows, "table": self.table[rows].clone(), "g2sum": self.g2sum[rows].clone()}
-        if self.idmap is not None:
-            snap["idmap"] = self.idmap.snapshot()
-        return snap
+        scalars = self.scalars.clone() if isinstance(self.opt, Adam) else None
+        return self.store.snapshot(self.touched_rows(inputs)), scalars
 
     def restore(self, snap):
-        rows = snap["rows"]
-        if isinstance(self.opt, Adam):
-            self.arena[rows] = snap["arena"]
-            self.scalars.copy_(snap["scalars"])
-        else:
-            self.table[rows] = snap["table"]
-            self.g2sum[rows] = snap["g2sum"]
-        if "idmap" in snap:
-            self.idmap.restore(snap["idmap"])
+        rows, scalars = snap
+        self.store.restore(rows)
+        if scalars is not None:
+            self.scalars.copy_(scalars)
 
     def _lookup(self, ids, cols):
-        """(ids, row_base, rows) the gather kernels read for the columns `cols`: the raw ids with the modulo geometry,
-        or (hash mode) the mapped arena rows with an identity geometry (row_base 0, rows = arena rows)."""
-        if self.idmap is None:
-            return (ids, *self._geom(cols))
-        mapped = self.idmap.resolve(ids, self.idmap.fields(cols), insert=torch.is_grad_enabled())
-        key = ("identity", len(cols))
-        g = self._geom_cache.get(key)
-        if g is None:
-            g = (torch.zeros(len(cols), dtype=torch.int64, device=self.dev),
-                 torch.full((len(cols),), self.idmap.total_rows, dtype=torch.int64, device=self.dev))
-            self._geom_cache[key] = g
-        return (mapped, *g)
-
-    def _geom(self, cols):
-        """(row_base, rows) device tensors of a column group, created once (no host->device copy per call:
-        the step stays CUDA-graph capturable)."""
-        g = self._geom_cache.get(cols)
-        if g is None:
-            idx = list(cols)
-            g = (torch.as_tensor(np.asarray(self.base)[idx], device=self.dev),
-                 torch.as_tensor(np.asarray(self.rows)[idx], device=self.dev))
-            self._geom_cache[cols] = g
-        return g
+        """(ids, row_base, rows) the gather kernels read for the columns `cols`; hash mode inserts new ids when
+        gradients are enabled (training)."""
+        return self.store.lookup(ids, cols, insert=torch.is_grad_enabled())
 
     def backward(self, grads: Dict[str, torch.Tensor]):
         """Push d(loss)/d(output) of every column: segment-sum per touched row + optimizer update."""

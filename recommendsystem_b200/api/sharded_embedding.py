@@ -25,11 +25,11 @@ from __future__ import annotations
 import ctypes
 from typing import Dict, List
 
-import numpy as np
 import torch
 import torch.distributed as dist
 
 from .. import cabi, ops
+from ..arena import check_sharded_id_map, field_slices
 from ..sharded import bucket_capacity, map_peer_buffers
 from .embedding import Adam, AdaGrad, EmbeddingColumn, EmbeddingFeatures
 
@@ -42,8 +42,7 @@ class _Group:
 class ShardedEmbeddingFeatures(EmbeddingFeatures):
     def __init__(self, embedding_columns: List[EmbeddingColumn], sparse_opt, name="embedding", device="cuda:0",
                  out_dtype=torch.float32, seed=0, group=None, capacity_factor=None, id_map="mod"):
-        if id_map != "mod":
-            raise NotImplementedError("ShardedEmbeddingFeatures supports id_map='mod' only (row-sharded id maps are not built)")
+        check_sharded_id_map(id_map)
         if not dist.is_initialized():
             raise RuntimeError("ShardedEmbeddingFeatures needs torch.distributed (one process per GPU)")
         self.group = group
@@ -53,34 +52,16 @@ class ShardedEmbeddingFeatures(EmbeddingFeatures):
         self.capacity_factor = capacity_factor
         self._ipc_opened = {}
         self._groups: Dict[tuple, _Group] = {}
-        super().__init__(embedding_columns, sparse_opt, name, device, out_dtype, seed)
+        super().__init__(embedding_columns, sparse_opt, name, device, out_dtype, seed, id_map)
         self.peer_tables = map_peer_buffers(self.table, self.world, self.rank, group, self._ipc_opened)
         self.flags = torch.zeros(16, dtype=torch.int32, device=self.dev)
         torch.cuda.synchronize(self.dev)
         self.peer_flags = map_peer_buffers(self.flags, self.world, self.rank, group, self._ipc_opened)
         self.overflow = torch.zeros(1, dtype=torch.int32, device=self.dev)
 
-    # ---- tables: this rank's rows of every column, same values as the unsharded layer with the same seed ----
-    def _alloc_tables(self, seed) -> int:
-        W = self.world
-        self.local_rows = (self.rows + W - 1) // W
-        self.local_base = np.concatenate([[0], np.cumsum(self.local_rows)[:-1]]).astype(np.int64)
-        n_local = int(self.local_rows.sum())
-        self._alloc_state(n_local)
-        total = int(self.rows.sum())
-        gen = torch.Generator(device=self.dev).manual_seed(seed)       # the SAME stream on every rank
-        base_t = torch.as_tensor(self.base, device=self.dev)
-        lbase_t = torch.as_tensor(self.local_base, device=self.dev)
-        chunk = 1 << 22
-        for r0 in range(0, total, chunk):
-            r1 = min(total, r0 + chunk)
-            vals = torch.empty(r1 - r0, self.d, device=self.dev).normal_(0.0, self._init_scale(), generator=gen)
-            r = torch.arange(r0, r1, device=self.dev)
-            col = torch.searchsorted(base_t, r, right=True) - 1
-            i = r - base_t[col]
-            mine = torch.remainder(i, W) == self.rank
-            self.table[(lbase_t[col] + torch.div(i, W, rounding_mode="floor"))[mine]] = vals[mine]
-        return n_local
+    # this rank's rows of every column hold the same values as the unsharded layer with the same seed
+    def _arena_shard(self):
+        return self.world, self.rank
 
     # ---- exchange buffers ------------------------------------------------------------------------------------
     def _group(self, gkey, n, cols, padded=False) -> _Group:
@@ -96,9 +77,7 @@ class ShardedEmbeddingFeatures(EmbeddingFeatures):
         # (rs_route_ids_padded_spread): the buckets stay balanced and the usual capacity holds.
         g.cap = bucket_capacity(n, W, self.capacity_factor)
         g.pad_spread = bool(padded)
-        idx = list(cols)
-        g.lbase_t = torch.as_tensor(self.local_base[idx], device=dev)
-        g.rows_t = torch.as_tensor(self.rows[idx], device=dev)
+        g.lbase_t, g.rows_t = self.store.geom(cols)
         g.send_rows = torch.empty(W * g.cap, dtype=torch.int32, device=dev)
         g.recv_rows = torch.empty(W * g.cap, dtype=torch.int32, device=dev)
         g.inverse = torch.empty(n, dtype=torch.int32, device=dev)
@@ -202,20 +181,13 @@ class ShardedEmbeddingFeatures(EmbeddingFeatures):
     # ---- state one step changes (GraphedTrainStep) / test helpers -------------------------------------------
     def touched_rows(self, inputs: Dict[str, torch.Tensor]) -> torch.Tensor:
         """LOCAL rows a step on the current inputs of ALL ranks updates on this rank (collective)."""
-        rows = []
-        for ci, c in enumerate(self.cols):
-            ids = inputs[c.categorical_column.key].to(self.dev, torch.int64)
-            if c.combiner is None and c.seq_max_len:
-                ids = ids[:, :c.seq_max_len]
-            ids = ids.reshape(-1).contiguous()
+        groups = []
+        for ids, cols in self._column_ids(inputs):
+            ids = ids.contiguous()
             everyone = [torch.empty_like(ids) for _ in range(self.world)]
             dist.all_gather(everyone, ids, group=self.group)
-            ids = torch.cat(everyone)
-            ids = ids[ids >= 0]
-            i = torch.remainder(ids, int(self.rows[ci]))
-            i = i[torch.remainder(i, self.world) == self.rank]
-            rows.append(int(self.local_base[ci]) + torch.div(i, self.world, rounding_mode="floor"))
-        return torch.unique(torch.cat(rows)) if rows else torch.empty(0, dtype=torch.int64, device=self.dev)
+            groups.append((torch.cat(everyone), cols))
+        return self.store.touched_rows(groups)
 
     def restore(self, snap):
         super().restore(snap)
@@ -227,10 +199,8 @@ class ShardedEmbeddingFeatures(EmbeddingFeatures):
         mine = self.table.contiguous()
         shards = [torch.empty_like(mine) for _ in range(self.world)]
         dist.all_gather(shards, mine, group=self.group)
-        out = torch.empty(int(self.rows.sum()), self.d, device=self.dev)
-        for ci in range(len(self.cols)):
-            R, b, lb = int(self.rows[ci]), int(self.base[ci]), int(self.local_base[ci])
-            for r in range(self.world):
-                n = len(range(r, R, self.world))
-                out[b + r: b + R: self.world] = shards[r][lb: lb + n]
+        out = torch.empty(self.store.total_rows, self.d, device=self.dev)
+        for r in range(self.world):
+            for g, loc in field_slices(self.rows, self.world, r):
+                out[g] = shards[r][loc]
         return out

@@ -23,7 +23,7 @@ import numpy as np
 import torch
 
 from . import cabi, ops
-from .idmap import IdMap, check_id_map
+from .arena import Arena
 
 
 class PhaseTimer:
@@ -111,21 +111,15 @@ class AutoIntTrainer:
         if self.dev.type != "cuda":
             raise RuntimeError("AutoIntTrainer runs on a CUDA device only (no CPU fallback)")
         self.act_dtype = {"f32": torch.float32, "bf16": torch.bfloat16}[cfg.dtype]
-        if check_id_map(cfg.id_map) == "hash" and tables is not None:
-            raise ValueError("tables= initialises rows by position; with id_map='hash' rows are initialised per id")
         F, d, U, B = cfg.num_fields, cfg.embed_dim, cfg.unit_num, cfg.batch
         if cfg.layer_num > 1 and d != U:
             raise ValueError("layer_num > 1 needs embed_dim == unit_num (InteractingLayer.py:41-46)")
-        rows = cfg.rows()
-        self.rows_host = np.asarray(rows, np.int64)
-        self.base_host = np.concatenate([[0], np.cumsum(self.rows_host)[:-1]]).astype(np.int64)
-        self.total_rows = int(self.rows_host.sum())
-        if self.total_rows >= 2 ** 31 - 1:
-            raise ValueError("arena rows must fit int32")
-        self.rows_t = torch.from_numpy(self.rows_host).to(self.dev)
-        self.base_t = torch.from_numpy(self.base_host).to(self.dev)
-        self.idmap = None
-        self._alloc_tables(tables)
+        self.store = ar = Arena(cfg.rows(), d, self.dev, shard=self._arena_shard(), id_map=cfg.id_map, seed=cfg.seed,
+                                scale=cfg.table_init_scale)
+        self.arena, self.table, self.table_m, self.table_v, self.table_ld = ar.records, ar.w, ar.m, ar.v, ar.ld
+        self.rows_host, self.base_host, self.rows_t, self.base_t = ar.rows, ar.base, ar.rows_t, ar.base_t
+        self.total_rows, self.idmap, self.row_bits = ar.total_rows, ar.idmap, ar.row_bits
+        self._init_tables(tables)
 
         # ---- dense parameters: one flat fp32 buffer (+ grads, m, v, bf16 shadow) with views
         self.spec = []
@@ -154,13 +148,11 @@ class AutoIntTrainer:
         T = self.act_dtype
         e = lambda *shape, dtype=T: torch.empty(*shape, device=self.dev, dtype=dtype)
         self.ids = torch.zeros(B, F, dtype=torch.int64, device=self.dev)
-        if self.idmap is not None:
-            # hash mode: the step's first two launches map ids -> arena rows (static buffer), and every gather reads
-            # those rows through an identity geometry (row_base 0, rows = total rows: id mod rows = id)
-            self.ids_rows = torch.full((B, F), -1, dtype=torch.int64, device=self.dev)
-            self.id_fields = self.idmap.fields(range(F))
-            self.id_base_t = torch.zeros(F, dtype=torch.int64, device=self.dev)
-            self.id_rows_t = torch.full((F,), self.total_rows, dtype=torch.int64, device=self.dev)
+        # hash mode: the step's first two launches map ids -> arena rows (static buffer) that every lookup reads
+        self.ids_rows = None if self.idmap is None else torch.full((B, F), -1, dtype=torch.int64, device=self.dev)
+        self.fields = tuple(range(F))
+        # (ids, row_base, rows) the step's embedding lookups read
+        self.lookup = (self.ids if self.idmap is None else self.ids_rows, *ar.geom(self.fields))
         self.labels = torch.zeros(B, 1, device=self.dev)
         self.X = e(B, F, d)
         self.keys = torch.empty(B * F, dtype=torch.int64, device=self.dev)
@@ -200,31 +192,19 @@ class AutoIntTrainer:
         self.head_ws = ops.logit_head_workspace(B, self.zw, self.dev)     # head partials, reduced on the side stream
 
     # ------------------------------------------------------------------ setup
-    def _alloc_tables(self, tables):
-        cfg, d = self.cfg, self.cfg.embed_dim
-        gen = torch.Generator(device=self.dev).manual_seed(cfg.seed)
-        self._alloc_arena(self.total_rows, d)
-        if cfg.id_map == "hash":                         # a row is initialised when its id is first inserted
-            self.idmap = IdMap(self.rows_host, self.dev, cfg.seed, cfg.table_init_scale, self.table,
-                               [(self.table_m, 0.0), (self.table_v, 0.0)])
-        elif tables is None:
-            chunk = 1 << 22                              # initialise through bounded temporaries
-            for r0 in range(0, self.total_rows, chunk):
-                r1 = min(self.total_rows, r0 + chunk)
-                self.table[r0:r1] = torch.empty(r1 - r0, d, device=self.dev).normal_(0.0, cfg.table_init_scale,
-                                                                                     generator=gen)
-        else:
-            assert tuple(tables.shape) == (self.total_rows, d)
-            self.table.copy_(tables.to(self.dev, torch.float32))
-        self.row_bits = ops.row_bits(self.total_rows)
+    def _arena_shard(self):
+        """(W, rank) of a row-sharded arena; None on one GPU."""
+        return None
 
-    def _alloc_arena(self, n_rows, d):
-        """One 3d-float record [w | m | v] per row: the sparse Adam reads and writes ONE contiguous 12d-byte
-        block per touched row (a third of the random DRAM accesses of three separate arrays); the gather reads
-        the first d floats of the record (row stride 3d)."""
-        self.arena = torch.zeros(n_rows, 3, d, device=self.dev)
-        self.table, self.table_m, self.table_v = self.arena[:, 0, :], self.arena[:, 1, :], self.arena[:, 2, :]
-        self.table_ld = 3 * d
+    def _init_tables(self, tables):
+        """The global tables [total rows, d] given, or N(0, table_init_scale) from cfg.seed (hash mode: a row is
+        initialised when its id is first inserted)."""
+        if tables is not None:
+            if self.idmap is not None:
+                raise ValueError("tables= initialises rows by position; with id_map='hash' rows are initialised per id")
+            self.store.load_global(tables)
+        elif self.idmap is None:
+            self.store.init_normal(self.cfg.seed, self.cfg.table_init_scale)
 
     def _add(self, name, shape):
         off = 0
@@ -279,7 +259,7 @@ class AutoIntTrainer:
         self._stamp("step_begin")
         if self.idmap is not None:
             with ph("idmap"):
-                self.idmap.resolve(self.ids, self.id_fields, insert=True, out=self.ids_rows)
+                self.store.lookup(self.ids, self.fields, insert=True, out=self.ids_rows)
         # Adam's step counter / bias corrections are read by the two optimizer kernels at the end of the step only:
         # advance them on the side stream now instead of between the backward and the sparse update
         self.side.wait_stream(main)
@@ -292,7 +272,7 @@ class AutoIntTrainer:
             # separate branch
             self._embed_forward(ph, st, T, gather=False)
             tabs, world, lbase_t, keys = self._lookup_args()
-            lk_ids, _, lk_rows = self._lookup_geom()
+            lk_ids, _, lk_rows = self.lookup
             with ph("interacting_fwd"):
                 cabi.call("rs_interacting_fwd_gather", tabs, self.table_ld, world, lk_ids.data_ptr(), lbase_t.data_ptr(),
                           lk_rows.data_ptr(), self.X.data_ptr(), d, 0, keys, T, P["Wqkvr"].data_ptr(),
@@ -428,20 +408,13 @@ class AutoIntTrainer:
             self._stamp("side_sort_end")
 
     # ---- embedding halves of the step (overridden by the row-sharded multi-GPU trainer)
-    def _lookup_geom(self):
-        """(ids, row_base, rows) the embedding lookups read: the raw ids with the modulo geometry, or (hash mode) the
-        mapped arena rows with the identity geometry."""
-        if self.idmap is None:
-            return self.ids, self.base_t, self.rows_t
-        return self.ids_rows, self.id_base_t, self.id_rows_t
-
     def _lookup_args(self):
         """(address of the W table pointers, W, per-field local row base, sort-key buffer) of the fused lookup."""
         if not hasattr(self, "_tab1"):
             import ctypes
             self._tab1 = (ctypes.c_void_p * 1)(self.table.data_ptr())
         import ctypes
-        return ctypes.addressof(self._tab1), 1, self._lookup_geom()[1], self.keys.data_ptr()
+        return ctypes.addressof(self._tab1), 1, self.lookup[1], self.keys.data_ptr()
 
     def _scatter_args(self):
         """(address of the W receive-buffer pointers, W, rank, inverse, cap) of the fused gradient push; None on one GPU."""
@@ -465,7 +438,7 @@ class AutoIntTrainer:
         n = c.batch * c.num_fields
         if not gather:
             return
-        ids, base, rows = self._lookup_geom()
+        ids, base, rows = self.lookup
         with ph("embed_gather"):
             cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(),
                       base.data_ptr(), rows.data_ptr(), n, c.num_fields, c.embed_dim, self.X.data_ptr(), T,
@@ -526,34 +499,24 @@ class AutoIntTrainer:
     def _touched_rows(self) -> torch.Tensor:
         """Arena rows the step on the CURRENT static id buffer updates (sorted unique int64); hash mode: the rows of
         the ids already mapped and every row the step's insert may hand out."""
-        if self.idmap is not None:
-            rows = self.idmap.resolve(self.ids, self.id_fields, insert=False)
-            pending = self.idmap.pending_rows([self.cfg.batch] * self.cfg.num_fields)
-            return torch.unique(torch.cat([rows[rows >= 0], pending]))
-        rows = self.base_t[None, :] + torch.remainder(self.ids, self.rows_t[None, :])
-        return torch.unique(rows[self.ids >= 0])
+        return self.store.touched_rows([(self.ids, self.fields)])
 
     def _snapshot(self):
         """Everything one optimizer step changes: the [w|m|v] records of the touched rows, the dense parameters
         with their moments and bf16 shadows, the Adam step scalars."""
-        rows = self._touched_rows()
-        snap = {"rows": rows, "arena": self.arena[rows].clone(), "flat": self.flat.clone(),
+        snap = {"arena": self.store.snapshot(self._touched_rows()), "flat": self.flat.clone(),
                 "flat_m": self.flat_m.clone(), "flat_v": self.flat_v.clone(), "flat_bf16": self.flat_bf16.clone(),
                 "scalars": self.adam_scalars.clone()}
         if self.bf16:
             snap["WT16"] = {k: v.clone() for k, v in self.WT16.items()}
-        if self.idmap is not None:
-            snap["idmap"] = self.idmap.snapshot()
         return snap
 
     def _restore(self, snap):
-        self.arena[snap["rows"]] = snap["arena"]
+        self.store.restore(snap["arena"])
         self.flat.copy_(snap["flat"]); self.flat_m.copy_(snap["flat_m"]); self.flat_v.copy_(snap["flat_v"])
         self.flat_bf16.copy_(snap["flat_bf16"]); self.adam_scalars.copy_(snap["scalars"])
         for k, v in snap.get("WT16", {}).items():
             self.WT16[k].copy_(v)
-        if "idmap" in snap:
-            self.idmap.restore(snap["idmap"])
 
     def capture(self):
         """Capture the step into a CUDA graph.  The warm-up launch (one real step on whatever the static id / label
@@ -643,8 +606,8 @@ class AutoIntTrainer:
 
     @torch.no_grad()
     def predict(self, ids: torch.Tensor) -> torch.Tensor:
-        """Forward only (clip(sigmoid) probabilities), eager launches.  Hash mode: ids are looked up, never inserted
-        (unseen ids read as zero vectors)."""
+        """Forward only on this rank's batch (clip(sigmoid) probabilities), eager launches.  Hash mode: ids are looked
+        up, never inserted (unseen ids read as zero vectors).  Sharded: collective, every rank must call it."""
         c = self.cfg
         F, d, U, B = c.num_fields, c.embed_dim, c.unit_num, c.batch
         assert ids.shape == (B, F)
@@ -652,11 +615,7 @@ class AutoIntTrainer:
         T = ops._DT[self.act_dtype]
         st = ops._stream()
         P = self.P
-        if self.idmap is not None:
-            self.idmap.resolve(self.ids, self.id_fields, insert=False, out=self.ids_rows)
-        ids, base, rows = self._lookup_geom()
-        cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(),
-                  base.data_ptr(), rows.data_ptr(), B * F, F, d, self.X.data_ptr(), T, None, None, st)
+        self._predict_lookup(st, T)
         cabi.call("rs_interacting_fwd", self.X.data_ptr(), d, 0, T, P["Wqkvr"].data_ptr(), P["bqkvr"].data_ptr(),
                   P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps, self.Z[:, self.n_deep:].data_ptr(), U,
                   self.zw, None, B, F, d, U, c.head_num, c.layer_num, int(c.use_res), 0, st)
@@ -667,3 +626,11 @@ class AutoIntTrainer:
         ops.logit_head(self.Z, P["out_W"], P["out_b"], self.labels, self.dZ, self.G["out_W"], self.G["out_b"],
                        p_out=self.p_raw, loss=self.loss)
         return self.p_raw.float().clamp(1e-6, 1.0)
+
+    def _predict_lookup(self, st, T):
+        """X = the embedding rows of the static id buffer, inserting no id."""
+        c = self.cfg
+        ids, base, rows = self.store.lookup(self.ids, self.fields, insert=False, out=self.ids_rows)
+        cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(), base.data_ptr(),
+                  rows.data_ptr(), c.batch * c.num_fields, c.num_fields, c.embed_dim, self.X.data_ptr(), T, None, None,
+                  st)

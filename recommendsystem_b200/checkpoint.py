@@ -15,7 +15,7 @@ sub-model whose Keras weight names are the serving contract (`rank/multi_head/au
 
 Every rank writes its own shard (device -> pinned host -> file in bounded chunks); rank 0 also
 writes meta.json and dense.npz (dense state is replicated).  Loading works for ANY world size:
-global row g of a field lives in shard g % W at local row g // W (`sharded.shard_layout`), so a
+global row g of a field lives in shard g % W at local row g // W (`arena.shard_layout`), so a
 rank of a W'-way job collects the rows g = r', r'+W', ... from whichever old shards hold them.
 State is copied INTO the trainer's existing buffers: captured CUDA graphs and peer (IPC) mappings
 stay valid.  Resuming is exact: train(2) -> save -> load -> train(2) equals train(4) bit for bit
@@ -32,19 +32,13 @@ from typing import Dict, Iterator, Tuple
 import numpy as np
 import torch
 
+from .arena import shard_layout as shard_rows     # (local_rows[F], local_base[F]) of a W-way job
+
 FORMAT = "rs_b200.checkpoint.v1"
 CHUNK_ROWS = 1 << 20                     # rows per host staging chunk (192 MB at d = 16)
 
 
 # ------------------------------------------------------------------ layout (pure numpy, CPU-testable)
-def shard_rows(rows_per_field, world: int) -> Tuple[np.ndarray, np.ndarray]:
-    """(local_rows[F], local_base[F]) of every rank of a `world`-way job (= sharded.shard_layout)."""
-    rows = np.asarray(rows_per_field, np.int64)
-    local_rows = (rows + world - 1) // world
-    local_base = np.concatenate([[0], np.cumsum(local_rows)[:-1]]).astype(np.int64)
-    return local_rows, local_base
-
-
 def shard_path(directory, rank: int, world: int) -> Path:
     return Path(directory) / f"tables.rank{rank}of{world}.bin"
 

@@ -22,6 +22,7 @@ import numpy as np
 import torch
 
 from . import ops
+from .arena import shard_layout
 
 ID_MAPS = ("mod", "hash")
 
@@ -46,7 +47,7 @@ class IdMap:
     def __init__(self, rows_per_field, device, seed: int, scale: float, w: torch.Tensor, states=()):
         self.dev = torch.device(device)
         self.rows = np.asarray(rows_per_field, np.int64)
-        self.base = np.concatenate([[0], np.cumsum(self.rows)[:-1]]).astype(np.int64)
+        _, self.base = shard_layout(self.rows, 1)
         self.total_rows = int(self.rows.sum())
         if w.shape[0] != self.total_rows:
             raise ValueError(f"IdMap: weight view has {w.shape[0]} rows, the fields {self.total_rows}")

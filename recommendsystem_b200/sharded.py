@@ -31,12 +31,12 @@ import ctypes
 import os
 import math
 
-import numpy as np
 import torch
 import torch.distributed as dist
 
 from . import cabi, ops
-from .autoint import AutoIntConfig, AutoIntTrainer
+from .arena import INIT_CHUNK_ROWS, check_sharded_id_map, shard_layout  # noqa: F401  (shard_layout: re-exported)
+from .autoint import AutoIntConfig, AutoIntTrainer, _Phase
 
 
 def bucket_capacity(n_lookups: int, world: int, factor: float | None = None) -> int:
@@ -48,14 +48,6 @@ def bucket_capacity(n_lookups: int, world: int, factor: float | None = None) -> 
     else:
         cap = mean + 8.0 * math.sqrt(max(mean * (1 - 1.0 / world), 1.0)) + 64
     return min(n_lookups, int(math.ceil(cap / 128.0) * 128))
-
-
-def shard_layout(rows_per_field, world):
-    """rows of field f on every rank = ceil(R_f / W); returns (local_rows[F], local_base[F])."""
-    rows = np.asarray(rows_per_field, np.int64)
-    local_rows = (rows + world - 1) // world
-    local_base = np.concatenate([[0], np.cumsum(local_rows)[:-1]]).astype(np.int64)
-    return local_rows, local_base
 
 
 def map_peer_buffers(tensor, world, rank, group, opened):
@@ -111,14 +103,12 @@ class ShardedAutoIntTrainer(AutoIntTrainer):
     def __init__(self, cfg: AutoIntConfig, device, group=None, global_tables: torch.Tensor | None = None,
                  dense_init: dict | None = None, capacity_factor: float | None = None,
                  peer_gather: bool | None = None, capacity: int | None = None, peer_ids: bool | None = None):
-        if cfg.id_map != "mod":
-            # the owners would have to map the routed ids before the peers read rows by index: not built yet
-            raise NotImplementedError("ShardedAutoIntTrainer supports id_map='mod' only (row-sharded id maps are not built)")
+        check_sharded_id_map(cfg.id_map)          # before any collective
         self.ex = Exchange(group)
         self.world, self.rank = self.ex.world, self.ex.rank
-        self._global_tables = global_tables
         self._capacity_factor = capacity_factor
-        super().__init__(cfg, device, tables=None, dense_init=dense_init)
+        super().__init__(cfg, device, tables=global_tables, dense_init=dense_init)
+        self.local_rows, self.local_base, self.lbase_t = self.store.local_rows, self.store.local_base, self.store.lbase_t
         W, n, d = self.world, cfg.batch * cfg.num_fields, cfg.embed_dim
         # `capacity` pins the slots per (source, owner) bucket exactly (tests: buckets filled to the brim, forced overflow)
         self.cap = int(capacity) if capacity is not None else bucket_capacity(n, W, capacity_factor)
@@ -135,7 +125,6 @@ class ShardedAutoIntTrainer(AutoIntTrainer):
         self.g_recv = torch.empty(W * self.cap, d, dtype=T, device=dev)
         self.keys = torch.empty(W * self.cap, dtype=torch.int64, device=dev)
         self.keys_sorted = torch.empty_like(self.keys)
-        self.lbase_t = torch.from_numpy(self.local_base).to(dev)
         if peer_gather is None:
             peer_gather = dist.get_backend(group) == "nccl" and W <= 8
         self.peer_gather = bool(peer_gather)
@@ -179,26 +168,20 @@ class ShardedAutoIntTrainer(AutoIntTrainer):
         with ph(name):
             cabi.call("rs_peer_barrier", ctypes.addressof(self.peer_flags), self.world, self.rank, ops._stream())
 
-    def _alloc_tables(self, tables):
-        cfg, d, W = self.cfg, self.cfg.embed_dim, self.world
-        self.local_rows, self.local_base = shard_layout(self.rows_host, W)
-        n_local = int(self.local_rows.sum())
-        self._alloc_arena(n_local, d)
-        if self._global_tables is not None:
-            # rows of field f owned by this rank: global rows rank, rank+W, ... (parity tests)
-            g = self._global_tables.to(torch.float32)
-            for f in range(cfg.num_fields):
-                src = g[int(self.base_host[f]) + self.rank: int(self.base_host[f] + self.rows_host[f]): W]
-                self.table[int(self.local_base[f]): int(self.local_base[f]) + src.shape[0]] = src.to(self.dev)
-            self._global_tables = None
-        else:
-            gen = torch.Generator(device=self.dev).manual_seed(cfg.seed + 7919 * self.rank)
-            chunk = 1 << 22
-            for r0 in range(0, n_local, chunk):
-                r1 = min(n_local, r0 + chunk)
-                self.table[r0:r1] = torch.empty(r1 - r0, d, device=self.dev).normal_(0.0, cfg.table_init_scale,
-                                                                                     generator=gen)
-        self.row_bits = ops.row_bits(n_local)
+    def _arena_shard(self):
+        return self.world, self.rank
+
+    def _init_tables(self, tables):
+        """This rank's rows of the global tables given (parity tests), or its own N(0, table_init_scale) draw in local
+        row order from seed + 7919 rank (not the single-GPU trainer's tables)."""
+        if tables is not None:
+            return super()._init_tables(tables)
+        gen = torch.Generator(device=self.dev).manual_seed(self.cfg.seed + 7919 * self.rank)
+        n_local, d = self.store.n_local, self.cfg.embed_dim
+        for r0 in range(0, n_local, INIT_CHUNK_ROWS):
+            r1 = min(n_local, r0 + INIT_CHUNK_ROWS)
+            self.table[r0:r1] = torch.empty(r1 - r0, d, device=self.dev).normal_(0.0, self.cfg.table_init_scale,
+                                                                                 generator=gen)
 
     # ---- embedding halves of the step -----------------------------------------------------
     def _lookup_args(self):
@@ -314,11 +297,7 @@ class ShardedAutoIntTrainer(AutoIntTrainer):
         """LOCAL arena rows the step on the current static id buffers of ALL ranks updates on this rank."""
         everyone = [torch.empty_like(self.ids) for _ in range(self.world)]
         dist.all_gather(everyone, self.ids, group=self.ex.group)
-        ids = torch.cat(everyone, 0)
-        g = torch.remainder(ids, self.rows_t[None, :])
-        mine = (torch.remainder(g, self.world) == self.rank) & (ids >= 0)
-        local = self.lbase_t[None, :] + torch.div(g, self.world, rounding_mode="floor")
-        return torch.unique(local[mine])
+        return self.store.touched_rows([(torch.cat(everyone, 0), self.fields)])
 
     def capture(self):
         """Capture the sharded step (collectives included).  The warm-up launch runs on whatever the static id
@@ -332,35 +311,12 @@ class ShardedAutoIntTrainer(AutoIntTrainer):
         dist.barrier(group=self.ex.group)
         return g
 
-    @torch.no_grad()
-    def predict(self, ids: torch.Tensor) -> torch.Tensor:
-        """Forward only on this rank's batch (clip(sigmoid) probabilities): the gather goes through the sharded
-        path (_embed_forward: peer reads, or route + all-to-alls), never through the local shard with global row
-        numbers.  Collective: every rank must call it."""
-        c = self.cfg
-        F, d, U, B = c.num_fields, c.embed_dim, c.unit_num, c.batch
-        assert ids.shape == (B, F)
-        self.ids.copy_(ids)
-        T = ops._DT[self.act_dtype]
-        st = ops._stream()
-        P = self.P
-
-        class _NoTimer:
-            def __enter__(self): return self
-            def __exit__(self, *a): return False
-        self._embed_forward(lambda name: _NoTimer(), st, T)
-        main = torch.cuda.current_stream(self.dev)
-        if self.peer_gather:
-            main.wait_stream(self.side2)           # the owners' key work of _embed_forward is not needed here
-        cabi.call("rs_interacting_fwd", self.X.data_ptr(), d, 0, T, P["Wqkvr"].data_ptr(), P["bqkvr"].data_ptr(),
-                  P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps, self.Z[:, self.n_deep:].data_ptr(), U,
-                  self.zw, None, B, F, d, U, c.head_num, c.layer_num, int(c.use_res), 0, st)
-        acts = [self.X.view(B, F * d)] + self.H + [self.Z[:, :self.n_deep]]
-        for i in range(len(c.mlp_hidden)):
-            self._dense_fwd(acts[i], f"mlp_W{i}", f"mlp_b{i}", acts[i + 1])
-        ops.logit_head(self.Z, P["out_W"], P["out_b"], self.labels, self.dZ, self.G["out_W"], self.G["out_b"],
-                       p_out=self.p_raw, loss=self.loss)
-        return self.p_raw.float().clamp(1e-6, 1.0)
+    def _predict_lookup(self, st, T):
+        """The sharded gather (_embed_forward: peer reads, or route + all-to-alls), never the local shard with global
+        row numbers."""
+        self._embed_forward(lambda name: _Phase(None, name), st, T)
+        if self.peer_gather:       # the owners' key work of _embed_forward is not needed here
+            torch.cuda.current_stream(self.dev).wait_stream(self.side2)
 
     def check_overflow(self):
         """Raise if any routing bucket ever exceeded its capacity (ids too skewed for `capacity_factor`)."""

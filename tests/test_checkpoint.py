@@ -45,16 +45,6 @@ def test_reshard_any_world(tmp_path, old_w, new_w):
             np.testing.assert_array_equal(got, want)      # bit-exact
 
 
-def test_shard_rows_matches_sharded_layout():
-    from recommendsystem_b200.sharded import shard_layout
-    rows = [1000, 7, 33]
-    for W in (1, 2, 3, 8):
-        a, b = ck.shard_rows(rows, W)
-        c, e = shard_layout(rows, W)
-        np.testing.assert_array_equal(a, c)
-        np.testing.assert_array_equal(b, e)
-
-
 def test_bad_format_raises(tmp_path):
     (tmp_path / "meta.json").write_text(json.dumps({"format": "something else"}))
     with pytest.raises(ValueError):
