@@ -34,7 +34,8 @@ extern "C" {
 #define RS_ABI_VERSION 5   /* 4: + rs_interacting_path; saved buffer grows by the per-head softmax statistics.
                               5: + deferred parameter-gradient reductions (rs_logit_head_reduce, rs_interacting_bwd_reduce),
                                  rs_peer_all_to_all_i32, rs_embed_keys_from_rows;
-                                 + rs_idmap_insert / _lookup / _rebuild (additions only, same version) */
+                                 + rs_idmap_insert / _lookup / _rebuild, rs_idmap_count / _evict
+                                 (additions only, same version) */
 
 enum rs_dtype { RS_F32 = 0, RS_BF16 = 1 };
 
@@ -315,7 +316,27 @@ int rs_permute_rows(const void* src, void* out, const int32_t* index, int64_t n,
  * rs_idmap_rebuild clears all `n_slots` slots (cudaMemsetAsync) and re-inserts
  * key_of_row[row_base_f + j] for j < counters[0][f] with its row; key_of_row past
  * the counters is set to -1.  Used to restore a map from a checkpoint or to roll it
- * back to earlier counters.  max_rows = max R_f. */
+ * back to earlier counters.  max_rows = max R_f.
+ *
+ * Eviction (TensorNet's feature_drop_show; the rules are this library's choice):
+ *   show        fp32[total rows]: the show count of each row.  A row no key owns has
+ *               show 0 at all times, so a newly inserted key starts from 0.
+ * rs_idmap_count adds 1.0f to show[rows[i]] for every rows[i] >= 0 (atomicAdd; every
+ * increment adds the same value, so the sum is independent of their order; it stops
+ * growing at 2^24).  Callers pass the rows of training lookups only.
+ * rs_idmap_evict, for 0 < decay <= 1 and a finite threshold (else RS_ERR_INVALID):
+ *   1. show = fp32(show * decay) for every live row (row_base_f + j, j < counters[0][f]);
+ *   2. drops every key whose decayed show is < threshold and compacts each field's
+ *      live rows back into [row_base_f, row_base_f + live_f): the k-th dropped row
+ *      below live_f receives the record of the k-th kept row at or above live_f
+ *      (both ascending) — w (d floats, stride w_ld), s0 / s1 (nullable, s*_width
+ *      floats at stride s*_ld; the arguments of rs_idmap_insert), show and key_of_row;
+ *   3. vacated rows get show 0 and key_of_row -1; counters[0][f] = live_f and
+ *      evicted[f] (int64[n_fields], caller-owned) grows by the keys dropped;
+ *   4. rebuilds the slots as rs_idmap_rebuild.
+ * Asynchronous on `stream` (no host synchronisation); `ws` (256-B aligned) holds
+ * rs_idmap_evict_workspace_bytes(total_rows) bytes.  The layout after it is a pure
+ * function of the layout before; an evicted key is like a key never seen. */
 int rs_idmap_insert(void* slots, int64_t* key_of_row, int64_t* counters, const int64_t* geom, int n_fields,
                     const int64_t* ids, int64_t n, int F, const int32_t* field_of_col, uint64_t seed, float scale,
                     float* w, int64_t w_ld, int d, float* s0, int64_t s0_ld, int s0_width, float s0_init,
@@ -324,6 +345,12 @@ int rs_idmap_lookup(const void* slots, int64_t* counters, const int64_t* geom, i
                     int64_t n, int F, const int32_t* field_of_col, int64_t* rows_out, int after_insert, void* stream);
 int rs_idmap_rebuild(void* slots, int64_t n_slots, int64_t* key_of_row, const int64_t* counters, const int64_t* geom,
                      int n_fields, int64_t max_rows, void* stream);
+int rs_idmap_count(float* show, const int64_t* rows, int64_t n, void* stream);
+size_t rs_idmap_evict_workspace_bytes(int64_t total_rows);
+int rs_idmap_evict(void* slots, int64_t n_slots, int64_t* key_of_row, int64_t* counters, const int64_t* geom,
+                   int n_fields, int64_t total_rows, float* show, float threshold, float decay, float* w, int64_t w_ld,
+                   int d, float* s0, int64_t s0_ld, int s0_width, float* s1, int64_t s1_ld, int s1_width,
+                   int64_t* evicted, void* ws, size_t ws_bytes, void* stream);
 
 /* ------------------------------------------------- K4 InteractingLayer ----
  * InteractingLayer.call (InteractingLayer.py:37-61; duplicate at

@@ -9,7 +9,7 @@ batch is served by a single gather launch and a single sorted-segment update lau
 
 `id_map="hash"` replaces the modulo rule by a collision-free map (recommendsystem_b200.idmap): every distinct
 (column, id) gets its own row of the column's `bucket_size` rows, as TensorNet's hash tables give every feature sign
-its own row."""
+its own row, and `evict` drops the ids whose decayed show count falls below AdaGrad's `feature_drop_show`."""
 from __future__ import annotations
 
 from dataclasses import dataclass
@@ -19,6 +19,7 @@ import torch
 
 from .. import cabi, ops
 from ..arena import Arena
+from ..idmap import check_evict_args
 
 
 @dataclass
@@ -57,12 +58,13 @@ class Adam:
 
 class AdaGrad:
     """tn.core.AdaGrad(learning_rate, initial_g2sum, initial_scale[, feature_drop_show]).
-    One g2sum scalar per row (TensorNet style); rows are initialised N(0,1) * initial_scale."""
+    One g2sum scalar per row (TensorNet style); rows are initialised N(0,1) * initial_scale.  `feature_drop_show` is
+    the show threshold EmbeddingFeatures.evict uses by default (id_map="hash"); -1 drops nothing."""
 
     def __init__(self, learning_rate=0.01, initial_g2sum=0, initial_scale=1, epsilon=1e-8, feature_drop_show=-1,
                  per_element=False):
         self.learning_rate, self.initial_g2sum, self.initial_scale = learning_rate, initial_g2sum, initial_scale
-        self.epsilon, self.per_element = epsilon, per_element
+        self.epsilon, self.per_element, self.feature_drop_show = epsilon, per_element, feature_drop_show
 
 
 class EmbeddingFeatures:
@@ -77,7 +79,8 @@ class EmbeddingFeatures:
     column's row capacity and each distinct id gets its own row the first time a call with gradients enabled
     (training) sees it, initialised N(0, scale) as a function of (seed, column, id); calls under torch.no_grad()
     (the nets' predict) give unseen ids zero vectors and change nothing.  Once a column's rows are used up, new ids
-    read as zero vectors and get no update, like padding (`idmap.stats()` counts them)."""
+    read as zero vectors and get no update, like padding (`idmap.stats()` counts them).  Training calls also count
+    every id's shows; `evict(threshold, decay)` decays them and frees the rows of the ids below the threshold."""
 
     def __init__(self, embedding_columns: List[EmbeddingColumn], sparse_opt, name="embedding", device="cuda:0",
                  out_dtype=torch.float32, seed=0, id_map="mod"):
@@ -104,6 +107,7 @@ class EmbeddingFeatures:
         if isinstance(sparse_opt, Adam):
             self.scalars = torch.zeros(4, device=self.dev)
         self._last = None
+        self._pending_backward = False
 
     def _arena_shard(self):
         """(W, rank) of a row-sharded layer; None on one GPU."""
@@ -175,6 +179,7 @@ class EmbeddingFeatures:
                     out[c.key] = (emb.view(B, bag, self.d).sum(1) / cnt[:, None]).to(self.out_dtype)
                     plan.append((c.key, keys, None, (bag, cnt)))
         self._last = plan
+        self._pending_backward = torch.is_grad_enabled()
         return out
 
     # ---- state one train step changes (GraphedTrainStep undoes its warm-up steps with these) -----------
@@ -204,9 +209,30 @@ class EmbeddingFeatures:
             self.scalars.copy_(scalars)
 
     def _lookup(self, ids, cols):
-        """(ids, row_base, rows) the gather kernels read for the columns `cols`; hash mode inserts new ids when
-        gradients are enabled (training)."""
-        return self.store.lookup(ids, cols, insert=torch.is_grad_enabled())
+        """(ids, row_base, rows) the gather kernels read for the columns `cols`; hash mode inserts new ids and counts
+        the shows of every id when gradients are enabled (training)."""
+        train = torch.is_grad_enabled()
+        lk = self.store.lookup(ids, cols, insert=train)
+        if train and self.idmap is not None:
+            self.idmap.count(lk[0])
+        return lk
+
+    def evict(self, threshold: Optional[float] = None, decay: float = 1.0):
+        """Hash mode: show = show * decay for every id, then drop the ids whose show is below `threshold` (default:
+        AdaGrad's feature_drop_show; with Adam it must be given).  Their rows are freed for new ids; an evicted id
+        reads as a zero vector until a training call sees it again.  Call it between steps: not while a training
+        forward waits for its backward (its sort keys hold row numbers)."""
+        if threshold is None:
+            if not isinstance(self.opt, AdaGrad):
+                raise ValueError("evict: with Adam the threshold must be given (AdaGrad defaults to feature_drop_show)")
+            threshold = self.opt.feature_drop_show
+        threshold, decay = check_evict_args(threshold, decay)
+        if self.idmap is None:
+            raise ValueError("evict needs id_map='hash' (mod-mode tables have no ids to drop)")
+        if self._pending_backward:
+            raise RuntimeError("evict called between a training forward and its backward")
+        self._last = None                          # the plan of an inference call names rows that may move
+        self.idmap.evict(threshold, decay)
 
     def backward(self, grads: Dict[str, torch.Tensor]):
         """Push d(loss)/d(output) of every column: segment-sum per touched row + optimizer update."""
@@ -240,3 +266,4 @@ class EmbeddingFeatures:
                 ops.segsum_adagrad(self.table, self.g2sum, g, ks, self.opt.learning_rate, self.opt.epsilon,
                                    self.opt.per_element)
         self._last = None
+        self._pending_backward = False

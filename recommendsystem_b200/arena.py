@@ -162,13 +162,17 @@ class Arena:
             rows.append(self.idmap.pending_rows(lookups))
         return torch.unique(torch.cat(rows)) if rows else torch.empty(0, dtype=torch.int64, device=self.dev)
 
+    def _undo_state(self):
+        """Per-row arrays a train step changes: the optimizer records and (hash mode) the show counts."""
+        return self.state if self.idmap is None else self.state + [self.idmap.show]
+
     def snapshot(self, rows: torch.Tensor):
-        """The weights and optimizer state of `rows`, and the id map's counters."""
-        return rows, [t[rows].clone() for t in self.state], None if self.idmap is None else self.idmap.snapshot()
+        """The weights, optimizer state and (hash mode) show counts of `rows`, and the id map's counters."""
+        return rows, [t[rows].clone() for t in self._undo_state()], None if self.idmap is None else self.idmap.snapshot()
 
     def restore(self, snap):
         rows, saved, idmap = snap
-        for t, v in zip(self.state, saved):
+        for t, v in zip(self._undo_state(), saved):
             t[rows] = v
         if idmap is not None:
             self.idmap.restore(idmap)

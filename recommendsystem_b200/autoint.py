@@ -24,6 +24,7 @@ import torch
 
 from . import cabi, ops
 from .arena import Arena
+from .idmap import check_evict_args
 
 
 class PhaseTimer:
@@ -266,6 +267,11 @@ class AutoIntTrainer:
         with torch.cuda.stream(self.side):
             ops.adam_advance(self.adam_scalars, c.beta1, c.beta2)
             self.adam_done.record(self.side)
+            if self.idmap is not None:
+                # hash mode: the show counts of the mapped rows, a branch off the map lookup (nothing in the step
+                # reads them; the forward only reads ids_rows) that joins the main stream at the end of the step
+                with ph("idmap_count"):
+                    self.idmap.count(self.ids_rows)
         if self.fused:
             # K1 inside K4: the forward's tile loader reads the embedding rows itself (local table, or the owners' HBM
             # over NVLink) and writes X and the sort keys as by-products; only the owners' key work (multi-GPU) is a
@@ -480,6 +486,15 @@ class AutoIntTrainer:
         else:
             ops.gemm(x, dy, self.G[wname], transA=True)
         ops.colsum(dy, out=self.G[bname])
+
+    def evict(self, threshold: float, decay: float = 1.0):
+        """Hash mode: show = show * decay for every id, then drop the ids whose show is below `threshold`; their rows
+        are freed for new ids (idmap.IdMap.evict).  Runs on the current stream between steps; the buffers stay where
+        they are, so a captured step remains valid."""
+        threshold, decay = check_evict_args(threshold, decay)
+        if self.idmap is None:
+            raise ValueError("evict needs id_map='hash' (mod-mode tables have no ids to drop)")
+        self.idmap.evict(threshold, decay)
 
     # --------------------------------------------------------------- frontends
     def step(self, ids: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:

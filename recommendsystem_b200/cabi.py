@@ -56,6 +56,10 @@ PROTOTYPES = {
                              _p, _i64, _i, _f, _p]),
     "rs_idmap_lookup": (_i, [_p, _p, _p, _i, _p, _i64, _i, _p, _p, _i, _p]),
     "rs_idmap_rebuild": (_i, [_p, _i64, _p, _p, _p, _i, _i64, _p]),
+    "rs_idmap_count": (_i, [_p, _p, _i64, _p]),
+    "rs_idmap_evict_workspace_bytes": (_sz, [_i64]),
+    "rs_idmap_evict": (_i, [_p, _i64, _p, _p, _p, _i, _i64, _p, _f, _f, _p, _i64, _i, _p, _i64, _i, _p, _i64, _i, _p,
+                            _p, _sz, _p]),
     "rs_interacting_workspace_bytes": (_sz, [_i, _i, _i, _i]),
     "rs_interacting_saved_bytes": (_sz, [_i, _i, _i, _i]),
     "rs_interacting_path": (_i, [_i, _i, _i, _i, _i, _i, _f]),

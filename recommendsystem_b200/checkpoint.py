@@ -9,9 +9,11 @@ sub-model whose Keras weight names are the serving contract (`rank/multi_head/au
     dense.npz                      fp32 master weights by name, `m/<name>`, `v/<name>`, `adam_scalars`
     tables.rank<r>of<W>.bin        that rank's arena as it lies in HBM: [n_local, 3, d] fp32 records
                                    [w | m | v] (DESIGN.md §2), field f at rows local_base[f]...
-    idmap.npz                      id_map="hash" trainers only (meta.json "id_map": "hash"): the ids owning the used
-                                   rows of every field (`key_of_row`, field after field), `rows_used`, `overflow`,
-                                   `rows_per_field`; loading copies the arena and rebuilds the map from it
+    idmap.npz                      id_map="hash" trainers only (meta.json "id_map": "hash"): the ids owning the live
+                                   rows of every field and their show counts (`key_of_row`, `show`, field after
+                                   field), `rows_used`, `overflow`, `evicted`, `rows_per_field`; loading copies the
+                                   arena and rebuilds the map from it (a file without `show` / `evicted`, written
+                                   before eviction existed, loads with zero shows and zero evictions)
 
 Every rank writes its own shard (device -> pinned host -> file in bounded chunks); rank 0 also
 writes meta.json and dense.npz (dense state is replicated).  Loading works for ANY world size:

@@ -9,6 +9,12 @@
 //   lookup  every lookup probes again (read-only) and emits its arena row, or -1 (padding, unseen, overflowed).
 // No thread waits for another: a probe loop ends after at most S_f slots, and a key found before its row is
 // written is simply left alone (the lookup pass, after the kernel boundary, reads the row).
+// Eviction (rs_idmap_evict) decays every live row's show count, drops the keys whose count falls below a threshold,
+// compacts each field's live rows back to the front of its range and rebuilds the slots from key_of_row.
+#include <cmath>
+
+#include <cub/device/device_scan.cuh>
+
 #include "common.cuh"
 
 namespace rs {
@@ -153,6 +159,103 @@ idmap_rebuild_kernel(IdSlot* __restrict__ slots, long long* __restrict__ key_of_
   }
 }
 
+// show[row] += 1 per training lookup that resolved to a row.  Every increment adds the same value, so the sum does not
+// depend on the order of the atomics (it stops growing at 2^24, where x + 1 rounds back to x).
+__global__ void __launch_bounds__(256)
+idmap_count_kernel(float* __restrict__ show, const int64_t* __restrict__ rows, int64_t n) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = rows[i];
+    if (r >= 0) atomicAdd(show + r, 1.f);
+  }
+}
+
+// ---- eviction: decay + mark, exclusive scan of the keep flags (pos), hole list, moves, counters, rebuild.
+// Field f (blockIdx.y) has used_f live rows [0, used_f) before and live_f = kept rows after; the k-th dropped row
+// below live_f (a hole) receives the k-th kept row at or above live_f (a mover), both in ascending order.  Holes lie
+// below live_f and movers at or above it, so no record is read after it is written.
+__global__ void __launch_bounds__(256)
+idmap_evict_mark_kernel(float* __restrict__ show, const long long* __restrict__ counters,
+                        const int64_t* __restrict__ geom, float threshold, float decay, int* __restrict__ keep,
+                        int64_t total_rows) {
+  const int f = blockIdx.y;
+  const FieldGeom g = field_geom(geom, f);
+  const long long used = min(counters[f], g.cap);
+  if (f == 0 && blockIdx.x == 0 && threadIdx.x == 0) keep[total_rows] = 0;    // pos[total_rows] = rows kept in all
+  for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < g.cap; j += (long long)gridDim.x * blockDim.x) {
+    const int64_t row = g.row_base + j;
+    int k = 0;
+    if (j < used) {
+      const float s = __fmul_rn(show[row], decay);
+      show[row] = s;
+      k = !(s < threshold);
+    }
+    keep[row] = k;
+  }
+}
+
+__global__ void __launch_bounds__(256)
+idmap_evict_holes_kernel(const int* __restrict__ pos, const int64_t* __restrict__ geom, int* __restrict__ hole_row) {
+  const int f = blockIdx.y;
+  const FieldGeom g = field_geom(geom, f);
+  const int k0 = pos[g.row_base];
+  const long long live = pos[g.row_base + g.cap] - k0;
+  for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < live; j += (long long)gridDim.x * blockDim.x) {
+    const int64_t row = g.row_base + j;
+    if (pos[row + 1] == pos[row])                                   // dropped: hole number j - (kept rows below j)
+      hole_row[g.row_base + (j - (pos[row] - k0))] = (int)j;
+  }
+}
+
+struct MoveArgs {
+  float* w; int64_t w_ld; int d;
+  float* s[2]; int64_t s_ld[2]; int s_width[2];
+};
+
+__global__ void __launch_bounds__(256)
+idmap_evict_move_kernel(const int* __restrict__ pos, const int* __restrict__ hole_row,
+                        const long long* __restrict__ counters, const int64_t* __restrict__ geom,
+                        long long* __restrict__ key_of_row, float* __restrict__ show, MoveArgs a) {
+  const int f = blockIdx.y;
+  const FieldGeom g = field_geom(geom, f);
+  const long long used = min(counters[f], g.cap);
+  const int k0 = pos[g.row_base];
+  const long long live = pos[g.row_base + g.cap] - k0;
+  const long long kept_below = pos[g.row_base + live] - k0;       // kept rows that stay where they are
+  for (long long j = live + (long long)blockIdx.x * blockDim.x + threadIdx.x; j < used;
+       j += (long long)gridDim.x * blockDim.x) {
+    const int64_t src = g.row_base + j;
+    if (pos[src + 1] != pos[src]) {                                 // kept: mover number (kept rows in [live, j))
+      const int64_t dst = g.row_base + hole_row[g.row_base + (pos[src] - k0 - kept_below)];
+      const float* ws = a.w + src * a.w_ld;
+      float* wd = a.w + dst * a.w_ld;
+      for (int k = 0; k < a.d; ++k) wd[k] = ws[k];
+#pragma unroll
+      for (int q = 0; q < 2; ++q) {
+        if (!a.s[q]) continue;
+        const float* ss = a.s[q] + src * a.s_ld[q];
+        float* sd = a.s[q] + dst * a.s_ld[q];
+        for (int k = 0; k < a.s_width[q]; ++k) sd[k] = ss[k];
+      }
+      show[dst] = show[src];
+      key_of_row[dst] = key_of_row[src];
+    }
+    show[src] = 0.f;                                                // vacated: owned by no key
+    key_of_row[src] = -1;
+  }
+}
+
+__global__ void idmap_evict_counters_kernel(const int* __restrict__ pos, long long* __restrict__ counters,
+                                            const int64_t* __restrict__ geom, int n_fields,
+                                            long long* __restrict__ evicted) {
+  for (int f = threadIdx.x; f < n_fields; f += blockDim.x) {
+    const FieldGeom g = field_geom(geom, f);
+    const long long used = min(counters[f], g.cap);
+    const long long live = pos[g.row_base + g.cap] - pos[g.row_base];
+    evicted[f] += used - live;
+    counters[f] = live;
+  }
+}
+
 static unsigned grid_for(int64_t n, int threads) {
   int64_t blocks = cdiv(n, threads);
   const int64_t cap = (int64_t)sm_count() * 32;
@@ -209,6 +312,72 @@ int rs_idmap_rebuild(void* slots, int64_t n_slots, int64_t* key_of_row, const in
   idmap_rebuild_kernel<<<dim3((unsigned)bx, (unsigned)n_fields), threads, 0, as_stream(stream)>>>(
       (IdSlot*)slots, (long long*)key_of_row, (const long long*)counters, geom);
   return check_launch("idmap_rebuild");
+}
+
+int rs_idmap_count(float* show, const int64_t* rows, int64_t n, void* stream) {
+  RS_REQUIRE(n >= 0 && (show || n == 0), "idmap_count: n=%lld", (long long)n);
+  if (n == 0) return 0;
+  const int threads = 256;
+  idmap_count_kernel<<<grid_for(n, threads), threads, 0, as_stream(stream)>>>(show, rows, n);
+  return check_launch("idmap_count");
+}
+
+static size_t evict_flags_bytes(int64_t total_rows) { return (size_t)cdiv((total_rows + 1) * 4, 256) * 256; }
+
+size_t rs_idmap_evict_workspace_bytes(int64_t total_rows) {
+  if (total_rows <= 0 || total_rows >= INT32_MAX) return 0;
+  size_t scan = 0;
+  cub::DeviceScan::ExclusiveSum((void*)nullptr, scan, (const int*)nullptr, (int*)nullptr, (int)(total_rows + 1),
+                                (cudaStream_t)0);
+  return 2 * evict_flags_bytes(total_rows) + scan + 256;
+}
+
+int rs_idmap_evict(void* slots, int64_t n_slots, int64_t* key_of_row, int64_t* counters, const int64_t* geom,
+                   int n_fields, int64_t total_rows, float* show, float threshold, float decay, float* w, int64_t w_ld,
+                   int d, float* s0, int64_t s0_ld, int s0_width, float* s1, int64_t s1_ld, int s1_width,
+                   int64_t* evicted, void* ws, size_t ws_bytes, void* stream) {
+  RS_REQUIRE(n_fields > 0 && n_fields <= 65535 && n_slots > 0 && total_rows > 0 && total_rows < INT32_MAX,
+             "idmap_evict: n_fields=%d n_slots=%lld total_rows=%lld", n_fields, (long long)n_slots,
+             (long long)total_rows);
+  RS_REQUIRE(decay > 0.f && decay <= 1.f && std::isfinite(threshold), "idmap_evict: decay=%g threshold=%g",
+             (double)decay, (double)threshold);
+  RS_REQUIRE(show && evicted && w && d > 0 && w_ld >= d, "idmap_evict: show / evicted / w / d=%d", d);
+  RS_REQUIRE((!s0 || (s0_width > 0 && s0_ld >= s0_width)) && (!s1 || (s1_width > 0 && s1_ld >= s1_width)),
+             "idmap_evict: optimizer state width / stride");
+  RS_REQUIRE(((uintptr_t)slots & 15) == 0 && ((uintptr_t)geom & 15) == 0 && ((uintptr_t)ws & 255) == 0,
+             "idmap_evict: slots / geom not 16-B aligned or workspace not 256-B aligned");
+  const size_t need = rs_idmap_evict_workspace_bytes(total_rows);
+  if (ws_bytes < need) {
+    set_error("idmap_evict: workspace %zu < %zu", ws_bytes, need);
+    return RS_ERR_WORKSPACE;
+  }
+  cudaStream_t st = as_stream(stream);
+  int* keep = (int*)ws;                                            // keep flags, then the hole list
+  int* pos = (int*)((char*)ws + evict_flags_bytes(total_rows));     // exclusive scan of the flags
+  void* scan_ws = (char*)ws + 2 * evict_flags_bytes(total_rows);
+  size_t scan_bytes = need - 2 * evict_flags_bytes(total_rows);
+  const int threads = 256;
+  int64_t bx = cdiv(total_rows, threads);
+  if (bx > 4096) bx = 4096;
+  const dim3 grid((unsigned)bx, (unsigned)n_fields);
+  idmap_evict_mark_kernel<<<grid, threads, 0, st>>>(show, (const long long*)counters, geom, threshold, decay, keep,
+                                                    total_rows);
+  if (int rc = check_launch("idmap_evict_mark")) return rc;
+  RS_CUDA(cub::DeviceScan::ExclusiveSum(scan_ws, scan_bytes, (const int*)keep, pos, (int)(total_rows + 1), st));
+  g_launches.fetch_add(2, std::memory_order_relaxed);
+  idmap_evict_holes_kernel<<<grid, threads, 0, st>>>(pos, geom, keep);
+  if (int rc = check_launch("idmap_evict_holes")) return rc;
+  MoveArgs ma{};
+  ma.w = w; ma.w_ld = w_ld; ma.d = d;
+  ma.s[0] = s0; ma.s_ld[0] = s0_ld; ma.s_width[0] = s0_width;
+  ma.s[1] = s1; ma.s_ld[1] = s1_ld; ma.s_width[1] = s1_width;
+  idmap_evict_move_kernel<<<grid, threads, 0, st>>>(pos, keep, (const long long*)counters, geom,
+                                                    (long long*)key_of_row, show, ma);
+  if (int rc = check_launch("idmap_evict_move")) return rc;
+  idmap_evict_counters_kernel<<<1, 256, 0, st>>>(pos, (long long*)counters, geom, n_fields, (long long*)evicted);
+  if (int rc = check_launch("idmap_evict_counters")) return rc;
+  // (the rebuild kernel grid-strides over a field's rows, so total_rows serves as its max_rows)
+  return rs_idmap_rebuild(slots, n_slots, key_of_row, counters, geom, n_fields, total_rows, stream);
 }
 
 }  // extern "C"

@@ -217,6 +217,30 @@ def idmap_rebuild(slots, key_of_row, counters, geom, max_rows):
          geom.shape[0], int(max_rows), _stream())
 
 
+def idmap_count(show, rows):
+    """rs_idmap_count: show[r] += 1 for every row r >= 0 of `rows` (int64, any shape)."""
+    _need(rows.dtype == torch.int64 and rows.is_contiguous(), "rows must be contiguous int64")
+    _need(show.dtype == torch.float32 and show.is_contiguous(), "show must be contiguous fp32")
+    call("rs_idmap_count", _ptr(show), _ptr(rows), rows.numel(), _stream())
+
+
+def idmap_evict(slots, key_of_row, counters, geom, show, evicted, threshold, decay, w, states=()):
+    """rs_idmap_evict: decay the live rows' show, drop the keys below `threshold`, compact every field's live rows
+    (w and the `states` views move with them, the arguments of idmap_insert), rebuild the slots."""
+    _need(w.dtype == torch.float32 and w.dim() == 2 and w.stride(1) == 1, "w must be fp32 [R, d] with contiguous rows")
+    st = []
+    for t in states:
+        _need(t.dtype == torch.float32 and (t.dim() == 1 or t.stride(1) == 1), "optimizer state: fp32, contiguous rows")
+        st += [_ptr(t), t.stride(0), 1 if t.dim() == 1 else t.shape[1]]
+    st += [None, 0, 0] * (2 - len(states))
+    total = key_of_row.numel()
+    nbytes = cabi.load().rs_idmap_evict_workspace_bytes(total)
+    ws = torch.empty(int(nbytes), dtype=torch.uint8, device=show.device)
+    call("rs_idmap_evict", _ptr(slots), slots.numel() // 2, _ptr(key_of_row), _ptr(counters), _ptr(geom),
+         geom.shape[0], total, _ptr(show), float(threshold), float(decay), _ptr(w), w.stride(0), w.shape[1], *st,
+         _ptr(evicted), _ptr(ws), ws.numel(), _stream())
+
+
 def permute_rows(src, index, scatter=False, out=None):
     n, d = index.numel(), src.shape[-1]
     out = torch.empty(n, d, dtype=src.dtype, device=src.device) if out is None else out

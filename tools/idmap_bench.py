@@ -4,13 +4,17 @@ B = 8192, bf16 AutoInt.  Prints one JSON line:
   map       insert and lookup pass times (CUDA events around CUDA-graph replays of each pass, mean over batches) in
             three states: first touch (every key of the batch is new), steady (every key already mapped) and Zipf(1.05)
             ids over the same pool (mostly hits, some new keys);
-  step      AutoInt train-step time in mod and hash mode, both captured, alternated in rounds in this one process;
+  step      AutoInt train-step time in mod and hash mode, both captured, alternated in rounds in this one process
+            (the hash step includes the show count, a branch off the map lookup);
+  evict     IdMap.evict on a full map (every row of the 39 x 1 M owned, Adam [w|m|v] records) with about half the
+            keys dropped: random shows in [0, 1), threshold 0.5, decay 0.9 (CUDA events; the map is refilled with
+            the same keys and the shows redrawn before each round);
   gpu       card name and power limit (nvidia-smi), which every number above depends on.
 
 Ids are 63-bit signs drawn from a per-field pool of 1 M random keys (uniform, or Zipf(1.05) by rank as bench.py
 --ids zipf).  The map's slots (1.25 GB) and the arenas (7.5 GB each) are far larger than the 126 MB L2.
 
-    python tools/idmap_bench.py [--batches 48] [--steps 100] [--rounds 5]
+    python tools/idmap_bench.py [--batches 48] [--steps 100] [--rounds 5] [--evict-rounds 3]
 """
 from __future__ import annotations
 
@@ -44,6 +48,7 @@ def main():
     ap.add_argument("--steps", type=int, default=100, help="train steps per round and mode")
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--warm-steps", type=int, default=500, help="hash-trainer steps before timing (fills the map)")
+    ap.add_argument("--evict-rounds", type=int, default=3)
     args = ap.parse_args()
 
     import numpy as np
@@ -151,8 +156,31 @@ def main():
     step["hash_over_mod"] = step["hash"]["ms_median"] / step["mod"]["ms_median"] - 1.0
     step["hash_rows_used"] = int(sum(st["rows_used"]))
     step["hash_overflow"] = int(sum(st["overflow"]))
+    del trs
+    torch.cuda.empty_cache()
+
+    # ---------------------------------------------------------------- evict on a full map
+    arena = torch.zeros(F * ROWS, 3, 16, device=dev)
+    m = IdMap([ROWS] * F, dev, 1, 0.1, arena[:, 0, :], [(arena[:, 1, :], 0.0), (arena[:, 2, :], 0.0)])
+    fill = pool.t().contiguous()                                  # [1 M, F]: every pool key of every field
+    ev = {"ms": [], "dropped": []}
+    for _ in range(args.evict_rounds + 1):                        # the first round warms up (workspace, cub)
+        m.resolve(fill, m.fields(range(F)), insert=True)
+        assert int(m.counters[0].sum()) == F * ROWS, "the map is not full"
+        m.show.uniform_(0.0, 1.0, generator=g)
+        before = int(m.evicted.sum())
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        m.evict(0.5, 0.9)
+        e1.record()
+        e1.synchronize()
+        ev["ms"].append(e0.elapsed_time(e1))
+        ev["dropped"].append(int(m.evicted.sum()) - before)
+    ev = {"ms_median": float(np.median(ev["ms"][1:])), "ms_rounds": [round(x, 3) for x in ev["ms"][1:]],
+          "dropped_rounds": ev["dropped"][1:], "rows": F * ROWS}
     print(json.dumps({"bench": "idmap", "fields": F, "rows_per_field": ROWS, "batch": B, "dtype": "bf16",
-                      "map": res_map, "step": step, "gpu": gpu_info(),
+                      "map": res_map, "step": step, "evict": ev, "gpu": gpu_info(),
                       "note": "step times include the ids/labels device copies of each step (both modes)"}))
 
 
