@@ -185,14 +185,19 @@ class _AutoIntFullModel:
         embs = self.emb(inputs)
         leaves = [embs[s].detach().requires_grad_(True) for s in self.slots]
         pred = self.sub_model(leaves)
-        if self.opt is None:
-            self.opt = DenseAdam(self.sub_model.parameters(), lr=1e-5, beta1=0.9, beta2=0.999, eps=1e-8, group=self.group)
+        opt = self.dense_optimizer()
         loss = cross_entropy(labels, pred).mean()
-        self.opt.zero_grad()
+        opt.zero_grad()
         loss.backward()
-        self.opt.step()
+        opt.step()
         self.emb.backward({s: l.grad for s, l in zip(self.slots, leaves)})
         return loss.detach(), pred.detach()
+
+    def dense_optimizer(self):
+        """The dense Adam of sub_model (lr 1e-5), created at the first call: the lazily-built layers must exist."""
+        if self.opt is None:
+            self.opt = DenseAdam(self.sub_model.parameters(), lr=1e-5, beta1=0.9, beta2=0.999, eps=1e-8, group=self.group)
+        return self.opt
 
     # the InteractingLayer's device-side dropout counter is part of what a step changes (api.graph warm-up undo)
     def extra_state_snapshot(self):

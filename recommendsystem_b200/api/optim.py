@@ -46,6 +46,7 @@ class DenseAdam:
                 view.copy_(p.data)
                 p.data = view
                 p.grad = self.flat_g[o:o + p.numel()].view(p.shape)
+        self.offsets = offs
         self.group = group            # torch.distributed group: gradients are averaged over its ranks
 
     def zero_grad(self):
@@ -64,6 +65,12 @@ class DenseAdam:
         ops.adam_advance(self.scalars, self.beta1, self.beta2)
         ops.dense_adam(self.flat, self.flat_m, self.flat_v, self.flat_g, self.lr, self.beta1, self.beta2, self.eps,
                        self.scalars, None)
+
+    def moments(self):
+        """(parameter, m, v) of every parameter: views of the flat moment buffers shaped like the parameter."""
+        for p, o in zip(self.params, self.offsets):
+            k = p.numel()
+            yield p, self.flat_m[o:o + k].view(p.shape), self.flat_v[o:o + k].view(p.shape)
 
     # state that one step changes (GraphedTrainStep undoes its warm-up with these)
     def snapshot(self):

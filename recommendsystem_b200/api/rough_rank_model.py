@@ -187,15 +187,20 @@ class DssmNet:
         e = self.emb({k: v for k, v in inputs.items() if k != C.DENSE_MASK_ID})
         leaves = {k: v.detach().requires_grad_(True) for k, v in e.items()}
         out = self.sub_model(leaves, inputs[C.DENSE_MASK_ID].to(self.emb.dev))
-        if self.opt is None:
-            self.opt = DenseAdam(self.sub_model.parameters(), lr=0.0001, beta1=0.9, beta2=0.999, eps=1e-8, group=getattr(self, 'group', None))
+        opt = self.dense_optimizer()
         loss = (binary_crossentropy(labels["student"], out["student"]) +
                 binary_crossentropy(labels["teacher"], out["teacher"]) + y_pred_loss(None, out["distill"]))
-        self.opt.zero_grad()
+        opt.zero_grad()
         loss.backward()
-        self.opt.step()
+        opt.step()
         self.emb.backward({k: v.grad for k, v in leaves.items()})
         return loss.detach(), {k: v.detach() for k, v in out.items()}
+
+    def dense_optimizer(self):
+        """The dense Adam of sub_model (lr 1e-4), created at the first call: the lazily-built layers must exist."""
+        if self.opt is None:
+            self.opt = DenseAdam(self.sub_model.parameters(), lr=0.0001, beta1=0.9, beta2=0.999, eps=1e-8, group=getattr(self, 'group', None))
+        return self.opt
 
 
 def DSSM(**kw):

@@ -137,6 +137,7 @@ class ShardedEmbeddingFeatures(EmbeddingFeatures):
                 out[c.key] = (emb.view(B, bag, self.d).sum(1) / cnt[:, None]).to(self.out_dtype)
                 plan.append((c.key, g, (bag, cnt)))
         self._last = plan
+        self._pending_backward = torch.is_grad_enabled()
         return out
 
     def _barrier(self):
@@ -172,6 +173,7 @@ class ShardedEmbeddingFeatures(EmbeddingFeatures):
                                    self.opt.epsilon, self.opt.per_element, grad_scale=scale)
         self._barrier()                                          # every owner's update precedes the next peer reads
         self._last = None
+        self._pending_backward = False
 
     def check_overflow(self):
         if int(self.overflow.item()) != 0:

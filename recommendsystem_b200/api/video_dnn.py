@@ -248,12 +248,11 @@ class MtlNet:
         le = embs.detach().requires_grad_(True) if stacked else {s: v.detach().requires_grad_(True) for s, v in embs.items()}
         ls = {s: (v[0].detach().requires_grad_(True), v[1]) for s, v in seqs.items()}
         out, _ = self.sub_model(le, ls)
-        if self.opt is None:
-            self.opt = DenseAdam(self.sub_model.parameters(), lr=0.0005, beta1=0.9, beta2=0.999, eps=1e-8, group=getattr(self, 'group', None))
+        opt = self.dense_optimizer()
         loss = sum(LOSS_WEIGHTS[k] * LOSSES[k](labels[k], out[k]).mean() for k in TASK_KEYS)
-        self.opt.zero_grad()
+        opt.zero_grad()
         loss.backward()
-        self.opt.step()
+        opt.step()
         if stacked:
             grads = {"emb_col_%s" % s: le.grad[:, i, :] for i, s in enumerate(sorted(self.slots))}
         else:
@@ -261,6 +260,12 @@ class MtlNet:
         grads.update({"emb_col_seq_%s" % s: v[0].grad for s, v in ls.items()})
         self.emb.backward(grads)
         return loss.detach(), {k: v.detach() for k, v in out.items()}
+
+    def dense_optimizer(self):
+        """The dense Adam of sub_model (lr 5e-4), created at the first call: the lazily-built layers must exist."""
+        if self.opt is None:
+            self.opt = DenseAdam(self.sub_model.parameters(), lr=0.0005, beta1=0.9, beta2=0.999, eps=1e-8, group=getattr(self, 'group', None))
+        return self.opt
 
 
 def mtl_net(slots, seq_slots, seq_max_len, dnn_hidden_units=(64, 32), **kw):

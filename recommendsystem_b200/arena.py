@@ -7,6 +7,8 @@ This module is the only code that knows the arena's layout (DESIGN.md §2):
                  each rank holding ceil(R_f / W) rows of every field (shard_layout); W = 1 is the unsharded arena
     storage      Adam: one [w | m | v] record of 3d floats per row (the sparse update touches ONE contiguous block
                  per row); AdaGrad: w [n, d] and g2sum [n] or [n, d]
+    record       a checkpoint's fp32 row (pack / unpack): Adam [w | m | v] (3d), AdaGrad [w | g2sum] (d + 1 per row,
+                 2d per element)
     hash mode    (recommendsystem_b200.idmap, one rank only) ids are first mapped to rows, which the kernels read
                  through the identity geometry (row_base 0, rows = total rows)
 The arena issues no collective: the sharded classes gather the ids of every rank before asking it for touched rows.
@@ -87,6 +89,7 @@ class Arena:
             states = [(self.g2sum, g2sum0)]
         self.ld = self.w.stride(0)
         self.state = [self.records] if adagrad is None else [self.w, self.g2sum]     # what an update changes per row
+        self.record_floats = sum(int(np.prod(t.shape[1:])) for t in self.state)
         self.idmap = IdMap(self.rows, self.dev, seed, scale, self.w, states) if id_map == "hash" else None
         all_cols = tuple(range(len(self.rows)))
         self._geom = {} if self.idmap is not None else {all_cols: (self.lbase_t, self.rows_t)}
@@ -161,6 +164,19 @@ class Arena:
         if self.idmap is not None:
             rows.append(self.idmap.pending_rows(lookups))
         return torch.unique(torch.cat(rows)) if rows else torch.empty(0, dtype=torch.int64, device=self.dev)
+
+    # ---- fp32 per-row records (checkpoints)
+    def pack(self, rows) -> torch.Tensor:
+        """[n, record_floats] fp32 records of `rows` (a slice or an int64 index tensor): Adam [w | m | v] (3d floats,
+        the `records` array itself), AdaGrad [w | g2sum] (d + 1 floats per row, 2d per element)."""
+        return torch.cat([t[rows].reshape(-1, int(np.prod(t.shape[1:]))) for t in self.state], 1)
+
+    def unpack(self, rows, rec: torch.Tensor) -> None:
+        """Inverse of pack: copy the records `rec` [n, record_floats] into `rows`, in place (captured CUDA graphs and
+        peer mappings of the arena stay valid)."""
+        widths = [int(np.prod(t.shape[1:])) for t in self.state]
+        for t, part in zip(self.state, torch.split(rec.to(self.dev, torch.float32), widths, dim=1)):
+            t[rows] = part.reshape((-1,) + tuple(t.shape[1:]))
 
     def _undo_state(self):
         """Per-row arrays a train step changes: the optimizer records and (hash mode) the show counts."""

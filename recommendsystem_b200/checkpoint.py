@@ -3,15 +3,32 @@
 The reference delegates persistence to TensorNet (`model.save_weights` on every shard; sparse
 tables and their optimizer state live on the parameter shards) and exposes the dense part as a
 sub-model whose Keras weight names are the serving contract (`rank/multi_head/autoint:53-54`,
-`rough_rank/model.py:62-63`, `staytime/VideoDnn.py:193-215`).  Here a checkpoint is a directory:
+`rough_rank/model.py:62-63`, `staytime/VideoDnn.py:193-215`).
 
-    meta.json                      format, config, world size, rows per field, dense spec, step
-    dense.npz                      fp32 master weights by name, `m/<name>`, `v/<name>`, `adam_scalars`
-    tables.rank<r>of<W>.bin        that rank's arena as it lies in HBM: [n_local, 3, d] fp32 records
-                                   [w | m | v] (DESIGN.md §2), field f at rows local_base[f]...
-    idmap.npz                      id_map="hash" trainers only (meta.json "id_map": "hash"): the ids owning the live
-                                   rows of every field and their show counts (`key_of_row`, `show`, field after
-                                   field), `rows_used`, `overflow`, `evicted`, `rows_per_field`; loading copies the
+Two kinds of object are saved and loaded:
+  * an AutoIntTrainer / ShardedAutoIntTrainer (`arena`, `spec`, `flat`, `flat_m`, ...);
+  * a composed net: any object with `emb` (api.embedding.EmbeddingFeatures or api.sharded_embedding.
+    ShardedEmbeddingFeatures), `sub_model` (an nn.Module) and optionally `opt` (api.optim.DenseAdam, created through
+    the net's `dense_optimizer()` when a load finds none) - MtlNet, DssmNet, RankCtrNet, the AUTOINT model, or a
+    user's net that follows the same protocol as api.graph.GraphedTrainStep.
+
+A checkpoint is a directory:
+
+    meta.json                      format, world size, rows per field, dense spec, step; trainer: its config; net:
+                                   model class, columns (key, bucket_size), embed_dim, sparse optimizer
+                                   (adam | adagrad, per_element), record_floats, id_map (hash mode: id_map_seed,
+                                   id_map_scale, which a load must match)
+    dense.npz                      fp32 master weights by name, `m/<name>`, `v/<name>`, `adam_scalars`; net: the
+                                   sub_model.state_dict() entries, the moments of the parameters DenseAdam owns,
+                                   `sparse_scalars` (sparse Adam step scalars) and `dropout/<module path>` = [host
+                                   call count, device call count] of every layer with a dropout counter
+    tables.rank<r>of<W>.bin        that rank's arena as it lies in HBM: fp32 records, field f at rows local_base[f]...
+                                   trainer [n_local, 3, d] = [w | m | v] (DESIGN.md §2); net [n_local, record_floats]
+                                   from arena.Arena.pack: Adam [w | m | v] (3d), AdaGrad [w | g2sum] (d + 1 per row,
+                                   2d per element)
+    idmap.npz                      id_map="hash" trainers and nets only (meta.json "id_map": "hash"): the ids
+                                   owning the live rows of every field and their show counts (`key_of_row`, `show`,
+                                   field after field), `rows_used`, `overflow`, `evicted`, `rows_per_field`; loading copies the
                                    arena and rebuilds the map from it (a file without `show` / `evicted`, written
                                    before eviction existed, loads with zero shows and zero evictions)
 
@@ -19,9 +36,11 @@ Every rank writes its own shard (device -> pinned host -> file in bounded chunks
 writes meta.json and dense.npz (dense state is replicated).  Loading works for ANY world size:
 global row g of a field lives in shard g % W at local row g // W (`arena.shard_layout`), so a
 rank of a W'-way job collects the rows g = r', r'+W', ... from whichever old shards hold them.
-State is copied INTO the trainer's existing buffers: captured CUDA graphs and peer (IPC) mappings
-stay valid.  Resuming is exact: train(2) -> save -> load -> train(2) equals train(4) bit for bit
-(tests/test_gpu_checkpoint.py).
+State is copied INTO the model's existing buffers: captured CUDA graphs (AutoIntTrainer.capture, a
+GraphedTrainStep captured before the load) and peer (IPC) mappings stay valid.  Resuming is exact: train(2) -> save
+-> load -> train(2) equals train(4) bit for bit (tests/test_gpu_checkpoint.py, tests/test_gpu_net_checkpoint.py).
+A net is loaded after its lazily-built layers exist (one `predict`); a save between a training forward and its
+backward raises RuntimeError.
 """
 from __future__ import annotations
 
@@ -46,7 +65,8 @@ def shard_path(directory, rank: int, world: int) -> Path:
 
 
 def write_shard(path, chunks: Iterator[np.ndarray]) -> int:
-    """Append the chunks ([n, 3, d] fp32, C-contiguous) to `path`; returns the rows written."""
+    """Append the chunks (fp32 records of any width, [n, 3, d] for the trainer, [n, record_floats] for a net) to
+    `path`; returns the rows written."""
     n = 0
     tmp = str(path) + ".tmp"
     with open(tmp, "wb") as f:
@@ -60,7 +80,7 @@ def write_shard(path, chunks: Iterator[np.ndarray]) -> int:
 
 def reshard_plan(rows_per_field, old_world: int, new_world: int, new_rank: int, chunk_rows: int = CHUNK_ROWS):
     """Yield (old_rank, src_rows, dst_rows): int64 index arrays saying which local rows of old shard
-    `old_rank` become which local rows of rank `new_rank` in a `new_world`-way job."""
+    `old_rank` become which local rows of rank `new_rank` in a `new_world`-way job (whole records: any width)."""
     rows = np.asarray(rows_per_field, np.int64)
     _, old_base = shard_rows(rows, old_world)
     _, new_base = shard_rows(rows, new_world)
@@ -77,14 +97,16 @@ def reshard_plan(rows_per_field, old_world: int, new_world: int, new_rank: int, 
 
 
 def load_shard_rows(directory, meta: dict, new_world: int, new_rank: int, chunk_rows: int = CHUNK_ROWS):
-    """Yield (dst_rows int64[n], records float32[n, 3, d]) for rank `new_rank` of a `new_world`-way job."""
+    """Yield (dst_rows int64[n], records) for rank `new_rank` of a `new_world`-way job: records float32
+    [n, record_floats] when meta.json names `record_floats` (a net's checkpoint), else the trainer's [n, 3, d]."""
     d, W = int(meta["embed_dim"]), int(meta["world"])
+    rec_shape = (int(meta["record_floats"]),) if "record_floats" in meta else (3, d)
     maps = {}
     for s, src, dst in reshard_plan(meta["rows_per_field"], W, new_world, new_rank, chunk_rows):
         if s not in maps:
             p = shard_path(directory, s, W)
-            n = os.path.getsize(p) // (3 * d * 4)
-            maps[s] = np.memmap(p, dtype=np.float32, mode="r", shape=(n, 3, d))
+            n = os.path.getsize(p) // (int(np.prod(rec_shape)) * 4)
+            maps[s] = np.memmap(p, dtype=np.float32, mode="r", shape=(n,) + rec_shape)
         if src.size and (np.diff(src) == 1).all():
             rec = np.asarray(maps[s][int(src[0]): int(src[-1]) + 1])
         elif src.size > 1 and (np.diff(src) == (src[1] - src[0])).all():
@@ -111,9 +133,24 @@ def _id_map(trainer) -> str:
     return "hash" if getattr(trainer, "idmap", None) is not None else "mod"
 
 
-def save_checkpoint(trainer, directory, step: int | None = None) -> Path:
-    """Write `trainer`'s tables, sparse-Adam state, dense weights and dense-Adam state.  Collective
-    for a ShardedAutoIntTrainer: every rank calls it; the caller barriers before reading."""
+def save_checkpoint(obj, directory, step: int | None = None) -> Path:
+    """Write the tables, sparse-optimizer state, dense weights and dense-Adam state of `obj`: an (Sharded)AutoIntTrainer
+    or a composed net (an object with `emb` and `sub_model`, see the module docstring).  Collective when the tables
+    are row-sharded: every rank calls it; the caller barriers before reading."""
+    if _is_net(obj):
+        return _save_net(obj, directory, step)
+    return _save_trainer(obj, directory, step)
+
+
+def load_checkpoint(obj, directory, tables: bool = True, dense: bool = True) -> dict:
+    """Restore `obj` (a trainer or a composed net) in place from `directory` (any world size); returns meta.json.
+    Raises ValueError when the checkpoint was written by another kind of model or its geometry differs."""
+    if _is_net(obj):
+        return _load_net(obj, directory, tables, dense)
+    return _load_trainer(obj, directory, tables, dense)
+
+
+def _save_trainer(trainer, directory, step: int | None = None) -> Path:
     directory = Path(directory)
     directory.mkdir(parents=True, exist_ok=True)
     W, r = _world_rank(trainer)
@@ -131,11 +168,7 @@ def save_checkpoint(trainer, directory, step: int | None = None) -> Path:
 
     write_shard(shard_path(directory, r, W), chunks())
     if r == 0:
-        # a reused directory may hold table shards of an earlier save at another world size: remove them so
-        # that the directory only ever describes ONE checkpoint (meta.json names the world size that counts)
-        for stale in directory.glob("tables.rank*of*.bin"):
-            if not stale.name.endswith(f"of{W}.bin"):
-                stale.unlink()
+        _remove_stale_shards(directory, W)
         dense = {}
         for name, shape, off in trainer.spec:
             k = int(np.prod(shape))
@@ -144,10 +177,7 @@ def save_checkpoint(trainer, directory, step: int | None = None) -> Path:
             dense["v/" + name] = trainer.flat_v[off:off + k].view(shape).cpu().numpy()
         dense["adam_scalars"] = trainer.adam_scalars.cpu().numpy()
         np.savez(directory / "dense.npz", **dense)
-        if _id_map(trainer) == "hash":
-            np.savez(directory / "idmap.npz", **trainer.idmap.state())
-        elif (directory / "idmap.npz").exists():           # left by an earlier hash-mode save into this directory
-            (directory / "idmap.npz").unlink()
+        _save_idmap(directory, trainer.idmap if _id_map(trainer) == "hash" else None)
         meta = {
             "format": FORMAT, "world": W, "embed_dim": int(d),
             "rows_per_field": [int(x) for x in trainer.rows_host],
@@ -157,10 +187,29 @@ def save_checkpoint(trainer, directory, step: int | None = None) -> Path:
         }
         if _id_map(trainer) == "hash":
             meta["id_map"] = "hash"
-        tmp = directory / "meta.json.tmp"
-        tmp.write_text(json.dumps(meta, indent=1))
-        os.replace(tmp, directory / "meta.json")
+        _write_meta(directory, meta)
     return directory
+
+
+def _remove_stale_shards(directory: Path, world: int):
+    # a reused directory may hold table shards of an earlier save at another world size: remove them so
+    # that the directory only ever describes ONE checkpoint (meta.json names the world size that counts)
+    for stale in directory.glob("tables.rank*of*.bin"):
+        if not stale.name.endswith(f"of{world}.bin"):
+            stale.unlink()
+
+
+def _save_idmap(directory: Path, idmap):
+    if idmap is not None:
+        np.savez(directory / "idmap.npz", **idmap.state())
+    elif (directory / "idmap.npz").exists():               # left by an earlier hash-mode save into this directory
+        (directory / "idmap.npz").unlink()
+
+
+def _write_meta(directory: Path, meta: dict):
+    tmp = directory / "meta.json.tmp"
+    tmp.write_text(json.dumps(meta, indent=1))
+    os.replace(tmp, directory / "meta.json")
 
 
 def read_meta(directory) -> dict:
@@ -170,12 +219,12 @@ def read_meta(directory) -> dict:
     return meta
 
 
-def load_checkpoint(trainer, directory, tables: bool = True, dense: bool = True) -> dict:
-    """Restore `trainer` in place from `directory` (any world size).  Raises ValueError when the
-    table geometry or the dense parameter shapes differ."""
+def _load_trainer(trainer, directory, tables: bool = True, dense: bool = True) -> dict:
     directory = Path(directory)
     meta = read_meta(directory)
     W, r = _world_rank(trainer)
+    if "model" in meta:
+        raise ValueError(f"{directory}: a checkpoint of a {meta['model']} net, not of an AutoInt trainer")
     if meta.get("id_map", "mod") != _id_map(trainer):
         raise ValueError(f"checkpoint id_map={meta.get('id_map', 'mod')!r} does not match the trainer's "
                          f"id_map={_id_map(trainer)!r}")
@@ -219,6 +268,157 @@ def _refresh_dense_shadows(trainer):
         trainer.flat_bf16.copy_(trainer.flat)
     if hasattr(trainer, "WT16"):                 # bf16 activations: transposed bf16 weight shadows
         trainer._refresh_wt()
+
+
+# ------------------------------------------------------------------ composed nets (emb + sub_model [+ opt])
+def _is_net(obj) -> bool:
+    return hasattr(obj, "emb") and hasattr(obj, "sub_model")
+
+
+def _net_geometry(net) -> dict:
+    """What a net's checkpoint must agree with to load: model class, columns, record layout, id map and, in hash mode,
+    the init rule of the rows the map hands out after the load (N(0, scale) from the seed)."""
+    emb, store = net.emb, net.emb.store
+    geom = {"model": type(net).__name__,
+            "columns": [[c.key, int(c.categorical_column.bucket_size)] for c in emb.cols],
+            "embed_dim": int(emb.d),
+            "sparse_optimizer": "adam" if store.g2sum is None else "adagrad",
+            "per_element": store.g2sum is not None and store.g2sum.dim() == 2,
+            "record_floats": int(store.record_floats),
+            "id_map": "hash" if store.idmap is not None else "mod"}
+    if store.idmap is not None:
+        # the seed and scale are launch arguments of the insert kernel (frozen into captured graphs): a load cannot
+        # change them in place, so a net that would initialise new ids differently is refused
+        geom["id_map_seed"], geom["id_map_scale"] = int(store.idmap.seed), float(store.idmap.scale)
+    return geom
+
+
+def _dense_spec(net):
+    return [[k, list(v.shape)] for k, v in net.sub_model.state_dict().items()]
+
+
+def _unbuilt_layers(module):
+    """Paths of lazily-built layers (Keras `build` at the first call) that have no parameters yet."""
+    return [p for p, m in module.named_modules()
+            if getattr(m, "built", True) is False or (hasattr(m, "kernel") and m.kernel is None)]
+
+
+def _dropout_layers(module):
+    """(path, layer) of every layer with a dropout call counter (InteractingLayer: `_drop_step` on the device,
+    `_dropout_calls` its host mirror)."""
+    return [(p, m) for p, m in module.named_modules() if hasattr(m, "_drop_step")]
+
+
+def _dense_opt(net, create: bool):
+    """The net's DenseAdam; `create` builds it through the net's dense_optimizer() when it does not exist yet."""
+    opt = net.dense_optimizer() if create and hasattr(net, "dense_optimizer") else getattr(net, "opt", None)
+    if opt is not None and not hasattr(opt, "moments"):
+        raise TypeError(f"checkpoints hold the dense state of api.optim.DenseAdam, not of {type(opt).__name__}")
+    return opt
+
+
+def _save_net(net, directory, step):
+    directory = Path(directory)
+    emb, store = net.emb, net.emb.store
+    if getattr(emb, "_pending_backward", False):
+        raise RuntimeError("save_checkpoint called between a training forward and its backward")
+    directory.mkdir(parents=True, exist_ok=True)
+    W, r = _world_rank(emb)
+    torch.cuda.synchronize(emb.dev)
+    n, rf = store.n_local, store.record_floats
+    stage = torch.empty(min(n, CHUNK_ROWS), rf, dtype=torch.float32, pin_memory=True)
+
+    def chunks():
+        for r0 in range(0, n, CHUNK_ROWS):
+            r1 = min(n, r0 + CHUNK_ROWS)
+            stage[: r1 - r0].copy_(store.pack(slice(r0, r1)))
+            torch.cuda.synchronize(emb.dev)
+            yield stage[: r1 - r0].numpy()
+
+    write_shard(shard_path(directory, r, W), chunks())
+    if r == 0:
+        _remove_stale_shards(directory, W)
+        sub = net.sub_model
+        dense = {k: v.detach().cpu().numpy() for k, v in sub.state_dict().items()}
+        names = {id(p): k for k, p in sub.named_parameters()}
+        opt = _dense_opt(net, create=False)
+        if opt is None:                                  # not trained yet: the state a new DenseAdam starts from
+            for k, p in sub.named_parameters():
+                if p.requires_grad:
+                    dense["m/" + k] = dense["v/" + k] = np.zeros(tuple(p.shape), np.float32)
+            dense["adam_scalars"] = np.zeros(4, np.float32)
+        else:
+            for p, m, v in opt.moments():
+                dense["m/" + names[id(p)]] = m.cpu().numpy()
+                dense["v/" + names[id(p)]] = v.cpu().numpy()
+            dense["adam_scalars"] = opt.scalars.cpu().numpy()
+        for path, layer in _dropout_layers(sub):
+            dev_step = 0 if layer._drop_step is None else int(layer._drop_step.item())
+            dense["dropout/" + path] = np.array([layer._dropout_calls, dev_step], np.int64)
+        if getattr(emb, "scalars", None) is not None:
+            dense["sparse_scalars"] = emb.scalars.cpu().numpy()
+        np.savez(directory / "dense.npz", **dense)
+        _save_idmap(directory, store.idmap)
+        meta = {"format": FORMAT, "world": W, "rows_per_field": [int(x) for x in store.rows],
+                "record": "fp32 [w|m|v] (adam) or [w|g2sum] (adagrad), row stride record_floats",
+                **_net_geometry(net), "dense_spec": _dense_spec(net), "step": step}
+        _write_meta(directory, meta)
+    return directory
+
+
+def _load_net(net, directory, tables: bool, dense: bool) -> dict:
+    directory = Path(directory)
+    meta = read_meta(directory)
+    emb, store = net.emb, net.emb.store
+    W, r = _world_rank(emb)
+    for k, want in _net_geometry(net).items():
+        got = meta.get(k, "mod" if k == "id_map" else None)
+        if got != want:
+            raise ValueError(f"checkpoint {k} = {got!r} does not match the net's {want!r}")
+    if dense:
+        unbuilt = _unbuilt_layers(net.sub_model)
+        if unbuilt:
+            raise ValueError(f"layers {unbuilt[:4]} of the net have no parameters yet: run one predict first")
+        if _dense_spec(net) != meta["dense_spec"]:
+            raise ValueError("checkpoint dense parameters (names / shapes) do not match the net's sub_model")
+    for s in range(meta["world"]):
+        if tables and not shard_path(directory, s, meta["world"]).exists():
+            raise FileNotFoundError(shard_path(directory, s, meta["world"]))
+    with np.load(directory / "dense.npz") as z:
+        if tables:
+            for dst, rec in load_shard_rows(directory, meta, W, r):
+                t = torch.from_numpy(np.array(rec, np.float32, copy=True)).to(emb.dev)
+                contiguous = dst.size and (np.diff(dst) == 1).all()
+                store.unpack(slice(int(dst[0]), int(dst[-1]) + 1) if contiguous else torch.from_numpy(dst).to(emb.dev), t)
+            if "sparse_scalars" in z.files:
+                emb.scalars.copy_(torch.from_numpy(z["sparse_scalars"]))
+            if store.idmap is not None:
+                with np.load(directory / "idmap.npz") as zi:
+                    store.idmap.load_state({k: zi[k] for k in zi.files})
+        if dense:
+            sub = net.sub_model
+            opt = _dense_opt(net, create=True)           # a GraphedTrainStep made after the load keeps its state
+            with torch.no_grad():
+                for k, v in sub.state_dict().items():    # views of the live tensors: copied in place
+                    v.copy_(torch.from_numpy(z[k]))
+                if opt is not None:
+                    names = {id(p): k for k, p in sub.named_parameters()}
+                    for p, m, v in opt.moments():
+                        m.copy_(torch.from_numpy(z["m/" + names[id(p)]]))
+                        v.copy_(torch.from_numpy(z["v/" + names[id(p)]]))
+                    opt.scalars.copy_(torch.from_numpy(z["adam_scalars"]))
+            for path, layer in _dropout_layers(sub):
+                calls, dev_step = (int(x) for x in z["dropout/" + path])
+                layer._dropout_calls = calls
+                if layer._drop_step is None:
+                    layer._drop_step = torch.zeros(1, dtype=torch.int64, device=emb.dev)
+                layer._drop_step.fill_(dev_step)
+    torch.cuda.synchronize(emb.dev)
+    if W > 1:
+        # the next step's peer gather reads the OTHER ranks' shards at its very start
+        import torch.distributed as dist
+        dist.barrier(group=getattr(emb, "group", None))
+    return meta
 
 
 # ------------------------------------------------------------------ Keras weights
