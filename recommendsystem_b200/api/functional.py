@@ -69,10 +69,15 @@ class DinFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, mode, q, keys, values, seq_len, mask, W1, b1, W2, b2):
         _require_cuda(q, keys)
+        if keys.dtype != q.dtype or (values is not None and values.dtype != q.dtype):
+            raise ValueError(f"DIN: q, keys and values must share one dtype (got {q.dtype}, {keys.dtype}, "
+                             f"{None if values is None else values.dtype})")
         q = q.contiguous()
-        if keys.stride(-1) != 1 or keys.stride(0) != keys.shape[1] * keys.stride(1):
+        # the kernels address row (b, t) of keys and values at (b*T + t) * kv_ld: a view laid out otherwise (a T-slice
+        # of a longer sequence, an expanded tensor) is copied, and both are copied when their row strides differ
+        if not ops.din_rows_at(keys, ops.din_kv_ld(keys)):
             keys = keys.contiguous()
-        if values is not None and (values.stride(-1) != 1 or values.stride(1) != keys.stride(1)):
+        if values is not None and not ops.din_rows_at(values, ops.din_kv_ld(keys)):
             values = values.contiguous()
             keys = keys.contiguous()
         out = ops.din_fwd(mode, q, keys, values, seq_len, mask, W1, b1.contiguous(), W2.contiguous(), b2.contiguous())

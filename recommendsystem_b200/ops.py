@@ -299,11 +299,46 @@ def interacting_bwd(x, saved, Wqkvr, bqkvr, gamma, beta, ln_eps, H, L, dy, use_r
 # --------------------------------------------------------------------- DIN
 
 
+def din_rows_at(t, ld):
+    """True when row (b, t) of the [B, T, H] view `t` lies at element (b*T + t) * ld of its storage: the only layout
+    the DIN kernels address (keys, values and their gradients share one row stride `ld`)."""
+    B, T = t.shape[0], t.shape[1]
+    return t.stride(2) == 1 and (T == 1 or t.stride(1) == ld) and (B == 1 or t.stride(0) == T * ld)
+
+
+def din_kv_ld(keys):
+    """The row stride of a [B, T, H] keys view as the DIN kernels read it (kv_ld)."""
+    B, T, H = keys.shape
+    return keys.stride(1) if T > 1 else (keys.stride(0) if B > 1 else H)
+
+
+def _din_check(mode, q, keys, values, seq_len, mask, W1, b1, W2, b2, kv_ld):
+    _need(q.dim() == 2 and q.is_contiguous(), "din: q must be a contiguous [B, H] tensor")
+    B, H = q.shape
+    _need(keys.dim() == 3 and keys.shape[0] == B and keys.shape[2] == H, "din: keys must be [B, T, H]")
+    _need(keys.dtype == q.dtype, f"din: keys dtype {keys.dtype} differs from q dtype {q.dtype}")
+    _need(din_rows_at(keys, kv_ld), f"din: keys rows must lie at (b*T + t) * {kv_ld} (strides {keys.stride()})")
+    if values is not None:
+        _need(values.shape == keys.shape, "din: values must have the shape of keys")
+        _need(values.dtype == q.dtype, f"din: values dtype {values.dtype} differs from q dtype {q.dtype}")
+        _need(din_rows_at(values, kv_ld),
+              f"din: values rows must lie at (b*T + t) * {kv_ld}, as keys' (strides {values.stride()})")
+    if seq_len is not None:
+        _need(seq_len.dtype == torch.int32 and seq_len.is_contiguous() and seq_len.numel() == B,
+              "din: seq_len must be contiguous int32 [B]")
+    if mask is not None:
+        _need(mask.dtype in (torch.uint8, torch.bool) and mask.is_contiguous() and mask.numel() == B * keys.shape[1],
+              "din: mask must be contiguous uint8 [B, T]")
+    for w in (W1, b1, W2, b2):
+        _need(w.dtype == torch.float32 and w.is_contiguous(), "din: W1, b1, W2, b2 must be contiguous fp32")
+
+
 def din_fwd(mode, q, keys, values, seq_len, mask, W1, b1, W2, b2, kv_ld=None):
     B, T = keys.shape[0], keys.shape[1]
     H = q.shape[1]
     Hd = W1.shape[1]
-    kv_ld = kv_ld or keys.stride(1)
+    kv_ld = kv_ld or din_kv_ld(keys)
+    _din_check(mode, q, keys, values, seq_len, mask, W1, b1, W2, b2, kv_ld)
     out = torch.empty(B, H, dtype=q.dtype, device=q.device)
     call("rs_din_fwd", mode, _ptr(q), _ptr(keys), _ptr(values), kv_ld, _dt(q), _ptr(seq_len), _ptr(mask),
          _ptr(W1), _ptr(b1), _ptr(W2), _ptr(b2), _ptr(out), B, T, H, Hd, _stream())
@@ -314,7 +349,9 @@ def din_bwd(mode, q, keys, values, seq_len, mask, W1, b1, W2, b2, dout, kv_ld=No
     B, T = keys.shape[0], keys.shape[1]
     H = q.shape[1]
     Hd = W1.shape[1]
-    kv_ld = kv_ld or keys.stride(1)
+    kv_ld = kv_ld or din_kv_ld(keys)
+    _din_check(mode, q, keys, values, seq_len, mask, W1, b1, W2, b2, kv_ld)
+    _need(dout.shape == q.shape and dout.dtype == q.dtype, "din: dout must be [B, H] of q's dtype")
     dq = torch.empty_like(q)
     dkeys = torch.empty(B, T, H, dtype=q.dtype, device=q.device)
     dvalues = torch.empty(B, T, H, dtype=q.dtype, device=q.device) if mode == cabi.DIN_A else None
