@@ -18,10 +18,10 @@ import torch
 from torch import nn
 
 from ..autoint import AutoIntConfig, AutoIntTrainer
-from .embedding import Adam, EmbeddingFeatures, category_column, embedding_column
-from .optim import DenseAdam
+from .embedding import Adam, category_column, embedding_column
 from .functional import dense
 from .interacting_layer import InteractingLayer
+from .net import ComposedNet
 
 
 def cross_entropy(y_true, y_pred, a=1.0, reduce_mean=False):
@@ -155,15 +155,15 @@ class ModelResult:
     model_predict = None
 
 
-class _AutoIntFullModel:
+class _AutoIntFullModel(ComposedNet):
     """`full_model` of AUTOINT: sparse ids -> EmbeddingFeatures -> sub_model.  Callable like a Keras model
     (`model(inputs)` -> [B,7] predictions); train_step() runs forward, the summed 7-label BCE
     (rank/multi_head/model.py:18-22), backward, the dense Adam (lr 1e-5, :52-53: rs_dense_adam) and the sparse push."""
+    dense_lr = 1e-5
 
-    def __init__(self, slots, emb, sub_model, training, group=None):
-        self.slots, self.emb, self.sub_model, self.training = slots, emb, sub_model, bool(training)
-        self.opt = None
-        self.group = group
+    def __init__(self, slots, cols, sub_model, training, device, seed, embedding_cls, group, id_map):
+        super().__init__(cols, Adam(5e-5, 0.9, 0.999, 1e-8), "linear", device, seed, embedding_cls, group, id_map)
+        self.slots, self.sub_model, self.training = slots, sub_model, bool(training)
         self.sub_model.train(self.training)
 
     def __call__(self, inputs: Dict[str, torch.Tensor]):
@@ -179,39 +179,17 @@ class _AutoIntFullModel:
         finally:
             self.sub_model.train(was)
 
-    def train_step(self, inputs: Dict[str, torch.Tensor], labels):
+    def _leaves(self, inputs):
+        embs = self.emb(inputs)
+        return [embs[s].detach().requires_grad_(True) for s in self.slots]
+
+    def _column_grads(self, x):
+        return {s: l.grad for s, l in zip(self.slots, x)}
+
+    def _loss(self, pred, labels):
         if isinstance(labels, dict):
             labels = torch.cat([labels[k].reshape(-1, 1) for k in AUTOINT_LABELS], dim=1)
-        embs = self.emb(inputs)
-        leaves = [embs[s].detach().requires_grad_(True) for s in self.slots]
-        pred = self.sub_model(leaves)
-        opt = self.dense_optimizer()
-        loss = cross_entropy(labels, pred).mean()
-        opt.zero_grad()
-        loss.backward()
-        opt.step()
-        self.emb.backward({s: l.grad for s, l in zip(self.slots, leaves)})
-        return loss.detach(), pred.detach()
-
-    def dense_optimizer(self):
-        """The dense Adam of sub_model (lr 1e-5), created at the first call: the lazily-built layers must exist."""
-        if self.opt is None:
-            self.opt = DenseAdam(self.sub_model.parameters(), lr=1e-5, beta1=0.9, beta2=0.999, eps=1e-8, group=self.group)
-        return self.opt
-
-    # the InteractingLayer's device-side dropout counter is part of what a step changes (api.graph warm-up undo)
-    def extra_state_snapshot(self):
-        il = self.sub_model.interacting_layer
-        return (il._dropout_calls, None if il._drop_step is None else il._drop_step.clone())
-
-    def extra_state_restore(self, st):
-        il = self.sub_model.interacting_layer
-        il._dropout_calls = st[0]
-        if il._drop_step is not None:
-            if st[1] is None:
-                il._drop_step.zero_()
-            else:
-                il._drop_step.copy_(st[1])
+        return cross_entropy(labels, pred).mean()
 
 
 def create_autoint_sub_model(slot_zip_user_embs, dense_inputs_map, deep_hidden_units, training, device="cuda:0"):
@@ -231,17 +209,10 @@ def AUTOINT(linear_features, dense_features, training, dnn_hidden_units=(32, 16)
     every distinct slot id its own row (api.embedding.EmbeddingFeatures)."""
     features = sorted(set(linear_features))                                   # :215-218
     cols = [embedding_column(category_column(s, bucket_size), dimension=8, combiner="mean") for s in features]
-    E = embedding_cls or EmbeddingFeatures
-    kw = {"group": group} if embedding_cls is not None else {}      # None = the default process group
-    if id_map != "mod":
-        kw["id_map"] = id_map
-    emb = E(cols, Adam(5e-5, 0.9, 0.999, 1e-8), "linear", device=device, seed=seed, **kw)
     sub_model = create_autoint_sub_model([(s, None) for s in linear_features], {k: None for k in dense_features},
                                          dnn_hidden_units, training, device=device)
-    if embedding_cls is not None and group is None:
-        from .optim import _world_group
-        group = _world_group()
-    full = _AutoIntFullModel(list(linear_features), emb, sub_model, training, group=group)
+    full = _AutoIntFullModel(list(linear_features), cols, sub_model, training, device, seed, embedding_cls, group,
+                             id_map)
     ret = ModelResult()
     ret.model = full                                                           # :247
     ret.sub_model = sub_model                                                  # :248

@@ -9,12 +9,13 @@ sort + sorted-segment sparse update - is captured ONCE and replayed:
     step = GraphedTrainStep(net, example_inputs, example_labels)      # warm-up + capture
     loss, outputs = step(inputs, labels)                               # copy into the static buffers, replay
 
-The warm-up steps (they allocate workspaces and create the optimizer state) are UNDONE before the capture: the
-embedding rows they touched, the dense parameters and both optimizers' state are restored bit for bit, so capturing
+The warm-up steps (they allocate workspaces) are UNDONE before the capture: the embedding rows they touched, the dense
+parameters, both optimizers' state and the InteractingLayers' dropout counters are restored bit for bit, so capturing
 after loading a checkpoint does not change the loaded weights and the first replay is the first train step.
 
-`net` is any object with `train_step(inputs: dict, labels: dict) -> (loss, outputs: dict)` (api.video_dnn.MtlNet,
-api.rough_rank_model.DssmNet, api.rank_ctr.RankCtrNet, ...).  Shapes and dtypes are fixed by the example batch;
+`net` is a composed net (api.net: `emb`, `sub_model`, `opt` / `dense_optimizer()`, `predict`, `train_step(inputs: dict,
+labels: dict) -> (loss, outputs)`), e.g. api.video_dnn.MtlNet, api.rough_rank_model.DssmNet, api.rank_ctr.RankCtrNet,
+the AUTOINT model.  Shapes and dtypes are fixed by the example batch;
 a different batch size needs its own GraphedTrainStep.  Inputs may live on the host (pinned or not): the copy
 into the static device buffers is the only per-step host work besides the replay.
 """
@@ -23,6 +24,8 @@ from __future__ import annotations
 from typing import Dict
 
 import torch
+
+from .interacting_layer import dropout_layers
 
 
 def _static(d: Dict, dev):
@@ -44,7 +47,7 @@ class GraphedTrainStep:
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(side):
-            for _ in range(max(1, warmup)):          # allocates workspaces, creates the optimizer state
+            for _ in range(max(1, warmup)):          # allocates workspaces
                 net.train_step(self.inputs, self.labels)
         torch.cuda.current_stream(dev).wait_stream(side)
         torch.cuda.synchronize(dev)
@@ -57,34 +60,25 @@ class GraphedTrainStep:
 
     @staticmethod
     def _snapshot(net, inputs):
-        """Everything the warm-up steps change.  Lazily built layers are built first (a forward has no side effects)
-        so that there are initial weights to return to."""
-        if not hasattr(net, "emb") or not hasattr(net.emb, "snapshot"):
-            return None
+        """Everything the warm-up steps change.  The lazily built layers are built first and the dense optimizer is
+        created, so that there are initial weights and optimizer state to return to.  The dropout counters are taken
+        before that forward: a sub_model in training mode advances them in `predict` too."""
+        dropout = [(m, m.dropout_state()) for _, m in dropout_layers(net.sub_model)]
         with torch.no_grad():
             net.predict(inputs)
-        snap = {"emb": net.emb.snapshot(inputs), "params": [p.detach().clone() for p in net.sub_model.parameters()]}
-        opt = getattr(net, "opt", None)
-        snap["opt"] = opt.snapshot() if opt is not None and hasattr(opt, "snapshot") else None
-        if hasattr(net, "extra_state_snapshot"):
-            snap["extra"] = net.extra_state_snapshot()
-        return snap
+        opt = net.dense_optimizer()
+        return {"emb": net.emb.snapshot(inputs), "params": [p.detach().clone() for p in net.sub_model.parameters()],
+                "opt": opt.snapshot(), "dropout": dropout}
 
     @staticmethod
     def _restore(net, snap):
-        if snap is None:
-            return
         net.emb.restore(snap["emb"])
-        opt = getattr(net, "opt", None)
-        if snap["opt"] is not None:
-            opt.restore(snap["opt"])
-        elif opt is not None and hasattr(opt, "flat_m"):          # created by the warm-up: back to a fresh state
-            opt.flat_m.zero_(); opt.flat_v.zero_(); opt.scalars.zero_()
+        net.opt.restore(snap["opt"])
         with torch.no_grad():
             for p, v in zip(net.sub_model.parameters(), snap["params"]):
                 p.copy_(v)
-        if "extra" in snap:
-            net.extra_state_restore(snap["extra"])
+        for layer, state in snap["dropout"]:
+            layer.load_dropout_state(state)
 
     def __call__(self, inputs: Dict, labels: Dict):
         for k, v in inputs.items():

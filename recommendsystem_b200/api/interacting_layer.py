@@ -88,7 +88,24 @@ class InteractingLayer(nn.Module):
         return InteractingFn.apply(inputs, W, b, self.layer_norm_gamma, self.layer_norm_beta, self.ln_eps,
                                    self.head_num, self.layer_num, self.use_res, rate, seed, step)
 
+    def dropout_state(self):
+        """(host call count, device call count) of the dropout mask counter: the state a training call advances."""
+        return self._dropout_calls, 0 if self._drop_step is None else int(self._drop_step.item())
+
+    def load_dropout_state(self, state):
+        """Set the counter to a dropout_state() value, in place: a captured CUDA graph of the step keeps reading it."""
+        self._dropout_calls, step = (int(x) for x in state)
+        if self._drop_step is not None:
+            self._drop_step.fill_(step)
+        elif step:
+            self._drop_step = torch.full((1,), step, dtype=torch.int64, device=self.layer_norm_gamma.device)
+
     def get_config(self):
         return dict(layer_num=self.layer_num, unit_num=self.unit_num, head_num=self.head_num,
                     use_dropout=self.use_dropout, dropout_rate=self.dropout_rate, use_res=self.use_res,
                     ln_eps=self.ln_eps)
+
+
+def dropout_layers(module: nn.Module):
+    """(path, layer) of every InteractingLayer in `module`: the layers whose dropout counter a train step advances."""
+    return [(p, m) for p, m in module.named_modules() if isinstance(m, InteractingLayer)]

@@ -15,11 +15,6 @@ import torch
 from .. import ops
 
 
-def _world_group():
-    import torch.distributed as dist
-    return dist.group.WORLD
-
-
 class DenseAdam:
     def __init__(self, params: Iterable[torch.nn.Parameter], lr, beta1=0.9, beta2=0.999, eps=1e-8, group=None):
         self.params = [p for p in params if p.requires_grad]

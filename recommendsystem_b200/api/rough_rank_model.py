@@ -15,8 +15,8 @@ import torch
 from torch import nn
 
 from .builders import _KerasDense
-from .optim import DenseAdam, _world_group
-from .embedding import Adam, EmbeddingFeatures, category_column, embedding_column
+from .embedding import Adam, category_column, embedding_column
+from .net import ComposedNet
 from .rough_rank_layer import DNN, PLE, CrossNet, KDLoss
 
 
@@ -156,23 +156,22 @@ def binary_crossentropy(y_true, y_pred, eps=1e-7):
     return (-(y * torch.log(p) + (1.0 - y) * torch.log(1.0 - p))).mean()
 
 
-class DssmNet:
+class DssmNet(ComposedNet):
     """DSSM() (model.py:118-187): 16-d embeddings (combiner mean, bucket 25600, sparse Adam 1e-3, :89-115)
-    for the user and item feature ids + the dense mask input '4575'."""
+    for the user and item feature ids + the dense mask input '4575'.  `train_step` is the create_model() compile
+    (model.py:206-222): dense Adam 1e-4; BCE(student) + BCE(teacher) + mean(distill)."""
+    dense_lr = 0.0001
 
     def __init__(self, user_ids=C.USER_FEATURE_IDS, item_ids=C.ITEM_FEATURE_IDS, bucket_size=25600,
                  device="cuda:0", seed=0, embedding_cls=None, group=None):
-        self.group = group if (group is not None or embedding_cls is None) else _world_group()
         self.ids = list(user_ids) + list(item_ids)
         dims = [C.USER_OUTPUT_DIM] * len(user_ids) + [C.ITEM_OUTPUT_DIM] * len(item_ids)
         cols = [embedding_column(category_column(C.get_feature_id(f) if f in C.ALL_FEATURE_ID_2_SLOT else f,
                                                  bucket_size), dimension=d, combiner="mean")
                 for f, d in zip(self.ids, dims)]
-        E, kw = (embedding_cls, {"group": group}) if embedding_cls is not None else (EmbeddingFeatures, {})
-        self.emb = E(cols, Adam(learning_rate=0.001, beta1=0.9, beta2=0.999, epsilon=1e-8),
-                     "sparse_emb_input", device=device, seed=seed, **kw)
+        super().__init__(cols, Adam(learning_rate=0.001, beta1=0.9, beta2=0.999, epsilon=1e-8), "sparse_emb_input",
+                         device, seed, embedding_cls, group)
         self.sub_model = DssmSubModel(user_ids, item_ids).to(device)
-        self.opt = None
 
     def train(self, inputs):
         e = self.emb({k: v for k, v in inputs.items() if k != C.DENSE_MASK_ID})
@@ -182,25 +181,12 @@ class DssmNet:
         with torch.no_grad():
             return self.train(inputs)
 
-    def train_step(self, inputs, labels: Dict[str, torch.Tensor]):
-        """create_model() compile (model.py:206-222): dense Adam 1e-4; BCE(student) + BCE(teacher) + mean(distill)."""
-        e = self.emb({k: v for k, v in inputs.items() if k != C.DENSE_MASK_ID})
-        leaves = {k: v.detach().requires_grad_(True) for k, v in e.items()}
-        out = self.sub_model(leaves, inputs[C.DENSE_MASK_ID].to(self.emb.dev))
-        opt = self.dense_optimizer()
-        loss = (binary_crossentropy(labels["student"], out["student"]) +
-                binary_crossentropy(labels["teacher"], out["teacher"]) + y_pred_loss(None, out["distill"]))
-        opt.zero_grad()
-        loss.backward()
-        opt.step()
-        self.emb.backward({k: v.grad for k, v in leaves.items()})
-        return loss.detach(), {k: v.detach() for k, v in out.items()}
+    def _forward(self, x, inputs):
+        return self.sub_model(x, inputs[C.DENSE_MASK_ID].to(self.emb.dev))
 
-    def dense_optimizer(self):
-        """The dense Adam of sub_model (lr 1e-4), created at the first call: the lazily-built layers must exist."""
-        if self.opt is None:
-            self.opt = DenseAdam(self.sub_model.parameters(), lr=0.0001, beta1=0.9, beta2=0.999, eps=1e-8, group=getattr(self, 'group', None))
-        return self.opt
+    def _loss(self, out, labels):
+        return (binary_crossentropy(labels["student"], out["student"]) +
+                binary_crossentropy(labels["teacher"], out["teacher"]) + y_pred_loss(None, out["distill"]))
 
 
 def DSSM(**kw):

@@ -18,8 +18,8 @@ import torch
 from torch import nn
 
 from .builders import _KerasDense, fused_dense
-from .optim import DenseAdam, _world_group
-from .embedding import AdaGrad, EmbeddingFeatures, category_column, embedding_column
+from .embedding import AdaGrad, category_column, embedding_column
+from .net import ComposedNet
 from .staytime_config import Config as C
 from .staytime_layer import DIN, DeepCrossLayer
 
@@ -198,17 +198,15 @@ LOSSES = {TASK_KEYS[0]: custom_kl_loss, TASK_KEYS[1]: cross_entropy, TASK_KEYS[2
 LOSS_WEIGHTS = {TASK_KEYS[0]: 2.0, TASK_KEYS[1]: 2.0, TASK_KEYS[2]: 1.0}                     # model.py:85-87
 
 
-class MtlNet:
+class MtlNet(ComposedNet):
     """mtl_net(...) (staytime/VideoDnn.py:266-302): 32-d embeddings for every slot (combiner mean) plus the
     `[B, seq_max_len, 32]` sequence lookups of `seq_slots` (combiner None), sparse AdaGrad(0.005, g2sum 0.1,
     scale 0.1) (:233), feeding VideoDnnSubModel.  `train` / `predict` are the two graph outputs of the
     reference; `train_step` adds the compile() of staytime/model.py:72-90 (dense Adam 5e-4, weighted losses)."""
+    dense_lr = 0.0005
 
     def __init__(self, slots, seq_slots, seq_max_len, dnn_hidden_units=(64, 32), bucket_size=81920, device="cuda:0",
                  seed=0, embedding_cls=None, group=None):
-        # embedding_cls = api.sharded_embedding.ShardedEmbeddingFeatures (+ its process group): row-sharded tables
-        # over the ranks, dense gradients averaged over them (staytime/parse.py:77-79)
-        self.group = group if (group is not None or embedding_cls is None) else _world_group()
         self.slots, self.seq_slots = list(slots), list(seq_slots)
         cats = {s: category_column(s, bucket_size) for s in self.slots}                                  # :219-220
         # single-valued columns in sorted-slot order: the stacked gather output [B, n, 32] then IS the sub-model's
@@ -216,11 +214,9 @@ class MtlNet:
         cols = [embedding_column(cats[s], 32, combiner="mean", name="emb_col_%s" % s) for s in sorted(self.slots)]
         cols += [embedding_column(cats[s], 32, combiner=None, seq_max_len=seq_max_len, name="emb_col_seq_%s" % s)
                  for s in self.seq_slots]                                                                # :228-231
-        E, kw = (embedding_cls, {"group": group}) if embedding_cls is not None else (EmbeddingFeatures, {})
-        self.emb = E(cols, AdaGrad(learning_rate=0.005, initial_g2sum=0.1, initial_scale=0.1),
-                     "sparse_emb_input", device=device, seed=seed, **kw)
+        super().__init__(cols, AdaGrad(learning_rate=0.005, initial_g2sum=0.1, initial_scale=0.1), "sparse_emb_input",
+                         device, seed, embedding_cls, group)
         self.sub_model = VideoDnnSubModel(self.slots, self.seq_slots, dnn_hidden_units).to(device)
-        self.opt = None
 
     def _embed(self, inputs):
         e = self.emb(inputs)
@@ -242,30 +238,26 @@ class MtlNet:
             embs, seqs = self._embed(inputs)
             return self.sub_model(embs, seqs)[1]
 
-    def train_step(self, inputs, labels: Dict[str, torch.Tensor]):
+    def _leaves(self, inputs):
         embs, seqs = self._embed(inputs)
         stacked = not isinstance(embs, dict)
         le = embs.detach().requires_grad_(True) if stacked else {s: v.detach().requires_grad_(True) for s, v in embs.items()}
-        ls = {s: (v[0].detach().requires_grad_(True), v[1]) for s, v in seqs.items()}
-        out, _ = self.sub_model(le, ls)
-        opt = self.dense_optimizer()
-        loss = sum(LOSS_WEIGHTS[k] * LOSSES[k](labels[k], out[k]).mean() for k in TASK_KEYS)
-        opt.zero_grad()
-        loss.backward()
-        opt.step()
-        if stacked:
+        return le, {s: (v[0].detach().requires_grad_(True), v[1]) for s, v in seqs.items()}
+
+    def _column_grads(self, x):
+        le, ls = x
+        if torch.is_tensor(le):                                # stacked [B, n, 32] leaf
             grads = {"emb_col_%s" % s: le.grad[:, i, :] for i, s in enumerate(sorted(self.slots))}
         else:
             grads = {"emb_col_%s" % s: v.grad for s, v in le.items()}
         grads.update({"emb_col_seq_%s" % s: v[0].grad for s, v in ls.items()})
-        self.emb.backward(grads)
-        return loss.detach(), {k: v.detach() for k, v in out.items()}
+        return grads
 
-    def dense_optimizer(self):
-        """The dense Adam of sub_model (lr 5e-4), created at the first call: the lazily-built layers must exist."""
-        if self.opt is None:
-            self.opt = DenseAdam(self.sub_model.parameters(), lr=0.0005, beta1=0.9, beta2=0.999, eps=1e-8, group=getattr(self, 'group', None))
-        return self.opt
+    def _forward(self, x, inputs):
+        return self.sub_model(*x)[0]
+
+    def _loss(self, out, labels):
+        return sum(LOSS_WEIGHTS[k] * LOSSES[k](labels[k], out[k]).mean() for k in TASK_KEYS)
 
 
 def mtl_net(slots, seq_slots, seq_max_len, dnn_hidden_units=(64, 32), **kw):

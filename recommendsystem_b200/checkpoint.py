@@ -48,11 +48,12 @@ import dataclasses
 import json
 import os
 from pathlib import Path
-from typing import Dict, Iterator, Tuple
+from typing import Dict, Iterator
 
 import numpy as np
 import torch
 
+from .api.interacting_layer import dropout_layers
 from .arena import shard_layout as shard_rows     # (local_rows[F], local_base[F]) of a W-way job
 
 FORMAT = "rs_b200.checkpoint.v1"
@@ -125,12 +126,8 @@ def _cfg_dict(cfg) -> dict:
     return out
 
 
-def _world_rank(trainer) -> Tuple[int, int]:
-    return int(getattr(trainer, "world", 1)), int(getattr(trainer, "rank", 0))
-
-
 def _id_map(trainer) -> str:
-    return "hash" if getattr(trainer, "idmap", None) is not None else "mod"
+    return "hash" if trainer.store.idmap is not None else "mod"
 
 
 def save_checkpoint(obj, directory, step: int | None = None) -> Path:
@@ -145,30 +142,23 @@ def save_checkpoint(obj, directory, step: int | None = None) -> Path:
 def load_checkpoint(obj, directory, tables: bool = True, dense: bool = True) -> dict:
     """Restore `obj` (a trainer or a composed net) in place from `directory` (any world size); returns meta.json.
     Raises ValueError when the checkpoint was written by another kind of model or its geometry differs."""
-    if _is_net(obj):
-        return _load_net(obj, directory, tables, dense)
-    return _load_trainer(obj, directory, tables, dense)
+    meta = (_load_net if _is_net(obj) else _load_trainer)(obj, directory, tables, dense)
+    store = obj.emb.store if _is_net(obj) else obj.store
+    torch.cuda.synchronize(store.dev)
+    if store.world > 1:
+        # the next step's peer gather reads the OTHER ranks' shards at its very start: nobody may run ahead of a
+        # rank that is still copying its shard in
+        import torch.distributed as dist
+        dist.barrier(group=obj.emb.group if _is_net(obj) else obj.ex.group)
+    return meta
 
 
 def _save_trainer(trainer, directory, step: int | None = None) -> Path:
     directory = Path(directory)
     directory.mkdir(parents=True, exist_ok=True)
-    W, r = _world_rank(trainer)
-    torch.cuda.synchronize(trainer.dev)
-    arena = trainer.arena                                    # [n_local, 3, d]
-    n, d = arena.shape[0], arena.shape[2]
-    stage = torch.empty(min(n, CHUNK_ROWS), 3, d, dtype=torch.float32, pin_memory=True)
-
-    def chunks():
-        for r0 in range(0, n, CHUNK_ROWS):
-            r1 = min(n, r0 + CHUNK_ROWS)
-            stage[: r1 - r0].copy_(arena[r0:r1])
-            torch.cuda.synchronize(trainer.dev)
-            yield stage[: r1 - r0].numpy()
-
-    write_shard(shard_path(directory, r, W), chunks())
-    if r == 0:
-        _remove_stale_shards(directory, W)
+    store = trainer.store
+    _save_tables(store, directory)
+    if store.rank == 0:
         dense = {}
         for name, shape, off in trainer.spec:
             k = int(np.prod(shape))
@@ -177,10 +167,9 @@ def _save_trainer(trainer, directory, step: int | None = None) -> Path:
             dense["v/" + name] = trainer.flat_v[off:off + k].view(shape).cpu().numpy()
         dense["adam_scalars"] = trainer.adam_scalars.cpu().numpy()
         np.savez(directory / "dense.npz", **dense)
-        _save_idmap(directory, trainer.idmap if _id_map(trainer) == "hash" else None)
         meta = {
-            "format": FORMAT, "world": W, "embed_dim": int(d),
-            "rows_per_field": [int(x) for x in trainer.rows_host],
+            "format": FORMAT, "world": store.world, "embed_dim": store.d,
+            "rows_per_field": [int(x) for x in store.rows],
             "record": "[w|m|v] fp32, row stride 3*embed_dim",
             "dense_spec": [[nm, list(sh)] for nm, sh, _ in trainer.spec],
             "config": _cfg_dict(trainer.cfg), "step": step,
@@ -191,19 +180,46 @@ def _save_trainer(trainer, directory, step: int | None = None) -> Path:
     return directory
 
 
-def _remove_stale_shards(directory: Path, world: int):
-    # a reused directory may hold table shards of an earlier save at another world size: remove them so
-    # that the directory only ever describes ONE checkpoint (meta.json names the world size that counts)
-    for stale in directory.glob("tables.rank*of*.bin"):
-        if not stale.name.endswith(f"of{world}.bin"):
-            stale.unlink()
+def _save_tables(store, directory: Path):
+    """This rank's shard of the arena `store`: its Arena.pack records, device -> pinned host -> file in bounded chunks.
+    Rank 0 also writes (hash mode) or removes idmap.npz."""
+    torch.cuda.synchronize(store.dev)
+    n = store.n_local
+    stage = torch.empty(min(n, CHUNK_ROWS), store.record_floats, dtype=torch.float32, pin_memory=True)
+
+    def chunks():
+        for r0 in range(0, n, CHUNK_ROWS):
+            r1 = min(n, r0 + CHUNK_ROWS)
+            stage[: r1 - r0].copy_(store.pack(slice(r0, r1)))
+            torch.cuda.synchronize(store.dev)
+            yield stage[: r1 - r0].numpy()
+
+    write_shard(shard_path(directory, store.rank, store.world), chunks())
+    if store.rank == 0:
+        # a reused directory may hold table shards of an earlier save at another world size: remove them so
+        # that the directory only ever describes ONE checkpoint (meta.json names the world size that counts)
+        for stale in directory.glob("tables.rank*of*.bin"):
+            if not stale.name.endswith(f"of{store.world}.bin"):
+                stale.unlink()
+        if store.idmap is not None:
+            np.savez(directory / "idmap.npz", **store.idmap.state())
+        elif (directory / "idmap.npz").exists():           # left by an earlier hash-mode save into this directory
+            (directory / "idmap.npz").unlink()
 
 
-def _save_idmap(directory: Path, idmap):
-    if idmap is not None:
-        np.savez(directory / "idmap.npz", **idmap.state())
-    elif (directory / "idmap.npz").exists():               # left by an earlier hash-mode save into this directory
-        (directory / "idmap.npz").unlink()
+def _load_tables(store, directory: Path, meta: dict):
+    """This rank's rows of the checkpoint's tables (any world size) and, in hash mode, the id map, into `store` in
+    place (Arena.unpack)."""
+    for s in range(meta["world"]):
+        if not shard_path(directory, s, meta["world"]).exists():
+            raise FileNotFoundError(shard_path(directory, s, meta["world"]))
+    for dst, rec in load_shard_rows(directory, meta, store.world, store.rank):
+        t = torch.from_numpy(np.array(rec, np.float32, copy=True)).reshape(dst.size, -1)     # trainer: [n, 3, d]
+        contiguous = dst.size and (np.diff(dst) == 1).all()
+        store.unpack(slice(int(dst[0]), int(dst[-1]) + 1) if contiguous else torch.from_numpy(dst).to(store.dev), t)
+    if store.idmap is not None:
+        with np.load(directory / "idmap.npz") as z:
+            store.idmap.load_state({k: z[k] for k in z.files})
 
 
 def _write_meta(directory: Path, meta: dict):
@@ -222,28 +238,16 @@ def read_meta(directory) -> dict:
 def _load_trainer(trainer, directory, tables: bool = True, dense: bool = True) -> dict:
     directory = Path(directory)
     meta = read_meta(directory)
-    W, r = _world_rank(trainer)
+    store = trainer.store
     if "model" in meta:
         raise ValueError(f"{directory}: a checkpoint of a {meta['model']} net, not of an AutoInt trainer")
     if meta.get("id_map", "mod") != _id_map(trainer):
         raise ValueError(f"checkpoint id_map={meta.get('id_map', 'mod')!r} does not match the trainer's "
                          f"id_map={_id_map(trainer)!r}")
     if tables:
-        if [int(x) for x in trainer.rows_host] != meta["rows_per_field"] or trainer.arena.shape[2] != meta["embed_dim"]:
+        if [int(x) for x in store.rows] != meta["rows_per_field"] or store.d != meta["embed_dim"]:
             raise ValueError("checkpoint tables do not match the trainer's rows_per_field / embed_dim")
-        for s in range(meta["world"]):
-            if not shard_path(directory, s, meta["world"]).exists():
-                raise FileNotFoundError(shard_path(directory, s, meta["world"]))
-        arena = trainer.arena
-        for dst, rec in load_shard_rows(directory, meta, W, r):
-            t = torch.from_numpy(np.array(rec, np.float32, copy=True)).to(trainer.dev)
-            if dst.size and (np.diff(dst) == 1).all():
-                arena[int(dst[0]): int(dst[-1]) + 1].copy_(t)
-            else:
-                arena.index_copy_(0, torch.from_numpy(dst).to(trainer.dev), t)
-        if _id_map(trainer) == "hash":
-            with np.load(directory / "idmap.npz") as z:
-                trainer.idmap.load_state({k: z[k] for k in z.files})
+        _load_tables(store, directory, meta)
     if dense:
         with np.load(directory / "dense.npz") as z:
             for name, shape, off in trainer.spec:
@@ -254,12 +258,6 @@ def _load_trainer(trainer, directory, tables: bool = True, dense: bool = True) -
                     buf[off:off + k].copy_(torch.from_numpy(np.ascontiguousarray(z[key], np.float32)).reshape(-1))
             trainer.adam_scalars.copy_(torch.from_numpy(z["adam_scalars"]))
         _refresh_dense_shadows(trainer)
-    torch.cuda.synchronize(trainer.dev)
-    if W > 1:
-        # the next step's peer gather reads the OTHER ranks' shards at its very start: nobody may run ahead of a
-        # rank that is still copying its shard in
-        import torch.distributed as dist
-        dist.barrier(group=getattr(getattr(trainer, "ex", None), "group", None))
     return meta
 
 
@@ -303,12 +301,6 @@ def _unbuilt_layers(module):
             if getattr(m, "built", True) is False or (hasattr(m, "kernel") and m.kernel is None)]
 
 
-def _dropout_layers(module):
-    """(path, layer) of every layer with a dropout call counter (InteractingLayer: `_drop_step` on the device,
-    `_dropout_calls` its host mirror)."""
-    return [(p, m) for p, m in module.named_modules() if hasattr(m, "_drop_step")]
-
-
 def _dense_opt(net, create: bool):
     """The net's DenseAdam; `create` builds it through the net's dense_optimizer() when it does not exist yet."""
     opt = net.dense_optimizer() if create and hasattr(net, "dense_optimizer") else getattr(net, "opt", None)
@@ -323,21 +315,8 @@ def _save_net(net, directory, step):
     if getattr(emb, "_pending_backward", False):
         raise RuntimeError("save_checkpoint called between a training forward and its backward")
     directory.mkdir(parents=True, exist_ok=True)
-    W, r = _world_rank(emb)
-    torch.cuda.synchronize(emb.dev)
-    n, rf = store.n_local, store.record_floats
-    stage = torch.empty(min(n, CHUNK_ROWS), rf, dtype=torch.float32, pin_memory=True)
-
-    def chunks():
-        for r0 in range(0, n, CHUNK_ROWS):
-            r1 = min(n, r0 + CHUNK_ROWS)
-            stage[: r1 - r0].copy_(store.pack(slice(r0, r1)))
-            torch.cuda.synchronize(emb.dev)
-            yield stage[: r1 - r0].numpy()
-
-    write_shard(shard_path(directory, r, W), chunks())
-    if r == 0:
-        _remove_stale_shards(directory, W)
+    _save_tables(store, directory)
+    if store.rank == 0:
         sub = net.sub_model
         dense = {k: v.detach().cpu().numpy() for k, v in sub.state_dict().items()}
         names = {id(p): k for k, p in sub.named_parameters()}
@@ -352,14 +331,12 @@ def _save_net(net, directory, step):
                 dense["m/" + names[id(p)]] = m.cpu().numpy()
                 dense["v/" + names[id(p)]] = v.cpu().numpy()
             dense["adam_scalars"] = opt.scalars.cpu().numpy()
-        for path, layer in _dropout_layers(sub):
-            dev_step = 0 if layer._drop_step is None else int(layer._drop_step.item())
-            dense["dropout/" + path] = np.array([layer._dropout_calls, dev_step], np.int64)
+        for path, layer in dropout_layers(sub):
+            dense["dropout/" + path] = np.array(layer.dropout_state(), np.int64)
         if getattr(emb, "scalars", None) is not None:
             dense["sparse_scalars"] = emb.scalars.cpu().numpy()
         np.savez(directory / "dense.npz", **dense)
-        _save_idmap(directory, store.idmap)
-        meta = {"format": FORMAT, "world": W, "rows_per_field": [int(x) for x in store.rows],
+        meta = {"format": FORMAT, "world": store.world, "rows_per_field": [int(x) for x in store.rows],
                 "record": "fp32 [w|m|v] (adam) or [w|g2sum] (adagrad), row stride record_floats",
                 **_net_geometry(net), "dense_spec": _dense_spec(net), "step": step}
         _write_meta(directory, meta)
@@ -370,7 +347,6 @@ def _load_net(net, directory, tables: bool, dense: bool) -> dict:
     directory = Path(directory)
     meta = read_meta(directory)
     emb, store = net.emb, net.emb.store
-    W, r = _world_rank(emb)
     for k, want in _net_geometry(net).items():
         got = meta.get(k, "mod" if k == "id_map" else None)
         if got != want:
@@ -381,20 +357,11 @@ def _load_net(net, directory, tables: bool, dense: bool) -> dict:
             raise ValueError(f"layers {unbuilt[:4]} of the net have no parameters yet: run one predict first")
         if _dense_spec(net) != meta["dense_spec"]:
             raise ValueError("checkpoint dense parameters (names / shapes) do not match the net's sub_model")
-    for s in range(meta["world"]):
-        if tables and not shard_path(directory, s, meta["world"]).exists():
-            raise FileNotFoundError(shard_path(directory, s, meta["world"]))
+    if tables:
+        _load_tables(store, directory, meta)
     with np.load(directory / "dense.npz") as z:
-        if tables:
-            for dst, rec in load_shard_rows(directory, meta, W, r):
-                t = torch.from_numpy(np.array(rec, np.float32, copy=True)).to(emb.dev)
-                contiguous = dst.size and (np.diff(dst) == 1).all()
-                store.unpack(slice(int(dst[0]), int(dst[-1]) + 1) if contiguous else torch.from_numpy(dst).to(emb.dev), t)
-            if "sparse_scalars" in z.files:
-                emb.scalars.copy_(torch.from_numpy(z["sparse_scalars"]))
-            if store.idmap is not None:
-                with np.load(directory / "idmap.npz") as zi:
-                    store.idmap.load_state({k: zi[k] for k in zi.files})
+        if tables and "sparse_scalars" in z.files:
+            emb.scalars.copy_(torch.from_numpy(z["sparse_scalars"]))
         if dense:
             sub = net.sub_model
             opt = _dense_opt(net, create=True)           # a GraphedTrainStep made after the load keeps its state
@@ -407,17 +374,8 @@ def _load_net(net, directory, tables: bool, dense: bool) -> dict:
                         m.copy_(torch.from_numpy(z["m/" + names[id(p)]]))
                         v.copy_(torch.from_numpy(z["v/" + names[id(p)]]))
                     opt.scalars.copy_(torch.from_numpy(z["adam_scalars"]))
-            for path, layer in _dropout_layers(sub):
-                calls, dev_step = (int(x) for x in z["dropout/" + path])
-                layer._dropout_calls = calls
-                if layer._drop_step is None:
-                    layer._drop_step = torch.zeros(1, dtype=torch.int64, device=emb.dev)
-                layer._drop_step.fill_(dev_step)
-    torch.cuda.synchronize(emb.dev)
-    if W > 1:
-        # the next step's peer gather reads the OTHER ranks' shards at its very start
-        import torch.distributed as dist
-        dist.barrier(group=getattr(emb, "group", None))
+            for path, layer in dropout_layers(sub):
+                layer.load_dropout_state(z["dropout/" + path])
     return meta
 
 

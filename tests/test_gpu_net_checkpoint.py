@@ -23,28 +23,35 @@ B = 48
 
 # ------------------------------------------------------------------ a small net over AdaGrad per element
 class _Tower(nn.Module):
-    def __init__(self, hidden):
+    def __init__(self, hidden, dropout=False):
         super().__init__()
+        from recommendsystem_b200.api import InteractingLayer
         from recommendsystem_b200.api.builders import _KerasDense
         self.hidden = _KerasDense(hidden, "relu")
         self.out = _KerasDense(1, "sigmoid")
+        # attention dropout over the columns: a counter every train step advances
+        self.interact = InteractingLayer(unit_num=8, head_num=2, use_dropout=True) if dropout else None
 
     def forward(self, embs):
-        return self.out(self.hidden(torch.cat(embs, dim=1)))
+        x = torch.cat(embs, dim=1)
+        if self.interact is not None:
+            x = torch.cat([x, self.interact(torch.stack(embs, dim=1)).flatten(1)], dim=1)
+        return self.out(self.hidden(x))
 
 
 class ElementNet:
     """Three single-valued columns and one padded bag column over EmbeddingFeatures(AdaGrad(per_element=True)), a
-    two-layer tower, dense Adam."""
+    two-layer tower (dropout=True: beside an InteractingLayer with attention dropout), dense Adam.  A user's net: no
+    subclass of api.net.ComposedNet."""
 
-    def __init__(self, dev, seed, bucket=300, d=8, opt="adagrad_element", id_map="mod", hidden=16):
+    def __init__(self, dev, seed, bucket=300, d=8, opt="adagrad_element", id_map="mod", hidden=16, dropout=False):
         from recommendsystem_b200.api.embedding import (Adam, AdaGrad, EmbeddingFeatures, category_column,
                                                         embedding_column)
         self.keys = ["c0", "c1", "c2", "bag"]
         cols = [embedding_column(category_column(k, bucket), d) for k in self.keys]
         sparse = Adam(1e-2) if opt == "adam" else AdaGrad(0.05, 0.1, 0.1, per_element=opt == "adagrad_element")
         self.emb = EmbeddingFeatures(cols, sparse, device=dev, seed=seed, id_map=id_map)
-        self.sub_model = _Tower(hidden).to(dev)
+        self.sub_model = _Tower(hidden, dropout).to(dev)
         self.opt = None
 
     def predict(self, inputs):
@@ -133,7 +140,7 @@ def _case(kind, dev):
         def batch():
             return ids(slots), {k: flag() for k in AUTOINT_LABELS}
     else:
-        make = lambda seed: ElementNet(dev, seed)
+        make = lambda seed: ElementNet(dev, seed, dropout=kind == "element_dropout")
 
         def batch():
             return _element_batch(g, dev)
@@ -177,7 +184,8 @@ def _assert_same(x, y):
 
 
 CASES = [(k, "eager") for k in ("mtl", "dssm", "rank_ctr", "autoint", "element")] + \
-        [(k, m) for k in ("mtl", "dssm", "autoint") for m in ("graph_after", "graph_before")]
+        [(k, m) for k in ("mtl", "dssm", "rank_ctr", "autoint", "element_dropout")
+         for m in ("graph_after", "graph_before")]
 
 
 @pytest.mark.parametrize("kind,mode", CASES)
