@@ -576,6 +576,26 @@ int rs_logit_head_fwd_bwd_relu(const void* Z, int64_t ldz, int dtype, const floa
 int rs_logit_head_reduce(const void* ws, size_t ws_bytes, float* dw, float* db, float* loss_out, int B, int zw,
                          void* stream);
 
+/* The head's parameter gradients and loss from a p_out computed elsewhere (rs_tower_step): the per-CTA partials of
+ * dw = Z^T dz, db = sum dz and the loss, dz derived from the stored p_out and y exactly as the two calls above derive
+ * it, are left in `ws` for rs_logit_head_reduce. */
+int rs_logit_head_grad(const void* Z, int64_t ldz, int dtype, const void* p, const float* y, float a, int B, int zw,
+                       void* ws, size_t ws_bytes, void* stream);
+
+/* The AutoInt tower's part of the bf16 train step in one launch (Dense(relu) N0 -> Dense(relu) N1 -> the logit head
+ * -> their backward down to the tower's input gradient), all activations bf16 and row-major:
+ *   H0 = relu(X W0 + b0) [B, N0];  Z[:, :N1] = relu(H0 W1 + b1);  p_out = sigmoid(Z w + ob) [B];
+ *   dz = d BCE(clip(p_out, 1e-6, 1), y; a) / d logit (mean over B, as rs_logit_head_fwd_bwd_relu);
+ *   dZ = dz w with dZ[:, :N1] multiplied by relu'(Z[:, :N1]);  dH0 = (dZ[:, :N1] W1^T) relu'(H0);  dX = dH0 W0^T.
+ * X [B, K0]; Z, dZ [B, N1 + Ki] (Z[:, N1:] is read); W0T [N0, K0] and W1T [N1, N0] are the transposed bf16 weights,
+ * W0 [K0, N0] and W1 [N0, N1] the weights as they lie; b0, b1, w [N1 + Ki], ob [1], y [B] fp32.  dX is stored, not
+ * accumulated.  The head's dw / db / loss are not computed (rs_logit_head_grad).  rs_tower_supported says whether the
+ * kernel exists for these widths (N0 = 256, N1 = 128, K0 and Ki multiples of 16, Ki <= 700). */
+int rs_tower_supported(int K0, int N0, int N1, int Ki);
+int rs_tower_step(const void* X, const void* W0T, const void* W1T, const void* W0, const void* W1, const float* b0,
+                  const float* b1, const float* w, const float* ob, const float* y, float a, void* Z, void* p_out,
+                  void* dZ, void* H0, void* dH0, void* dX, int B, int K0, int N0, int N1, int Ki, void* stream);
+
 /* dst[n, m] = src[m, n] (2-D transpose with leading dims; bf16 or fp32).  Used to
  * present activations K-major to the tensor-core weight-gradient GEMMs. */
 int rs_transpose2d(const void* src, int64_t lds, void* dst, int64_t ldd, int M, int N,

@@ -93,6 +93,9 @@ class AutoIntConfig:
     # "mod": row = row_base[f] + id mod rows_per_field[f].  "hash": every distinct (field, id) gets its own row of the
     # field's rows_per_field (a capacity) the first time a train step sees it (recommendsystem_b200.idmap)
     id_map: str = "mod"
+    # bf16 mode with the fused lookup: the whole tower (both Dense(relu) layers, the logit head and their backward
+    # down to dX) as one launch (rs_tower_step) where the kernel exists for the widths; False = 4 GEMMs + the head pass
+    fuse_tower: bool = True
 
     def rows(self) -> List[int]:
         if isinstance(self.rows_per_field, int):
@@ -183,6 +186,10 @@ class AutoIntTrainer:
         self.adam_done = torch.cuda.Event()
         self.fused = bool(cfg.fuse_embedding and self.bf16 and ops.interacting_path(
             F, d, U, cfg.head_num, torch.bfloat16, True) == cabi.PATH_TCGEN05 and self.table_ld % 16 == 0)
+        # the widths and buffers the tower kernel takes (whether it runs also depends on `fused`: fuse_tower)
+        self._tower_ok = bool(cfg.fuse_tower and self.bf16 and len(cfg.mlp_hidden) == 2 and ops.tower_supported(
+            F * d, cfg.mlp_hidden[0], cfg.mlp_hidden[1], F * U) and all(
+            self.P16[k].data_ptr() % 16 == 0 for k in ("mlp_W0", "mlp_W1")))
         self.graph = None
         self.timer = None               # set to a PhaseTimer for an instrumented (eager) step
         self.stamps, self.stamp_names = None, {}     # set `stamps` to an int64 buffer for tools/step_timeline.py
@@ -191,6 +198,13 @@ class AutoIntTrainer:
                    cabi.load().rs_colsum_workspace_bytes(B, max(widths + [self.zw])))
         self.ws = torch.empty(int(n_ws) + 256, dtype=torch.uint8, device=self.dev)
         self.head_ws = ops.logit_head_workspace(B, self.zw, self.dev)     # head partials, reduced on the side stream
+
+    @property
+    def fuse_tower(self) -> bool:
+        """The tower runs as one launch (rs_tower_step).  Only beside the fused InteractingLayer backward, which adds
+        its own part to the dX the tower kernel stores; read at step time, so a subclass that turns `fused` off (the
+        all-NCCL sharded path) also gets the separate tower kernels."""
+        return self._tower_ok and self.fused
 
     # ------------------------------------------------------------------ setup
     def _arena_shard(self):
@@ -304,44 +318,11 @@ class AutoIntTrainer:
         # K5: MLP tower; last hidden layer lands in Z[:, :n_deep], Flatten(A) in Z[:, n_deep:]
         Xf = self.X.view(B, F * d)
         acts = [Xf] + self.H + [self.Z[:, :self.n_deep]]
-        with ph("mlp_fwd"):
-            for i in range(nmlp):
-                self._dense_fwd(acts[i], f"mlp_W{i}", f"mlp_b{i}", acts[i + 1])
-        self._stamp("mlp_fwd_end")
-        with ph("logits_loss"):
-            # final Dense(1, sigmoid) + clip + BCE + the head's backward, one pass over Z
-            # dZ[:, :n_deep] leaves the head already multiplied by relu'(last hidden layer): it IS dH[nmlp-1]
-            # (its own parameter gradients and the loss are summed on the side stream: only the dense Adam and the
-            # host read them, the tower's backward needs dZ alone)
-            ops.logit_head(self.Z, P["out_W"], P["out_b"], self.labels, self.dZ, G["out_W"], G["out_b"],
-                           p_out=self.p_raw, loss=self.loss, relu_cols=self.n_deep, ws=self.head_ws, defer_reduce=True)
         bw, bb, br = self.branch          # weight gradients | bias gradients | small reductions
-        br.wait_stream(main)
-        with torch.cuda.stream(br):
-            with ph("logits_loss_reduce"):
-                ops.logit_head_reduce(self.head_ws, G["out_W"], G["out_b"], self.loss, B, self.zw)
-        self._stamp("head_end")
-        # MLP backward (relu masks from the saved activations)
-        with ph("mlp_bwd"):
-            for i in reversed(range(nmlp)):
-                # weight / bias gradients are only consumed by the dense Adam at the end of the step: they run as
-                # parallel branches off the dgrad -> InteractingLayer-backward chain (two streams, alternating, for
-                # the weight-gradient GEMMs of successive layers; one for the column sums)
-                # (launched as soon as their inputs exist: deferring them until after the backward leaves the tower's
-                # window to the GEMMs — 11 us — but the tail then outlasts the sparse update by 18 us)
-                sw = bw if (nmlp - 1 - i) % 2 == 0 else br
-                sw.wait_stream(main)
-                with torch.cuda.stream(sw):
-                    with ph("mlp_wgrad"):
-                        ops.gemm(acts[i], self.dH[i], self.G[f"mlp_W{i}"], transA=True)   # x^T dy, operands as they lie
-                bb.wait_stream(main)
-                with torch.cuda.stream(bb):
-                    with ph("mlp_bgrad"):
-                        ops.colsum(self.dH[i], out=self.G[f"mlp_b{i}"])
-                if i > 0:   # dH[i-1] = (dH[i] @ W_i^T) * relu'(h_{i-1}); W_i [in,out] is the K-major B operand
-                    ops.gemm(self.dH[i], self._w(f"mlp_W{i}"), self.dH[i - 1], aux=acts[i],
-                             epilogue=E.EPI_MUL_RELU_MASK, transB=True)
-        self._stamp("mlp_bwd_end")
+        if self.fuse_tower:
+            self._tower_fused(ph, acts, main)
+        else:
+            self._tower(ph, acts, main, B)
         # InteractingLayer backward -> dX, then dX += dH0 @ W0^T
         nW = d * 4 * U
         dparams = self.flat_g[self.spec[0][2]:]       # Wqkvr | bqkvr | gamma | beta are contiguous
@@ -349,9 +330,10 @@ class AutoIntTrainer:
         if self.fused:
             # the tower's input gradient first (plain store into dX); the InteractingLayer backward adds it to its own
             # dX row by row and, multi-GPU, stores the sum straight into the owners' receive buffers
-            with ph("mlp_dgrad_x"):
-                ops.gemm(self.dH[0], self._w("mlp_W0"), self.dX.view(B, F * d), transB=True)
-            self._stamp("mlp_dgrad_x_end")
+            if not self.fuse_tower:
+                with ph("mlp_dgrad_x"):
+                    ops.gemm(self.dH[0], self._w("mlp_W0"), self.dX.view(B, F * d), transB=True)
+                self._stamp("mlp_dgrad_x_end")
             with ph("interacting_bwd"):
                 self._interacting_bwd_fused(None, st, T, main)      # parameter-gradient partials stay in self.ws
         else:
@@ -395,6 +377,72 @@ class AutoIntTrainer:
         if getattr(self, "_join_side2", False):      # peer-gather barrier stream joins the step
             main.wait_stream(self.side2)
         self._stamp("step_end")
+
+    def _tower(self, ph, acts, main, B):
+        """The tower as 4 GEMMs + the head pass (fp32 parity mode, unsupported widths, fuse_tower=False)."""
+        c, E, G, P = self.cfg, cabi, self.G, self.P
+        nmlp = len(c.mlp_hidden)
+        br = self.branch[2]
+        with ph("mlp_fwd"):
+            for i in range(nmlp):
+                self._dense_fwd(acts[i], f"mlp_W{i}", f"mlp_b{i}", acts[i + 1])
+        self._stamp("mlp_fwd_end")
+        with ph("logits_loss"):
+            # final Dense(1, sigmoid) + clip + BCE + the head's backward, one pass over Z
+            # dZ[:, :n_deep] leaves the head already multiplied by relu'(last hidden layer): it IS dH[nmlp-1]
+            # (its own parameter gradients and the loss are summed on the side stream: only the dense Adam and the
+            # host read them, the tower's backward needs dZ alone)
+            ops.logit_head(self.Z, P["out_W"], P["out_b"], self.labels, self.dZ, G["out_W"], G["out_b"],
+                           p_out=self.p_raw, loss=self.loss, relu_cols=self.n_deep, ws=self.head_ws, defer_reduce=True)
+        br.wait_stream(main)
+        with torch.cuda.stream(br):
+            with ph("logits_loss_reduce"):
+                ops.logit_head_reduce(self.head_ws, G["out_W"], G["out_b"], self.loss, B, self.zw)
+        self._stamp("head_end")
+        # MLP backward (relu masks from the saved activations)
+        with ph("mlp_bwd"):
+            for i in reversed(range(nmlp)):
+                self._tower_param_grads(ph, acts, main, i)
+                if i > 0:   # dH[i-1] = (dH[i] @ W_i^T) * relu'(h_{i-1}); W_i [in,out] is the K-major B operand
+                    ops.gemm(self.dH[i], self._w(f"mlp_W{i}"), self.dH[i - 1], aux=acts[i],
+                             epilogue=E.EPI_MUL_RELU_MASK, transB=True)
+        self._stamp("mlp_bwd_end")
+
+    def _tower_fused(self, ph, acts, main):
+        """The tower (both Dense(relu) layers, head, their backward down to dX) as one launch; the parameter gradients
+        and the head's loss are side branches."""
+        c, P, G = self.cfg, self.P, self.G
+        B = c.batch
+        br = self.branch[2]
+        with ph("tower"):
+            ops.tower_step(acts[0], self.WT16["mlp_W0"], self.WT16["mlp_W1"], self.P16["mlp_W0"], self.P16["mlp_W1"],
+                           P["mlp_b0"], P["mlp_b1"], P["out_W"], P["out_b"], self.labels, self.Z, self.p_raw, self.dZ,
+                           self.H[0], self.dH[0], self.dX.view(B, -1))
+        self._stamp("tower_end")
+        br.wait_stream(main)
+        with torch.cuda.stream(br):
+            with ph("logits_loss_reduce"):
+                ops.logit_head_grad(self.Z, self.p_raw, self.labels, self.head_ws)
+                ops.logit_head_reduce(self.head_ws, G["out_W"], G["out_b"], self.loss, B, self.zw)
+        for i in reversed(range(len(c.mlp_hidden))):
+            self._tower_param_grads(ph, acts, main, i)
+
+    def _tower_param_grads(self, ph, acts, main, i):
+        # weight / bias gradients are only consumed by the dense Adam at the end of the step: they run as parallel
+        # branches off the dgrad -> InteractingLayer-backward chain (two streams, alternating, for the weight-gradient
+        # GEMMs of successive layers; one for the column sums)
+        # (launched as soon as their inputs exist: deferring them until after the backward leaves the tower's
+        # window to the GEMMs — 11 us — but the tail then outlasts the sparse update by 18 us)
+        bw, bb, br = self.branch
+        sw = bw if (len(self.cfg.mlp_hidden) - 1 - i) % 2 == 0 else br
+        sw.wait_stream(main)
+        with torch.cuda.stream(sw):
+            with ph("mlp_wgrad"):
+                ops.gemm(acts[i], self.dH[i], self.G[f"mlp_W{i}"], transA=True)   # x^T dy, operands as they lie
+        bb.wait_stream(main)
+        with torch.cuda.stream(bb):
+            with ph("mlp_bgrad"):
+                ops.colsum(self.dH[i], out=self.G[f"mlp_b{i}"])
 
     def _stamp(self, name):
         """Measurement aid (tools/step_timeline.py): with `self.stamps` set to an int64 device buffer, a one-thread

@@ -92,6 +92,9 @@ PROTOTYPES = {
     "rs_logit_head_fwd_bwd": (_i, [_p, _i64, _i, _p, _p, _p, _f, _p, _p, _p, _i64, _p, _p, _i, _i, _p, _sz, _p]),
     "rs_logit_head_fwd_bwd_relu": (_i, [_p, _i64, _i, _p, _p, _p, _f, _p, _p, _p, _i64, _p, _p, _i, _i, _i, _p, _sz, _p]),
     "rs_logit_head_reduce": (_i, [_p, _sz, _p, _p, _p, _i, _i, _p]),
+    "rs_logit_head_grad": (_i, [_p, _i64, _i, _p, _p, _f, _i, _i, _p, _sz, _p]),
+    "rs_tower_supported": (_i, [_i, _i, _i, _i]),
+    "rs_tower_step": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _f, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p]),
     "rs_cross_workspace_bytes": (_sz, [_i, _i, _i]),
     "rs_cross_fwd": (_i, [_p, _i64, _i, _p, _p, _p, _i64, _i, _i, _i, _p, _sz, _p]),
     "rs_cross_bwd": (_i, [_p, _i64, _p, _i64, _i, _p, _p, _p, _i64, _p, _p, _i, _i, _i, _p, _sz, _p]),

@@ -423,8 +423,8 @@ static EncodeTiledFn encode_fn() {
   return fn;
 }
 
-// 2-D bf16 row-major [rows, cols] with leading dim ld (elements); box = 64 cols x box_rows rows.
-static int make_map(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
+// 2-D bf16 row-major [rows, cols] with leading dim ld (elements); box = 64 cols x box_rows rows, SWIZZLE_128B.
+int make_map(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
   EncodeTiledFn fn = encode_fn();
   if (!fn) { set_error("gemm_tc: cuTensorMapEncodeTiled unavailable"); return RS_ERR_UNSUPPORTED; }
   cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};

@@ -13,7 +13,9 @@ namespace rs {
 
 constexpr int HEAD_WARPS = 8;
 
-template <int NV, typename T>
+// FROM_P: the forward and dZ were computed elsewhere (tower.cu): p is read from p_out (the stored bf16 activation,
+// the value every derivative below starts from) and only the partials of dw / db / loss are produced.
+template <int NV, typename T, bool FROM_P = false>
 __global__ void __launch_bounds__(HEAD_WARPS * 32)
 logit_head_kernel(const T* __restrict__ Z, int64_t ldz, const float* __restrict__ w,
                   const float* __restrict__ bias, const float* __restrict__ y, float a,
@@ -27,11 +29,11 @@ logit_head_kernel(const T* __restrict__ Z, int64_t ldz, const float* __restrict_
     const int c = (i * 32 + lane) * 4;
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
-      wv[i][u] = (c + u < zw) ? w[c + u] : 0.f;
+      wv[i][u] = (!FROM_P && c + u < zw) ? w[c + u] : 0.f;
       dw[i][u] = 0.f;
     }
   }
-  const float b0 = bias[0];
+  const float b0 = FROM_P ? 0.f : bias[0];
   const float invB = 1.f / (float)B;
   float db = 0.f, loss = 0.f;
   // rows are software-pipelined: the next row's loads are in flight while the current row is reduced
@@ -56,26 +58,31 @@ logit_head_kernel(const T* __restrict__ Z, int64_t ldz, const float* __restrict_
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
         z[i][u] = zn[i][u];
-        dot = fmaf(z[i][u], wv[i][u], dot);
+        if (!FROM_P) dot = fmaf(z[i][u], wv[i][u], dot);
       }
     }
     load_row(r + rstep, zn);
-    dot = warp_sum(dot);
-    const float pr = 1.f / (1.f + expf(-(dot + b0)));
-    const float prs = to_f<T>(from_f<T>(pr));        // the stored activation (bf16-rounded in bf16 mode)
+    float pr, prs;
+    if constexpr (FROM_P) {
+      pr = prs = to_f<T>(p_out[r]);
+    } else {
+      dot = warp_sum(dot);
+      pr = 1.f / (1.f + expf(-(dot + b0)));
+      prs = to_f<T>(from_f<T>(pr));                  // the stored activation (bf16-rounded in bf16 mode)
+    }
     const float p = fminf(fmaxf(prs, 1e-6f), 1.0f);
     const float yy = y[r];
     loss += -yy * logf(p + 1e-6f) - (a - yy) * logf(1.0f - p + 1e-6f);
     const float dp = (-yy / (p + 1e-6f) + (a - yy) / (1.0f - p + 1e-6f)) * invB;
     const float dz = (prs >= 1e-6f && prs <= 1.0f) ? dp * prs * (1.f - prs) : 0.f;
     db += dz;
-    if (lane == 0) p_out[r] = from_f<T>(pr);
+    if (!FROM_P && lane == 0) p_out[r] = from_f<T>(pr);
 #pragma unroll
     for (int i = 0; i < NV; ++i) {
       const int c = (i * 32 + lane) * 4;
 #pragma unroll
       for (int u = 0; u < 4; ++u) dw[i][u] = fmaf(dz, z[i][u], dw[i][u]);
-      if (c < zw) {
+      if (!FROM_P && c < zw) {
         float o[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
@@ -177,6 +184,34 @@ int rs_logit_head_fwd_bwd_relu(const void* Z, int64_t ldz, int dtype, const floa
   // complete here)
   if (dw == nullptr) return 0;
   return rs_logit_head_reduce(ws, ws_bytes, dw, db, loss_out, B, zw, stream);
+}
+
+int rs_logit_head_grad(const void* Z, int64_t ldz, int dtype, const void* p, const float* y, float a, int B, int zw,
+                       void* ws, size_t ws_bytes, void* stream) {
+  RS_REQUIRE(B > 0 && zw > 0 && zw % 4 == 0 && zw <= 2048, "logit_head_grad: B=%d zw=%d (zw %% 4 == 0, <= 2048)", B, zw);
+  RS_REQUIRE(ldz % 4 == 0, "logit_head_grad: leading dim must be a multiple of 4");
+  RS_REQUIRE(dtype == RS_F32 || dtype == RS_BF16, "logit_head_grad: bad dtype");
+  if (ws_bytes < rs_logit_head_workspace_bytes(B, zw)) { set_error("logit_head_grad: workspace too small"); return RS_ERR_WORKSPACE; }
+  cudaStream_t st = as_stream(stream);
+  const int grid = head_grid(B);
+  const size_t smem = (size_t)HEAD_WARPS * (zw + 2) * sizeof(float);
+  const int nv = (int)cdiv(zw, 128);
+#define RS_HEADG_GO(NV, TT)                                                                                \
+  do {                                                                                                     \
+    auto kern = logit_head_kernel<NV, TT, true>;                                                           \
+    RS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));           \
+    kern<<<grid, HEAD_WARPS * 32, smem, st>>>((const TT*)Z, ldz, nullptr, nullptr, y, a, (TT*)p, nullptr, 0, \
+                                              (float*)ws, B, zw, 0);                                       \
+  } while (0)
+  if (dtype == RS_F32) {
+    if (nv <= 4) RS_HEADG_GO(4, float); else if (nv <= 6) RS_HEADG_GO(6, float); else if (nv <= 8) RS_HEADG_GO(8, float);
+    else RS_HEADG_GO(16, float);
+  } else {
+    if (nv <= 4) RS_HEADG_GO(4, __nv_bfloat16); else if (nv <= 6) RS_HEADG_GO(6, __nv_bfloat16);
+    else if (nv <= 8) RS_HEADG_GO(8, __nv_bfloat16); else RS_HEADG_GO(16, __nv_bfloat16);
+  }
+#undef RS_HEADG_GO
+  return check_launch("logit_head_grad");
 }
 
 int rs_logit_head_reduce(const void* ws, size_t ws_bytes, float* dw, float* db, float* loss_out, int B, int zw,

@@ -79,6 +79,10 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N) {
 }
 
 
+// Host: TMA map of a 2-D bf16 row-major [rows, cols] tensor (leading dim ld elements), box = 64 cols x box_rows rows,
+// SWIZZLE_128B (gemm_tc.cu).
+int make_map(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_rows);
+
 // Generic-proxy shared-memory writes -> visible to the async proxy (tcgen05.mma / TMA reads).
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 

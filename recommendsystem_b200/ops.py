@@ -425,6 +425,28 @@ def logit_head_reduce(ws, dw, db, loss, B, zw):
     call("rs_logit_head_reduce", _ptr(ws), ws.numel(), _ptr(dw), _ptr(db), _ptr(loss), B, zw, _stream())
 
 
+def logit_head_grad(Z, p, y, ws, a=1.0):
+    """The head's dw / db / loss partials (left in `ws` for logit_head_reduce) from a p computed by tower_step."""
+    B, zw = Z.shape
+    call("rs_logit_head_grad", _ptr(Z), Z.stride(0), _dt(Z), _ptr(p), _ptr(y), a, B, zw, _ptr(ws), ws.numel(), _stream())
+
+
+def tower_supported(K0, N0, N1, Ki) -> bool:
+    return bool(cabi.load().rs_tower_supported(K0, N0, N1, Ki))
+
+
+def tower_step(X, W0T, W1T, W0, W1, b0, b1, w, ob, y, Z, p_out, dZ, H0, dH0, dX, a=1.0):
+    """The tower's part of the bf16 train step in one launch (rs_tower_step): H0, Z[:, :N1], p_out, dZ, dH0 and dX
+    (stored, not accumulated) from X [B, K0] and Z[:, N1:]."""
+    B, K0 = X.shape
+    N0, N1 = W0T.shape[0], W1T.shape[0]
+    Ki = Z.shape[1] - N1
+    for t in (X, W0T, W1T, W0, W1, Z, dZ, H0, dH0, dX):
+        _need(t.dtype == torch.bfloat16 and t.is_contiguous(), "tower_step: contiguous bf16 operands")
+    call("rs_tower_step", _ptr(X), _ptr(W0T), _ptr(W1T), _ptr(W0), _ptr(W1), _ptr(b0), _ptr(b1), _ptr(w), _ptr(ob),
+         _ptr(y), a, _ptr(Z), _ptr(p_out), _ptr(dZ), _ptr(H0), _ptr(dH0), _ptr(dX), B, K0, N0, N1, Ki, _stream())
+
+
 def colsum(x, out=None):
     _need(x.dim() == 2 and x.stride(1) == 1, "colsum: 2-D row-major view")
     M, N = x.shape

@@ -32,13 +32,15 @@ def main():
     ap.add_argument("--batch", type=int, default=8192)
     ap.add_argument("--reps", type=int, default=20)
     ap.add_argument("--rows", type=int, default=1_000_000)
+    ap.add_argument("--fuse-tower", type=int, default=1, help="0: the tower as 4 GEMMs + the head pass")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
     torch.cuda.set_device(dev)
     cfg = AutoIntConfig(num_fields=39, rows_per_field=args.rows, embed_dim=16, unit_num=16, head_num=2, layer_num=3,
-                        mlp_hidden=(256, 128), batch=args.batch, dtype="bf16")
+                        mlp_hidden=(256, 128), batch=args.batch, dtype="bf16",
+                        fuse_tower=bool(args.fuse_tower))
     if world > 1:       # torchrun: the row-sharded trainer (rank 0 prints its own timeline)
         import torch.distributed as dist
         from recommendsystem_b200.sharded import ShardedAutoIntTrainer
