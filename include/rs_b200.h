@@ -31,11 +31,13 @@
 extern "C" {
 #endif
 
-#define RS_ABI_VERSION 5   /* 4: + rs_interacting_path; saved buffer grows by the per-head softmax statistics.
+#define RS_ABI_VERSION 6   /* 4: + rs_interacting_path; saved buffer grows by the per-head softmax statistics.
                               5: + deferred parameter-gradient reductions (rs_logit_head_reduce, rs_interacting_bwd_reduce),
-                                 rs_peer_all_to_all_i32, rs_embed_keys_from_rows;
+                                 a peer-store all-to-all of the routed ids, rs_embed_keys_from_rows;
                                  + rs_idmap_insert / _lookup / _rebuild, rs_idmap_count / _evict
-                                 (additions only, same version) */
+                                 (additions only, same version)
+                              6: the peer-store all-to-all of the routed ids is removed (they reach their owners by a
+                                 NCCL all-to-all) */
 
 enum rs_dtype { RS_F32 = 0, RS_BF16 = 1 };
 
@@ -143,13 +145,6 @@ int rs_scatter_rows_peer(const void* src, void* const* peer_recv, int world, int
  * array and spins (acquire loads) until all `world` slots of its own array have reached it.  Everything the rank
  * wrote before (peer stores included) is visible to a peer once that peer leaves the barrier. */
 int rs_peer_barrier(unsigned int* const* peer_flags, int world, int rank, void* stream);
-/* The id half of the exchange over peer memory (replaces all_to_all_single(recv_rows, send_rows), the owners' view of
- * the reference's `dataset.shard` + parameter-server pull, staytime/parse.py:77-79): chunk o (cap int32 row indices,
- * rs_route_ids_padded's send order) of `send` is stored into slot my_rank of peer_recv[o] (HOST array of `world`
- * DEVICE pointers to every rank's [world * cap] receive buffer).  Follow it by rs_peer_barrier on a flag array of its
- * own before the owners read; small CTAs, so it runs beside the persistent InteractingLayer forward. */
-int rs_peer_all_to_all_i32(const int32_t* send, int32_t* const* peer_recv, int world, int my_rank, int cap,
-                           void* stream);
 /* sort_keys[i] = (rowidx[i] << 32 | i) for rs_embed_sort_keys: the keys rs_embed_gather_rows writes as a by-product,
  * without the gather (the owners of a sharded step only need the keys: the rows were read through peer memory). */
 int rs_embed_keys_from_rows(const int32_t* rowidx, int64_t n, uint64_t* sort_keys, void* stream);

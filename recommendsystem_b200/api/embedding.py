@@ -257,13 +257,16 @@ class EmbeddingFeatures:
             elif bag is not None:                                 # mean combiner: 1/count per occurrence
                 b, cnt = bag
                 g = (g.float() / cnt[:, None]).repeat_interleave(b, dim=0)
-            g = g.contiguous()
-            ks = ops.sort_keys(keys, self.row_bits)
-            if isinstance(self.opt, Adam):
-                ops.segsum_adam(self.table, self.m, self.v, g, ks, self.opt.learning_rate, self.opt.beta1,
-                                self.opt.beta2, self.opt.epsilon, self.scalars)
-            else:
-                ops.segsum_adagrad(self.table, self.g2sum, g, ks, self.opt.learning_rate, self.opt.epsilon,
-                                   self.opt.per_element)
+            self._sparse_update(g.contiguous(), ops.sort_keys(keys, self.row_bits))
         self._last = None
         self._pending_backward = False
+
+    def _sparse_update(self, grad, keys_sorted, grad_scale=1.0):
+        """Sorted-segment sum of the gradient rows `grad` + the sparse optimizer on the rows `keys_sorted` names."""
+        o = self.opt
+        if isinstance(o, Adam):
+            ops.segsum_adam(self.table, self.m, self.v, grad, keys_sorted, o.learning_rate, o.beta1, o.beta2, o.epsilon,
+                            self.scalars, grad_scale=grad_scale)
+        else:
+            ops.segsum_adagrad(self.table, self.g2sum, grad, keys_sorted, o.learning_rate, o.epsilon, o.per_element,
+                               grad_scale=grad_scale)

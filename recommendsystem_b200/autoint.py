@@ -16,6 +16,7 @@ comes from librs_b200.so.  There is no CPU path.
 """
 from __future__ import annotations
 
+from contextlib import contextmanager
 from dataclasses import dataclass, field
 from typing import List, Sequence
 
@@ -202,8 +203,7 @@ class AutoIntTrainer:
     @property
     def fuse_tower(self) -> bool:
         """The tower runs as one launch (rs_tower_step).  Only beside the fused InteractingLayer backward, which adds
-        its own part to the dX the tower kernel stores; read at step time, so a subclass that turns `fused` off (the
-        all-NCCL sharded path) also gets the separate tower kernels."""
+        its own part to the dX the tower kernel stores."""
         return self._tower_ok and self.fused
 
     # ------------------------------------------------------------------ setup
@@ -267,8 +267,7 @@ class AutoIntTrainer:
         E = cabi
         st = ops._stream()
         T = ops._DT[self.act_dtype]
-        P, G = self.P, self.G
-        nmlp = len(c.mlp_hidden)
+        P = self.P
         ph = lambda name: _Phase(self.timer, name)
         main = torch.cuda.current_stream(self.dev)
         self._stamp("step_begin")
@@ -288,24 +287,19 @@ class AutoIntTrainer:
                     self.idmap.count(self.ids_rows)
         if self.fused:
             # K1 inside K4: the forward's tile loader reads the embedding rows itself (local table, or the owners' HBM
-            # over NVLink) and writes X and the sort keys as by-products; only the owners' key work (multi-GPU) is a
-            # separate branch
-            self._embed_forward(ph, st, T, gather=False)
+            # over NVLink) and writes X and (one GPU) the sort keys as by-products
             tabs, world, lbase_t, keys = self._lookup_args()
             lk_ids, _, lk_rows = self.lookup
-            with ph("interacting_fwd"):
+            with self._backward_keys(ph), ph("interacting_fwd"):
                 cabi.call("rs_interacting_fwd_gather", tabs, self.table_ld, world, lk_ids.data_ptr(), lbase_t.data_ptr(),
                           lk_rows.data_ptr(), self.X.data_ptr(), d, 0, keys, T, P["Wqkvr"].data_ptr(),
                           P["bqkvr"].data_ptr(), P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps,
                           self.Z[:, self.n_deep:].data_ptr(), U, self.zw, self.saved.data_ptr(), B, F, d, U,
                           c.head_num, c.layer_num, int(c.use_res), st)
-            self._sort_keys(ph)
         else:
             # K1: gather (+ sort keys emitted for the backward)
-            self._embed_forward(ph, st, T)
-            # the key sort only needs the forward's keys: run it on the side stream, hidden behind the
-            # dense forward/backward (a parallel branch of the captured graph)
-            self._sort_keys(ph)
+            with self._backward_keys(ph):
+                self._embed_forward(ph, st, T)
             # K4: InteractingLayer forward
             with ph("interacting_fwd"):
                 # writes Flatten(A) straight into its columns of the concat buffer Z (autoint:36,45)
@@ -374,8 +368,6 @@ class AutoIntTrainer:
         main.wait_stream(self.side)
         for sj in self.branch:
             main.wait_stream(sj)
-        if getattr(self, "_join_side2", False):      # peer-gather barrier stream joins the step
-            main.wait_stream(self.side2)
         self._stamp("step_end")
 
     def _tower(self, ph, acts, main, B):
@@ -452,16 +444,20 @@ class AutoIntTrainer:
         i = self.stamp_names.setdefault(name, len(self.stamp_names))
         cabi.call("rs_debug_timestamp", self.stamps[i:].data_ptr(), ops._stream())
 
-    def _sort_keys(self, ph):
-        main = torch.cuda.current_stream(self.dev)
-        self.side.wait_stream(main)
+    # ---- embedding halves of the step (overridden by the row-sharded multi-GPU trainer)
+    @contextmanager
+    def _backward_keys(self, ph):
+        """Around the launch that makes the sort keys for the sparse update (the gather, or the forward with the lookup
+        inside): the key sort follows it on the side stream, hidden behind the dense forward / backward (a parallel
+        branch of the captured graph)."""
+        yield
+        self.side.wait_stream(torch.cuda.current_stream(self.dev))
         with torch.cuda.stream(self.side):
             with ph("sort_keys"):
                 ops.sort_keys(self.keys, self.row_bits, out=self.keys_sorted)
             self.sort_done.record(self.side)
             self._stamp("side_sort_end")
 
-    # ---- embedding halves of the step (overridden by the row-sharded multi-GPU trainer)
     def _lookup_args(self):
         """(address of the W table pointers, W, per-field local row base, sort-key buffer) of the fused lookup."""
         if not hasattr(self, "_tab1"):
@@ -487,11 +483,10 @@ class AutoIntTrainer:
                   c.head_num, c.layer_num,
                   int(c.use_res), self.ws.data_ptr(), self.ws.numel(), st)
 
-    def _embed_forward(self, ph, st, T, gather=True):
+    def _embed_forward(self, ph, st, T):
+        """The separate gather: X and the sort keys."""
         c = self.cfg
         n = c.batch * c.num_fields
-        if not gather:
-            return
         ids, base, rows = self.lookup
         with ph("embed_gather"):
             cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(),
@@ -499,11 +494,15 @@ class AutoIntTrainer:
                       self.keys.data_ptr(), None, st)
 
     def _embed_backward(self, ph, st, T, main):
-        c = self.cfg
         main.wait_event(self.sort_done)        # sorted keys (not the dense work queued behind them)
         with ph("embed_segsum_adam"):
-            ops.segsum_adam(self.table, self.table_m, self.table_v, self.dX.view(-1, c.embed_dim), self.keys_sorted,
-                            c.lr_sparse, c.beta1, c.beta2, c.eps, self.adam_scalars)
+            self._sparse_update(self.dX.view(-1, self.cfg.embed_dim), self.keys_sorted)
+
+    def _sparse_update(self, grad, keys_sorted, grad_scale=1.0):
+        """Sorted-segment sum of the gradient rows + sparse Adam on the rows `keys_sorted` names."""
+        c = self.cfg
+        ops.segsum_adam(self.table, self.table_m, self.table_v, grad, keys_sorted, c.lr_sparse, c.beta1, c.beta2, c.eps,
+                        self.adam_scalars, grad_scale=grad_scale)
 
     def _dense_sync(self, ph):
         """Single GPU: nothing to exchange.  (Multi-GPU: all-reduce of the flat dense gradient.)"""
@@ -525,15 +524,6 @@ class AutoIntTrainer:
             ops.gemm(x, self.WT16[wname], out, bias=self.P[bname], epilogue=cabi.EPI_BIAS_RELU, transB=True)
         else:
             ops.gemm(x, self.P[wname], out, bias=self.P[bname], epilogue=cabi.EPI_BIAS_RELU)
-
-    def _wgrad(self, x, dy, wname, bname):
-        """G[w] = x^T dy ; G[b] = colsum(dy)."""
-        if self.bf16:
-            # MN-major TMA/UMMA operands: x [B,in] and dy [B,out] are read as they lie (no transposes)
-            ops.gemm(x, dy, self.G[wname], transA=True)
-        else:
-            ops.gemm(x, dy, self.G[wname], transA=True)
-        ops.colsum(dy, out=self.G[bname])
 
     def evict(self, threshold: float, decay: float = 1.0):
         """Hash mode: show = show * decay for every id, then drop the ids whose show is below `threshold`; their rows
@@ -670,7 +660,7 @@ class AutoIntTrainer:
     @torch.no_grad()
     def predict(self, ids: torch.Tensor) -> torch.Tensor:
         """Forward only on this rank's batch (clip(sigmoid) probabilities), eager launches.  Hash mode: ids are looked
-        up, never inserted (unseen ids read as zero vectors).  Sharded: collective, every rank must call it."""
+        up, never inserted (unseen ids read as zero vectors).  Sharded: the rows are read from the owners' shards."""
         c = self.cfg
         F, d, U, B = c.num_fields, c.embed_dim, c.unit_num, c.batch
         assert ids.shape == (B, F)

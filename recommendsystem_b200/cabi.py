@@ -15,6 +15,7 @@ RS_F32, RS_BF16 = 0, 1
  EPI_ACCUM) = range(7)
 DIN_A, DIN_B = 0, 1
 PATH_NONE, PATH_FFMA, PATH_TCGEN05 = 0, 1, 2
+RS_MAX_PEERS = 8          # ranks a peer-memory kernel addresses (one NVSwitch domain)
 
 _p, _i, _i64, _f, _sz, _u64 = C.c_void_p, C.c_int, C.c_int64, C.c_float, C.c_size_t, C.c_uint64
 
@@ -36,7 +37,6 @@ PROTOTYPES = {
     "rs_embed_gather_peer_fwd": (_i, [_p, _i64, _i, _p, _p, _p, _i64, _i, _i, _p, _i, _p]),
     "rs_scatter_rows_peer": (_i, [_p, _p, _i, _i, _p, _i64, _i, _i, _p]),
     "rs_peer_barrier": (_i, [_p, _i, _i, _p]),
-    "rs_peer_all_to_all_i32": (_i, [_p, _p, _i, _i, _i, _p]),
     "rs_embed_keys_from_rows": (_i, [_p, _i64, _p, _p]),
     "rs_ipc_export": (_i, [_p, _p, _p]),
     "rs_ipc_import": (_i, [_p, _u64, _p]),

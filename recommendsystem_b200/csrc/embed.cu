@@ -768,20 +768,6 @@ __global__ void scatter_rows_peer_kernel(const uint2* __restrict__ src, PeerBufs
   o[((int64_t)my_rank * cap + k) * vec_per_row + c] = src[i * vec_per_row + c];
 }
 
-// All-to-all of equal int32 chunks over peer memory: chunk o of `send` goes to slot `my_rank` of rank o's receive buffer
-// (what all_to_all_single(recv, send) does, as peer stores).  128-thread CTAs: runs beside the persistent forward.
-struct PeerI32 { int32_t* p[RS_MAX_PEERS]; };
-
-__global__ void __launch_bounds__(128) peer_all_to_all_i32_kernel(const int32_t* __restrict__ send, PeerI32 dst, int world,
-                                                                  int my_rank, int cap) {
-  const int64_t total = (int64_t)world * cap;
-  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
-    const int o = (int)(t / cap);
-    const int k = (int)(t - (int64_t)o * cap);
-    dst.p[o][(int64_t)my_rank * cap + k] = send[t];
-  }
-}
-
 // sort keys of the owners' received row indices: (row << 32 | slot); row -1 (padding) sorts last
 __global__ void __launch_bounds__(128) keys_from_rows_kernel(const int32_t* __restrict__ rowidx, int64_t n,
                                                              uint64_t* __restrict__ keys) {
@@ -824,19 +810,6 @@ int rs_peer_barrier(unsigned int* const* peer_flags, int world, int rank, void* 
   for (int r = 0; r < RS_MAX_PEERS; ++r) f.p[r] = r < world ? peer_flags[r] : nullptr;
   peer_barrier_kernel<<<1, 32, 0, as_stream(stream)>>>(f, world, rank);
   return check_launch("peer_barrier");
-}
-
-int rs_peer_all_to_all_i32(const int32_t* send, int32_t* const* peer_recv, int world, int my_rank, int cap,
-                           void* stream) {
-  RS_REQUIRE(world >= 1 && world <= RS_MAX_PEERS && my_rank >= 0 && my_rank < world && cap > 0,
-             "peer_all_to_all_i32: world=%d rank=%d cap=%d", world, my_rank, cap);
-  RS_REQUIRE(send != nullptr && peer_recv != nullptr, "peer_all_to_all_i32: null argument");
-  PeerI32 dst;
-  for (int r = 0; r < RS_MAX_PEERS; ++r) dst.p[r] = r < world ? peer_recv[r] : nullptr;
-  int64_t blocks = cdiv((int64_t)world * cap, 128 * 4);
-  if (blocks > (int64_t)sm_count() * 8) blocks = (int64_t)sm_count() * 8;
-  peer_all_to_all_i32_kernel<<<(unsigned)blocks, 128, 0, as_stream(stream)>>>(send, dst, world, my_rank, cap);
-  return check_launch("peer_all_to_all_i32");
 }
 
 int rs_embed_keys_from_rows(const int32_t* rowidx, int64_t n, uint64_t* sort_keys, void* stream) {

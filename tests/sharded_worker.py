@@ -99,7 +99,7 @@ def main():
         worst = max(int(np.sum(owner[r * b:(r + 1) * b] == o)) for r in range(world) for o in range(world))
         capacity = worst if capmode == "tight" else worst - 1
     sh = ShardedAutoIntTrainer(AutoIntConfig(batch=b, **kw), dev, global_tables=torch.from_numpy(table), capacity=capacity)
-    print(f"[rank {rank}] world {world} dtype {dtype} b {b} cap {sh.cap} ({capmode}) peer_gather {sh.peer_gather} "
+    print(f"[rank {rank}] world {world} dtype {dtype} b {b} cap {sh.buckets.cap} ({capmode}) fused {sh.fused} "
           f"graph {use_graph}", flush=True)
     dense0 = sh.dense_state()
     steps = 3

@@ -24,7 +24,7 @@ def test_header_declares_entry_points():
         assert must in names
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_exports_every_declared_symbol_at_abi_v6():
     from recommendsystem_b200 import cabi
     if not cabi.LIB_PATH.exists():
         pytest.skip("library not built (run __graft_entry__.build())")
@@ -34,7 +34,7 @@ def test_library_exports_every_declared_symbol():
     exported = set(re.findall(r"\bT (rs_[a-z0-9_]+)", out))
     declared = set(_declared())
     assert declared <= exported, sorted(declared - exported)
-    assert lib.rs_abi_version() == 5 and lib.rs_built_for_sm100a() == 1
+    assert lib.rs_abi_version() == 6 and lib.rs_built_for_sm100a() == 1
 
 
 def test_prototype_table_matches_header():

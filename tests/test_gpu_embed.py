@@ -293,28 +293,24 @@ def test_embed_gather_peer_sharded_layout(cuda_dev, W, d, odt):
     assert float(got[5, 2].abs().sum()) == 0.0
 
 
-@pytest.mark.parametrize("W,cap", [(1, 1000), (2, 333), (8, 4101)])
-def test_peer_all_to_all_i32_and_keys(cuda_dev, W, cap):
-    """The id half of the sharded exchange as peer stores: W "ranks" resident on this GPU (CUDA-IPC mappings in the
-    multi-process trainer) — chunk o of rank r's send buffer must land in slot r of rank o's receive buffer, i.e. what
-    all_to_all_single computes; and rs_embed_keys_from_rows = the keys rs_embed_gather_rows writes (row << 32 | slot)."""
-    import ctypes
+@pytest.mark.parametrize("n", [1, 1000, 666, 32808, 300001])
+def test_embed_keys_from_rows(cuda_dev, n):
+    """The owners' sort keys of the sharded exchange: rs_embed_keys_from_rows = (row << 32 | slot), padding (row -1)
+    included, = the keys rs_embed_gather_rows_ld writes as a by-product of a gather by the same rows."""
     from recommendsystem_b200 import cabi, ops
-    rng = np.random.default_rng(W * 7 + cap)
-    send = [torch.from_numpy(rng.integers(-1, 2 ** 31 - 1, size=W * cap).astype(np.int32)).to(cuda_dev) for _ in range(W)]
-    recv = [torch.full((W * cap,), -5, dtype=torch.int32, device=cuda_dev) for _ in range(W)]
-    ptrs = (ctypes.c_void_p * W)(*[t.data_ptr() for t in recv])
-    for r in range(W):
-        cabi.call("rs_peer_all_to_all_i32", send[r].data_ptr(), ctypes.addressof(ptrs), W, r, cap, ops._stream())
-    torch.cuda.synchronize()
-    for o in range(W):
-        want = torch.cat([send[r][o * cap:(o + 1) * cap] for r in range(W)])
-        assert torch.equal(recv[o], want)
-    keys = torch.empty(W * cap, dtype=torch.int64, device=cuda_dev)
-    cabi.call("rs_embed_keys_from_rows", recv[0].data_ptr(), W * cap, keys.data_ptr(), ops._stream())
-    rows = recv[0].cpu().numpy().astype(np.int64)
-    want = ((rows & 0xFFFFFFFF) << 32) | np.arange(W * cap, dtype=np.int64)
+    rng = np.random.default_rng(n)
+    R, d = 5000, 16
+    rowidx = rng.integers(-1, R, size=n).astype(np.int32)
+    rows = torch.from_numpy(rowidx).to(cuda_dev)
+    keys = torch.empty(n, dtype=torch.int64, device=cuda_dev)
+    cabi.call("rs_embed_keys_from_rows", rows.data_ptr(), n, keys.data_ptr(), ops._stream())
+    want = ((rowidx.astype(np.int64) & 0xFFFFFFFF) << 32) | np.arange(n, dtype=np.int64)
     assert np.array_equal(keys.cpu().numpy().view(np.uint64), want.view(np.uint64))
+    table = torch.zeros(R, 3, d, device=cuda_dev)[:, 0, :]
+    keys_gather = torch.empty_like(keys)
+    cabi.call("rs_embed_gather_rows_ld", table.data_ptr(), table.stride(0), rows.data_ptr(), n, d, None, cabi.RS_F32,
+              None, keys_gather.data_ptr(), ops._stream())
+    assert torch.equal(keys, keys_gather)
 
 
 @pytest.mark.parametrize("d", [8, 16, 32])

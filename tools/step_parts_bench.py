@@ -26,8 +26,10 @@ parts = {
     "mlp_dgrad1 8192x128->256 (+relu mask)": lambda: ops.gemm(tr.dH[1], tr._w("mlp_W1"), tr.dH[0], aux=acts[1],
                                                                epilogue=E.EPI_MUL_RELU_MASK, transB=True),
     "mlp_dgrad_x 8192x256->624": lambda: ops.gemm(tr.dH[0], tr._w("mlp_W0"), tr.dX.view(B, F * d), transB=True),
-    "mlp_wgrad0 (side stream)": lambda: tr._wgrad(acts[0], tr.dH[0], "mlp_W0", "mlp_b0"),
-    "mlp_wgrad1 (side stream)": lambda: tr._wgrad(acts[1], tr.dH[1], "mlp_W1", "mlp_b1"),
+    "mlp_wgrad0 (side stream)": lambda: (ops.gemm(acts[0], tr.dH[0], tr.G["mlp_W0"], transA=True),
+                                         ops.colsum(tr.dH[0], out=tr.G["mlp_b0"])),
+    "mlp_wgrad1 (side stream)": lambda: (ops.gemm(acts[1], tr.dH[1], tr.G["mlp_W1"], transA=True),
+                                         ops.colsum(tr.dH[1], out=tr.G["mlp_b1"])),
     "sort_keys (side stream)": lambda: ops.sort_keys(tr.keys, tr.row_bits, out=tr.keys_sorted),
     "dense_adam + shadows (side stream)": lambda: (ops.dense_adam(tr.flat, tr.flat_m, tr.flat_v, tr.flat_g, 1e-3, 0.9, 0.999, 1e-8,
                                                                   tr.adam_scalars, tr.flat_bf16), tr._refresh_wt()),
