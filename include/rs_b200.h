@@ -405,6 +405,18 @@ int rs_interacting_fwd_gather(const float* const* peer_tables, int64_t table_ld,
                               const float* ln_gamma, const float* ln_beta, float ln_eps,
                               void* y, int64_t y_ld, int64_t y_bs, void* saved,
                               int B, int F, int D, int U, int H, int L, int use_res, void* stream);
+/* Bags in the fused lookup (one GPU, the local table): ids [B, S] int64, field f owning the slots
+ * [slot_off[f], slot_off[f+1]) of every sample (slot_off: F + 1 device int64, slot_off[F] = S, B * S < 2^31); id < 0 =
+ * padding.  x_out[b, f] = RNE(dtype) of the mean of the rows of the bag's valid ids (fp32 sum in slot order times
+ * 1 / count; an empty bag is zeros), inv_cnt[b * F + f] = 1 / count (0 for an empty bag) and, if not NULL,
+ * sort_keys[p] = (row << 32 | p) for slot p = b * S + slot_off[f] + k (all-ones for padding): bit-identical to
+ * rs_embed_bag_fwd_ld with offsets[b * F + f] = b * S + slot_off[f] followed by rs_interacting_fwd. */
+int rs_interacting_fwd_gather_bag(const float* table, int64_t table_ld, const int64_t* ids, const int64_t* slot_off,
+                                  const int64_t* row_base, const int64_t* rows, void* x_out, int64_t x_ld, int64_t x_bs,
+                                  unsigned long long* sort_keys, float* inv_cnt, int dtype, const float* Wqkvr,
+                                  const float* bqkvr, const float* ln_gamma, const float* ln_beta, float ln_eps,
+                                  void* y, int64_t y_ld, int64_t y_bs, void* saved,
+                                  int B, int F, int S, int D, int U, int H, int L, int use_res, void* stream);
 /* The backward with the embedding-gradient exchange fused in (tensor-core path only): dx_add (may be NULL) is added
  * to the layer's input gradient row by row (the MLP tower's dX, same strides as dx; dx_add == dx is allowed), and when
  * `inverse` is not NULL the finished row of lookup i is stored straight into slot (rank * cap + inverse[i] mod cap) of

@@ -1,8 +1,8 @@
 """AutoInt train step on one B200: the reference's CTR hot path as one captured stream of
 hand-written sm_100a kernels (include/rs_b200.h).
 
-    ids [B,F] -> embedding gather -> X [B,F,d] --+-> InteractingLayer (L x, shared weights) -> A
-                                                 +-> Flatten -> MultiLayerDense(relu)       -> deep
+    ids [B,S] -> embedding gather / bag mean -> X [B,F,d] --+-> InteractingLayer (L x, shared weights) -> A
+                                                            +-> Flatten -> MultiLayerDense(relu)       -> deep
     Z = concat[deep, Flatten(A)] -> Dense(1, sigmoid) -> clip(1e-6, 1) -> cross_entropy
     backward -> dense Adam (flat buffer) + sorted-segment sparse Adam on the touched rows
 
@@ -97,6 +97,10 @@ class AutoIntConfig:
     # bf16 mode with the fused lookup: the whole tower (both Dense(relu) layers, the logit head and their backward
     # down to dX) as one launch (rs_tower_step) where the kernel exists for the widths; False = 4 GEMMs + the head pass
     fuse_tower: bool = True
+    # multi-valued fields (VarLenFeature ids, combiner='mean'): the most ids field f takes per sample (int: every field).
+    # Field f owns the columns [off_f, off_f + K_f) of the [B, S] id input (S = sum K, off = exclusive cumsum of K); an
+    # id < 0 is padding and X[b, f] is the mean of the rows of the bag's valid ids (zeros for an empty bag)
+    bag_size: int | Sequence[int] = 1
 
     def rows(self) -> List[int]:
         if isinstance(self.rows_per_field, int):
@@ -104,12 +108,30 @@ class AutoIntConfig:
         assert len(self.rows_per_field) == self.num_fields
         return list(self.rows_per_field)
 
+    def bags(self) -> List[int]:
+        """K_f per field; ValueError for a length other than num_fields or a K_f < 1."""
+        if isinstance(self.bag_size, (int, np.integer)):
+            K = [int(self.bag_size)] * self.num_fields
+        else:
+            K = [int(k) for k in self.bag_size]
+            if len(K) != self.num_fields:
+                raise ValueError(f"bag_size has {len(K)} entries for {self.num_fields} fields")
+        if any(k < 1 for k in K):
+            raise ValueError(f"bag_size: every field takes at least one id, got {K}")
+        return K
+
 
 class AutoIntTrainer:
     """Owns tables, optimizer state and dense parameters; `step()` launches one train step."""
 
     def __init__(self, cfg: AutoIntConfig, device="cuda:0", tables: torch.Tensor | None = None,
                  dense_init: dict | None = None):
+        self.K = cfg.bags()
+        self.S = sum(self.K)                 # id columns per sample
+        if cfg.batch * self.S >= 2 ** 31:
+            raise ValueError(f"batch * sum(bag_size) = {cfg.batch * self.S} slots: sort-key positions are 32-bit")
+        # bags: the step's lookups take the mean over each field's slots; with every K_f = 1 they are plain gathers
+        self.bag = self.S > cfg.num_fields
         cabi.load()
         self.cfg = cfg
         self.dev = torch.device(device)
@@ -152,15 +174,26 @@ class AutoIntTrainer:
         # ---- static activation buffers (fixed addresses => CUDA-graph capturable)
         T = self.act_dtype
         e = lambda *shape, dtype=T: torch.empty(*shape, device=self.dev, dtype=dtype)
-        self.ids = torch.zeros(B, F, dtype=torch.int64, device=self.dev)
+        S = self.S
+        self.ids = torch.zeros(B, S, dtype=torch.int64, device=self.dev)
         # hash mode: the step's first two launches map ids -> arena rows (static buffer) that every lookup reads
-        self.ids_rows = None if self.idmap is None else torch.full((B, F), -1, dtype=torch.int64, device=self.dev)
+        self.ids_rows = None if self.idmap is None else torch.full((B, S), -1, dtype=torch.int64, device=self.dev)
         self.fields = tuple(range(F))
-        # (ids, row_base, rows) the step's embedding lookups read
+        self.slot_fields = tuple(f for f in range(F) for _ in range(self.K[f]))     # field of each id column
+        # (ids, row_base, rows) the step's embedding lookups read (per-field geometry: bags index it by field)
         self.lookup = (self.ids if self.idmap is None else self.ids_rows, *ar.geom(self.fields))
         self.labels = torch.zeros(B, 1, device=self.dev)
         self.X = e(B, F, d)
-        self.keys = torch.empty(B * F, dtype=torch.int64, device=self.dev)
+        self.keys = torch.empty(B * S, dtype=torch.int64, device=self.dev)
+        if self.bag:
+            # bag (b, f) = slots [b S + off_f, b S + off_f + K_f): CSR offsets of the B F bags, 1 / count per bag, and the
+            # per-slot gradient rows the sorted-segment update reads
+            off = np.concatenate([[0], np.cumsum(self.K)]).astype(np.int64)
+            self.slot_off = torch.from_numpy(off).to(self.dev)
+            self.bag_offsets = torch.from_numpy(np.append((np.arange(B, dtype=np.int64)[:, None] * S + off[None, :F])
+                                                          .reshape(-1), B * S)).to(self.dev)
+            self.inv_cnt = torch.zeros(B * F, device=self.dev)
+            self.g_occ = torch.empty(B * S, d, device=self.dev)
         self.keys_sorted = torch.empty_like(self.keys)
         self.saved = ops.interacting_saved(B, F, U, cfg.layer_num, self.dev)
         self.H = [e(B, w) for w in cfg.mlp_hidden[:-1]]
@@ -195,7 +228,7 @@ class AutoIntTrainer:
         self.timer = None               # set to a PhaseTimer for an instrumented (eager) step
         self.stamps, self.stamp_names = None, {}     # set `stamps` to an int64 buffer for tools/step_timeline.py
         n_ws = max(cabi.load().rs_interacting_workspace_bytes(B, F, d, U),
-                   cabi.load().rs_embed_sort_workspace_bytes(B * F),
+                   cabi.load().rs_embed_sort_workspace_bytes(B * S),
                    cabi.load().rs_colsum_workspace_bytes(B, max(widths + [self.zw])))
         self.ws = torch.empty(int(n_ws) + 256, dtype=torch.uint8, device=self.dev)
         self.head_ws = ops.logit_head_workspace(B, self.zw, self.dev)     # head partials, reduced on the side stream
@@ -273,7 +306,7 @@ class AutoIntTrainer:
         self._stamp("step_begin")
         if self.idmap is not None:
             with ph("idmap"):
-                self.store.lookup(self.ids, self.fields, insert=True, out=self.ids_rows)
+                self.store.lookup(self.ids, self.slot_fields, insert=True, out=self.ids_rows)
         # Adam's step counter / bias corrections are read by the two optimizer kernels at the end of the step only:
         # advance them on the side stream now instead of between the backward and the sparse update
         self.side.wait_stream(main)
@@ -291,11 +324,19 @@ class AutoIntTrainer:
             tabs, world, lbase_t, keys = self._lookup_args()
             lk_ids, _, lk_rows = self.lookup
             with self._backward_keys(ph), ph("interacting_fwd"):
-                cabi.call("rs_interacting_fwd_gather", tabs, self.table_ld, world, lk_ids.data_ptr(), lbase_t.data_ptr(),
-                          lk_rows.data_ptr(), self.X.data_ptr(), d, 0, keys, T, P["Wqkvr"].data_ptr(),
-                          P["bqkvr"].data_ptr(), P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps,
-                          self.Z[:, self.n_deep:].data_ptr(), U, self.zw, self.saved.data_ptr(), B, F, d, U,
-                          c.head_num, c.layer_num, int(c.use_res), st)
+                if self.bag:      # the bag means, their 1 / count and the per-slot keys come out of the tile loader
+                    cabi.call("rs_interacting_fwd_gather_bag", self.table.data_ptr(), self.table_ld, lk_ids.data_ptr(),
+                              self.slot_off.data_ptr(), lbase_t.data_ptr(), lk_rows.data_ptr(), self.X.data_ptr(), d, 0,
+                              keys, self.inv_cnt.data_ptr(), T, P["Wqkvr"].data_ptr(), P["bqkvr"].data_ptr(),
+                              P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps, self.Z[:, self.n_deep:].data_ptr(),
+                              U, self.zw, self.saved.data_ptr(), B, F, self.S, d, U, c.head_num, c.layer_num,
+                              int(c.use_res), st)
+                else:
+                    cabi.call("rs_interacting_fwd_gather", tabs, self.table_ld, world, lk_ids.data_ptr(),
+                              lbase_t.data_ptr(), lk_rows.data_ptr(), self.X.data_ptr(), d, 0, keys, T,
+                              P["Wqkvr"].data_ptr(), P["bqkvr"].data_ptr(), P["gamma"].data_ptr(), P["beta"].data_ptr(),
+                              c.ln_eps, self.Z[:, self.n_deep:].data_ptr(), U, self.zw, self.saved.data_ptr(), B, F, d,
+                              U, c.head_num, c.layer_num, int(c.use_res), st)
         else:
             # K1: gather (+ sort keys emitted for the backward)
             with self._backward_keys(ph):
@@ -488,15 +529,29 @@ class AutoIntTrainer:
         c = self.cfg
         n = c.batch * c.num_fields
         ids, base, rows = self.lookup
+        if self.bag:
+            with ph("embed_bag_fwd"):
+                cabi.call("rs_embed_bag_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(),
+                          self.bag_offsets.data_ptr(), base.data_ptr(), rows.data_ptr(), n, c.num_fields, c.embed_dim,
+                          self.X.data_ptr(), T, self.keys.data_ptr(), self.inv_cnt.data_ptr(), st)
+            return
         with ph("embed_gather"):
             cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(),
                       base.data_ptr(), rows.data_ptr(), n, c.num_fields, c.embed_dim, self.X.data_ptr(), T,
                       self.keys.data_ptr(), None, st)
 
     def _embed_backward(self, ph, st, T, main):
+        grad = self.dX.view(-1, self.cfg.embed_dim)
+        if self.bag:
+            # one gradient row per slot, dX[b, f] / count (padding slots are skipped by the segment sum)
+            with ph("embed_bag_grad"):
+                cabi.call("rs_embed_bag_grad", self.dX.data_ptr(), T, self.bag_offsets.data_ptr(),
+                          self.inv_cnt.data_ptr(), self.cfg.batch * self.cfg.num_fields, self.cfg.embed_dim,
+                          self.g_occ.data_ptr(), st)
+            grad = self.g_occ
         main.wait_event(self.sort_done)        # sorted keys (not the dense work queued behind them)
         with ph("embed_segsum_adam"):
-            self._sparse_update(self.dX.view(-1, self.cfg.embed_dim), self.keys_sorted)
+            self._sparse_update(grad, self.keys_sorted)
 
     def _sparse_update(self, grad, keys_sorted, grad_scale=1.0):
         """Sorted-segment sum of the gradient rows + sparse Adam on the rows `keys_sorted` names."""
@@ -535,8 +590,16 @@ class AutoIntTrainer:
         self.idmap.evict(threshold, decay)
 
     # --------------------------------------------------------------- frontends
+    def _check_ids(self, ids):
+        """ids must be [B, S]: S = sum(bag_size) id columns per sample."""
+        if tuple(ids.shape) != tuple(self.ids.shape):
+            raise ValueError(f"ids of shape {tuple(ids.shape)}: the trainer takes [batch, sum(bag_size)] = "
+                             f"{tuple(self.ids.shape)}")
+
     def step(self, ids: torch.Tensor, labels: torch.Tensor) -> torch.Tensor:
-        """Device-resident inputs -> one train step; returns the loss tensor (device, 1 element)."""
+        """Device-resident inputs -> one train step; returns the loss tensor (device, 1 element).  ids [B, S] int64
+        (S = sum(bag_size); field f in the columns [off_f, off_f + K_f)), labels [B, 1]."""
+        self._check_ids(ids)
         self.ids.copy_(ids, non_blocking=True)
         self.labels.copy_(labels, non_blocking=True)
         self.run()
@@ -552,7 +615,7 @@ class AutoIntTrainer:
     def _touched_rows(self) -> torch.Tensor:
         """Arena rows the step on the CURRENT static id buffer updates (sorted unique int64); hash mode: the rows of
         the ids already mapped and every row the step's insert may hand out."""
-        return self.store.touched_rows([(self.ids, self.fields)])
+        return self.store.touched_rows([(self.ids, self.slot_fields)])
 
     def _snapshot(self):
         """Everything one optimizer step changes: the [w|m|v] records of the touched rows, the dense parameters
@@ -593,13 +656,14 @@ class AutoIntTrainer:
 
     def step_from_host(self, ids_pinned: torch.Tensor, labels_pinned: torch.Tensor) -> float:
         """End-to-end call: pinned host ids/labels -> H2D -> step -> loss read back (D2H)."""
+        self._check_ids(ids_pinned)
         self.ids.copy_(ids_pinned, non_blocking=True)
         self.labels.copy_(labels_pinned, non_blocking=True)
         self.run()
         return float(self.loss.item())
 
     def fit_host(self, batches):
-        """End-to-end training loop over an iterable of (ids_pinned [B,F] int64, labels_pinned [B,1] f32) host
+        """End-to-end training loop over an iterable of (ids_pinned [B,S] int64, labels_pinned [B,1] f32) host
         batches; yields one loss (python float) per batch, in order.
 
         Input pipeline: batch n+1's host->device copy runs on a copy stream into the other half of a
@@ -623,6 +687,7 @@ class AutoIntTrainer:
 
         def upload(k, batch):
             ids_h, lab_h = batch
+            self._check_ids(ids_h)
             with torch.cuda.stream(p["copy"]):
                 p["copy"].wait_event(p["free"][k])
                 p["ids"][k].copy_(ids_h, non_blocking=True)
@@ -663,7 +728,7 @@ class AutoIntTrainer:
         up, never inserted (unseen ids read as zero vectors).  Sharded: the rows are read from the owners' shards."""
         c = self.cfg
         F, d, U, B = c.num_fields, c.embed_dim, c.unit_num, c.batch
-        assert ids.shape == (B, F)
+        self._check_ids(ids)
         self.ids.copy_(ids)
         T = ops._DT[self.act_dtype]
         st = ops._stream()
@@ -681,9 +746,15 @@ class AutoIntTrainer:
         return self.p_raw.float().clamp(1e-6, 1.0)
 
     def _predict_lookup(self, st, T):
-        """X = the embedding rows of the static id buffer, inserting no id."""
+        """X = the embedding rows (bags: their means) of the static id buffer, inserting no id."""
         c = self.cfg
-        ids, base, rows = self.store.lookup(self.ids, self.fields, insert=False, out=self.ids_rows)
+        ids = self.store.lookup(self.ids, self.slot_fields, insert=False, out=self.ids_rows)[0]
+        _, base, rows = self.lookup
+        if self.bag:
+            cabi.call("rs_embed_bag_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(),
+                      self.bag_offsets.data_ptr(), base.data_ptr(), rows.data_ptr(), c.batch * c.num_fields,
+                      c.num_fields, c.embed_dim, self.X.data_ptr(), T, None, None, st)
+            return
         cabi.call("rs_embed_gather_fwd_ld", self.table.data_ptr(), self.table_ld, ids.data_ptr(), base.data_ptr(),
                   rows.data_ptr(), c.batch * c.num_fields, c.num_fields, c.embed_dim, self.X.data_ptr(), T, None, None,
                   st)

@@ -65,6 +65,8 @@ PROTOTYPES = {
     "rs_interacting_path": (_i, [_i, _i, _i, _i, _i, _i, _f]),
     "rs_interacting_fwd_gather": (_i, [_p, _i64, _i, _p, _p, _p, _p, _i64, _i64, _p, _i, _p, _p, _p, _p, _f, _p, _i64, _i64, _p,
                                        _i, _i, _i, _i, _i, _i, _i, _p]),
+    "rs_interacting_fwd_gather_bag": (_i, [_p, _i64, _p, _p, _p, _p, _p, _i64, _i64, _p, _p, _i, _p, _p, _p, _p, _f, _p,
+                                           _i64, _i64, _p, _i, _i, _i, _i, _i, _i, _i, _i, _p]),
     "rs_interacting_bwd_scatter": (_i, [_p, _i64, _i64, _p, _i, _p, _p, _p, _p, _f, _p, _i64, _i64, _p, _i64, _i64, _p,
                                         _p, _i, _i, _p, _i, _p, _i, _i, _i, _i, _i, _i, _i, _p, _sz, _p]),
     "rs_interacting_bwd_reduce": (_i, [_p, _sz, _p, _i, _i, _i, _i, _i, _p]),

@@ -94,6 +94,33 @@ int rs_interacting_fwd_gather(const float* const* peer_tables, int64_t table_ld,
   return interacting_tc_fwd(a);
 }
 
+int rs_interacting_fwd_gather_bag(const float* table, int64_t table_ld, const int64_t* ids, const int64_t* slot_off,
+                                  const int64_t* row_base, const int64_t* rows, void* x_out, int64_t x_ld, int64_t x_bs,
+                                  unsigned long long* sort_keys, float* inv_cnt, int dtype, const float* Wqkvr,
+                                  const float* bqkvr, const float* ln_gamma, const float* ln_beta, float ln_eps, void* y,
+                                  int64_t y_ld, int64_t y_bs, void* saved, int B, int F, int S, int D, int U, int H, int L,
+                                  int use_res, void* stream) {
+  RS_REQUIRE(rs_interacting_path(F, D, U, H, dtype, 1, 0.f) == RS_PATH_TCGEN05,
+             "interacting_fwd_gather_bag: only the tensor-core path fuses the lookup (F=%d D=%d U=%d H=%d dtype=%d)", F, D,
+             U, H, dtype);
+  RS_REQUIRE(B > 0 && L >= 1 && S >= F, "interacting_fwd_gather_bag: B=%d L=%d S=%d F=%d", B, L, S, F);
+  RS_REQUIRE((int64_t)B * S < ((int64_t)1 << 31), "interacting_fwd_gather_bag: B*S = %lld slots (32-bit key positions)",
+             (long long)B * S);
+  RS_REQUIRE(table != nullptr && slot_off != nullptr && inv_cnt != nullptr,
+             "interacting_fwd_gather_bag: table, slot offsets and inv_cnt are required");
+  RS_REQUIRE(table_ld >= D && table_ld % 16 == 0, "interacting_fwd_gather_bag: table row stride %lld (64-byte aligned rows)",
+             (long long)table_ld);
+  RS_REQUIRE(x_ld % 4 == 0 && y_ld % 4 == 0, "interacting_fwd_gather_bag: leading dims must be multiples of 4");
+  if (x_bs == 0) x_bs = (int64_t)F * x_ld;
+  if (y_bs == 0) y_bs = (int64_t)F * y_ld;
+  RS_REQUIRE(x_bs % 4 == 0 && y_bs % 4 == 0, "interacting_fwd_gather_bag: batch strides must be multiples of 4");
+  IFwdArgs a{x_out, x_ld, x_bs, Wqkvr, bqkvr, ln_gamma, ln_beta, ln_eps, y, y_ld, y_bs, saved, B, F, L, use_res,
+             dtype, as_stream(stream)};
+  IGatherArgs g{&table, table_ld, 1, ids, row_base, rows, (uint64_t*)sort_keys, slot_off, inv_cnt, S};
+  a.gather = &g;
+  return interacting_tc_fwd(a);
+}
+
 int rs_interacting_bwd_scatter(const void* x, int64_t x_ld, int64_t x_bs, const void* saved, int dtype,
                                const float* Wqkvr, const float* bqkvr, const float* ln_gamma, const float* ln_beta,
                                float ln_eps, const void* dy, int64_t dy_ld, int64_t dy_bs, void* dx, int64_t dx_ld,

@@ -7,6 +7,8 @@ namespace rs {
 struct IGatherArgs {
   const float* const* tables; int64_t table_ld; int world; const int64_t* ids; const int64_t* local_base;
   const int64_t* rows; uint64_t* sort_keys;
+  // bags (rs_interacting_fwd_gather_bag): ids [B, bag_slots], field f owns slots [bag_off[f], bag_off[f+1])
+  const int64_t* bag_off = nullptr; float* inv_cnt = nullptr; int bag_slots = 0;
 };
 // fused gradient push of the tensor-core backward (rs_interacting_bwd_scatter)
 struct IScatterArgs {

@@ -24,6 +24,7 @@
 // backward) and the sort keys as by-products: the gather kernel disappears from the step.
 #include "tc_common.cuh"
 #include "interacting_args.cuh"
+#include <type_traits>
 
 namespace rs {
 
@@ -45,6 +46,17 @@ struct ItcGather {
   uint64_t* keys;            // [B*F] (local arena row << 32 | position) for the sorted-segment update, or NULL
 };
 
+// fused bag mean (rs_interacting_fwd_gather_bag, one GPU): ids [B, S], field f owns the slots [off[f], off[f+1]) of a
+// sample; keys [B*S] per slot (all-ones for padding) and inv_cnt [B*F]
+struct ItcBagGather : ItcGather {
+  const int64_t* off;        // [F+1] exclusive cumsum of the per-field bag sizes, off[F] = S
+  float* inv_cnt;            // [B*F] 1 / (valid ids of the bag), 0 for an empty bag
+  int S;
+};
+// rows of one bag requested together (independent loads in flight per thread; the register budget of the 384-thread
+// CTA bounds it: the chunk's rows live in registers until they are summed)
+constexpr int ITC_BAG_CHUNK = 4;
+
 __device__ __forceinline__ void ld_row64(const float* p, uint32_t (&v)[16]) {
   // one 64-byte embedding row as two 32-byte requests (LDG.256): a row-per-thread loader must not split a row into
   // four 16-byte requests (the NVLink path is request-rate bound); L2::64B: a miss fetches the 64-byte row, not 128 B
@@ -56,9 +68,9 @@ __device__ __forceinline__ void ld_row64(const float* p, uint32_t (&v)[16]) {
                : "l"(p + 8) : "memory");
 }
 
-template <int NCHF, typename T, bool GATHER>
+template <int NCHF, typename T, bool GATHER, typename GA = ItcGather>
 __global__ void __launch_bounds__(384, 1)
-interacting_tc_fwd_kernel(const ItcGather ga, T* __restrict__ x, int64_t x_ld, int64_t x_bs, const float* __restrict__ W,
+interacting_tc_fwd_kernel(const GA ga, T* __restrict__ x, int64_t x_ld, int64_t x_bs, const float* __restrict__ W,
                           const float* __restrict__ bias, const float* __restrict__ gamma,
                           const float* __restrict__ beta, float eps, T* __restrict__ y, int64_t y_ld,
                           int64_t y_bs, float* __restrict__ saved, int B, int F, int L, int use_res) {
@@ -66,6 +78,7 @@ interacting_tc_fwd_kernel(const ItcGather ga, T* __restrict__ x, int64_t x_ld, i
   using G = ItcGeom<NCHF>;
   constexpr int FP = G::FP, SPT = G::SPT, NCHK = G::NCHK, KP = G::KP;
   constexpr int FMIN = NCHF == 2 ? 0 : FP - 8;           // F > FMIN is guaranteed (NCHF = 2 also serves F <= 8)
+  constexpr bool BAG = !std::is_same<GA, ItcGather>::value;   // GATHER with a bag of slots per (sample, field)
   // ---- shared memory: only B operands live here (every A operand is TMEM-resident)
   constexpr int WG_BYTES = H * G::KX_BYTES + H * G::VX_BYTES;
   constexpr int OFF_KX = 0;                              // H x [FP keys][8 SPT] tf32, K-major: row j = [k_0j | k_1j | ..]
@@ -182,7 +195,50 @@ interacting_tc_fwd_kernel(const ItcGather ga, T* __restrict__ x, int64_t x_ld, i
       T* xo = x + smp_ * x_bs + (int64_t)f_loc * x_ld;
 #pragma unroll
       for (int c = 0; c < D / 2; c += 2) *reinterpret_cast<uint2*>(xo + 2 * c) = make_uint2(pk[c], pk[c + 1]);
-      if (ga.keys) ga.keys[smp_ * F + f_loc] = ((uint64_t)(uint32_t)lrow << 32) | (uint64_t)(uint32_t)(smp_ * F + f_loc);
+      if (!BAG && ga.keys) ga.keys[smp_ * F + f_loc] = ((uint64_t)(uint32_t)lrow << 32) | (uint64_t)(uint32_t)(smp_ * F + f_loc);
+    }
+  };
+  // BAG: the mean of the valid rows of (tile, row)'s bag as fp32 bits, with embed_bag_fwd_kernel's arithmetic (fp32 sum
+  // in slot order, times 1 / count; an empty bag is zeros); the slots' sort keys and the bag's 1 / count are written
+  // here.  Slots are read ITC_BAG_CHUNK at a time: the chunk's ids, then its rows, all requests independent.
+  int64_t b_lo = 0, b_n = 0;
+  if constexpr (BAG) {
+    if (in_tile && f_loc < F) { b_lo = ga.off[f_loc]; b_n = ga.off[f_loc + 1] - b_lo; }
+  }
+  auto load_bag = [&](int tile_, uint32_t (&raw)[D]) {
+    if constexpr (BAG) {
+      const int64_t smp_ = (int64_t)tile_ * SPT + s_loc;
+      const bool act_ = tile_ < ntiles && in_tile && f_loc < F && smp_ < B;
+      float acc[D];
+#pragma unroll
+      for (int c = 0; c < D; ++c) acc[c] = 0.f;
+      int cnt = 0;
+      const int64_t p0 = smp_ * ga.S + b_lo;
+      for (int64_t k0 = 0; act_ && k0 < b_n; k0 += ITC_BAG_CHUNK) {
+        int64_t id[ITC_BAG_CHUNK];
+#pragma unroll
+        for (int j = 0; j < ITC_BAG_CHUNK; ++j) id[j] = k0 + j < b_n ? ga.ids[p0 + k0 + j] : -1;
+        uint32_t rv[ITC_BAG_CHUNK][D];
+        int32_t lr[ITC_BAG_CHUNK];
+#pragma unroll
+        for (int j = 0; j < ITC_BAG_CHUNK; ++j) load_row(id[j], rv[j], lr[j]);
+#pragma unroll
+        for (int j = 0; j < ITC_BAG_CHUNK; ++j) {
+          if (k0 + j < b_n) {
+            const uint64_t p = (uint64_t)(p0 + k0 + j);
+            if (ga.keys) ga.keys[p] = id[j] >= 0 ? ((uint64_t)(uint32_t)lr[j] << 32) | (uint64_t)(uint32_t)p : ~0ULL;
+            if (id[j] >= 0) {
+#pragma unroll
+              for (int c = 0; c < D; ++c) acc[c] += __uint_as_float(rv[j][c]);
+              ++cnt;
+            }
+          }
+        }
+      }
+      const float inv = cnt > 0 ? 1.f / (float)cnt : 0.f;
+#pragma unroll
+      for (int c = 0; c < D; ++c) raw[c] = __float_as_uint(acc[c] * inv);
+      if (act_) ga.inv_cnt[smp_ * F + f_loc] = inv;
     }
   };
   auto wg_sync = [&]() { named_bar_sync(1 + wg, 128); };
@@ -192,7 +248,12 @@ interacting_tc_fwd_kernel(const ItcGather ga, T* __restrict__ x, int64_t x_ld, i
   uint32_t rawn[D];              // GATHER: the next tile's table row in flight
   int32_t lrown = -1;
   int64_t idn = -1;              // GATHER: the id of the tile after the next
-  if (GATHER) {
+  if (BAG) {
+    if (tile < ntiles) {
+      load_bag(tile, rawn);
+      consume_row(tile, rawn, lrown, xr);
+    }
+  } else if (GATHER) {
     if (tile < ntiles) {
       load_row(load_id(tile), rawn, lrown);
       consume_row(tile, rawn, lrown, xr);
@@ -227,7 +288,10 @@ interacting_tc_fwd_kernel(const ItcGather ga, T* __restrict__ x, int64_t x_ld, i
         tc_mma_tf32_ts(tmem + C_Z, tmem + C_ONE, make_nosw_desc(sbase + OFF_BT, 128, 256), ID_Z, 1u);
         tc_commit(bar);
       }
-      if (GATHER) {
+      if (BAG) {
+        // the next tile's bag means, summed while this tile's projection runs on the tensor cores
+        if (it == 0 && tile + tstride < ntiles) load_bag(tile + tstride, rawn);
+      } else if (GATHER) {
         // the id fetched a tile ago turns into the next tile's row loads; the id of the tile after it is requested
         // (requested at the tile's FIRST iteration: a whole tile, ~10 us, of cover for the NVLink round trip)
         if (it == 0 && tile + tstride < ntiles) { load_row(idn, rawn, lrown); idn = load_id(tile + 2 * tstride); }
@@ -433,7 +497,17 @@ static int launch_itc_fwd(const IFwdArgs& a) {
   // 131 — leaves 17 SMs to the step's other branches.  Measured on one and two GPUs: the key sort / NCCL kernels that
   // moved there ran 3x slower on so few SMs and slowed the step; every SM takes part.)
   ItcGather ga{};
-  if (a.gather) {
+  if (a.gather && a.gather->bag_off) {
+    ItcBagGather gb{};
+    gb.tab[0] = a.gather->tables[0];
+    gb.tld = a.gather->table_ld; gb.world = 1; gb.ids = a.gather->ids; gb.lbase = a.gather->local_base;
+    gb.rows = a.gather->rows; gb.keys = a.gather->sort_keys;
+    gb.off = a.gather->bag_off; gb.inv_cnt = a.gather->inv_cnt; gb.S = a.gather->bag_slots;
+    auto kern = interacting_tc_fwd_kernel<NCHF, T, true, ItcBagGather>;
+    RS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    kern<<<grid, 384, smem, a.st>>>(gb, (T*)a.x, a.x_ld, a.x_bs, a.W, a.b, a.gm, a.bt, a.eps, (T*)a.y, a.y_ld, a.y_bs,
+                                    (float*)a.saved, a.B, a.F, a.L, a.use_res);
+  } else if (a.gather) {
     for (int r = 0; r < RS_MAX_PEERS; ++r) ga.tab[r] = r < a.gather->world ? a.gather->tables[r] : nullptr;
     ga.tld = a.gather->table_ld; ga.world = a.gather->world; ga.ids = a.gather->ids; ga.lbase = a.gather->local_base;
     ga.rows = a.gather->rows; ga.keys = a.gather->sort_keys;

@@ -203,6 +203,9 @@ class ShardedAutoIntTrainer(AutoIntTrainer):
     def __init__(self, cfg: AutoIntConfig, device, group=None, global_tables: torch.Tensor | None = None,
                  dense_init: dict | None = None, capacity_factor: float | None = None, capacity: int | None = None):
         check_sharded_id_map(cfg.id_map)          # before any collective
+        if any(k > 1 for k in cfg.bags()):
+            # the fused gradient push sends one row per (sample, field): bags would need one per slot
+            raise ValueError("row-sharded bag fields are not built")
         self.ex = Exchange(group)
         self.world, self.rank = self.ex.world, self.ex.rank
         super().__init__(cfg, device, tables=global_tables, dense_init=dense_init)
