@@ -602,6 +602,14 @@ int rs_tower_supported(int K0, int N0, int N1, int Ki);
 int rs_tower_step(const void* X, const void* W0T, const void* W1T, const void* W0, const void* W1, const float* b0,
                   const float* b1, const float* w, const float* ob, const float* y, float a, void* Z, void* p_out,
                   void* dZ, void* H0, void* dH0, void* dX, int B, int K0, int N0, int N1, int Ki, void* stream);
+/* The forward half of rs_tower_step, for evaluation: H0 and H1 stay on chip, only p_out = sigmoid(Z w + ob) is written
+ * (rows >= B are masked), bit-identical to the p_out rs_tower_step writes for the same X, Z[:, N1:] and weights (the
+ * same kernel code: the bf16 rounding of H0 and H1, the order of the H1 w dot, the tensor-core dot of the interacting
+ * half, expf).  Z[:, :N1] is neither read nor written; no label, gradient or loss is computed.  W0 and W1 are not read
+ * (the backward's operands, in the argument order of rs_tower_step).  Same widths as rs_tower_supported. */
+int rs_tower_fwd(const void* X, const void* W0T, const void* W1T, const void* W0, const void* W1, const float* b0,
+                 const float* b1, const float* w, const float* ob, const void* Z, void* p_out, int B, int K0, int N0,
+                 int N1, int Ki, void* stream);
 
 /* dst[n, m] = src[m, n] (2-D transpose with leading dims; bf16 or fp32).  Used to
  * present activations K-major to the tensor-core weight-gradient GEMMs. */

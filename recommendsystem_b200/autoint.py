@@ -670,9 +670,26 @@ class AutoIntTrainer:
         double buffer while step n computes; step n's loss is copied device->host asynchronously into
         pinned memory and handed out one step later, when it has long arrived.  Every step still moves
         its own inputs H2D and its own loss D2H — they just do not serialise with the compute."""
+        def check(ids, labels):
+            self._check_ids(ids)
+            return self.cfg.batch
+
+        for _, loss in self._pipelined("fit", batches, check, lambda n: self.run(), self.loss):
+            yield loss
+
+    def _pipelined(self, key, batches, check, launch, out):
+        """The double-buffered input pipeline of fit_host and evaluate: for every (ids [n, S], labels [n, 1]) batch,
+        n = check(ids, labels) (raises for a bad batch), the batch is copied into rows [0, n) of the static id / label
+        buffers (ids of rows [n, B) = -1), launch(n) runs on the current stream, and (n, float(out)) is yielded, one
+        batch late.  Device-resident batches are read on the copy stream after the current stream's earlier work.
+        Every caller `key` has its own buffers, events and copy stream: an evaluate() run between two batches of a
+        fit_host loop leaves the training batch already uploaded, and the loss not yet handed out, where they are."""
         dev = self.dev
-        if not hasattr(self, "_pipe"):
-            self._pipe = {
+        B = self.cfg.batch
+        if not hasattr(self, "_pipes"):
+            self._pipes = {}
+        if key not in self._pipes:
+            self._pipes[key] = {
                 "copy": torch.cuda.Stream(device=dev),
                 "ids": [torch.empty_like(self.ids) for _ in range(2)],
                 "lab": [torch.empty_like(self.labels) for _ in range(2)],
@@ -681,17 +698,28 @@ class AutoIntTrainer:
                 "loss": [torch.empty(1, dtype=torch.float32).pin_memory() for _ in range(2)],
                 "done": [torch.cuda.Event() for _ in range(2)],        # loss of slot k is on the host
             }
-        p = self._pipe
+        p = self._pipes[key]
         main = torch.cuda.current_stream(dev)
         it = iter(batches)
+        rows = [0, 0]
 
         def upload(k, batch):
             ids_h, lab_h = batch
-            self._check_ids(ids_h)
+            n = rows[k] = check(ids_h, lab_h)
             with torch.cuda.stream(p["copy"]):
                 p["copy"].wait_event(p["free"][k])
-                p["ids"][k].copy_(ids_h, non_blocking=True)
-                p["lab"][k].copy_(lab_h, non_blocking=True)
+                if ids_h.is_cuda or lab_h.is_cuda:
+                    p["copy"].wait_stream(main)
+                for t in (ids_h, lab_h):
+                    if t.is_cuda:
+                        t.record_stream(p["copy"])
+                if n == B:
+                    p["ids"][k].copy_(ids_h, non_blocking=True)
+                    p["lab"][k].copy_(lab_h, non_blocking=True)
+                else:
+                    p["ids"][k][:n].copy_(ids_h, non_blocking=True)
+                    p["ids"][k][n:].fill_(-1)
+                    p["lab"][k][:n].copy_(lab_h, non_blocking=True)
                 p["ready"][k].record(p["copy"])
 
         for k in range(2):
@@ -709,18 +737,136 @@ class AutoIntTrainer:
             self.ids.copy_(p["ids"][k], non_blocking=True)          # device-to-device, a few microseconds
             self.labels.copy_(p["lab"][k], non_blocking=True)
             p["free"][k].record(main)
+            rows_k = rows[k]
             if nxt is not None:
                 upload(k ^ 1, nxt)                                   # overlaps the step below
-            self.run()
-            p["loss"][k].copy_(self.loss.reshape(1), non_blocking=True)
+            launch(rows_k)
+            p["loss"][k].copy_(out.reshape(1), non_blocking=True)
             p["done"][k].record(main)
             if pending is not None:
-                p["done"][pending].synchronize()
-                yield float(p["loss"][pending][0])
-            pending = k
+                p["done"][pending[0]].synchronize()
+                yield pending[1], float(p["loss"][pending[0]][0])
+            pending = (k, rows_k)
             n += 1
-        p["done"][pending].synchronize()
-        yield float(p["loss"][pending][0])
+        p["done"][pending[0]].synchronize()
+        yield pending[1], float(p["loss"][pending[0]][0])
+
+    # ---- evaluation: the train step's forward and the Keras metrics of its p ------------------------------------
+    @torch.no_grad()
+    def evaluate(self, batches, num_thresholds: int = 200, threshold: float = 0.5) -> dict:
+        """Keras `model.evaluate` with `compile(metrics=[AUC(), BinaryAccuracy(), CTR(), COPC()])`: the metrics of
+        `api.metrics.BinaryMetrics` (Keras AUC thresholds, accuracy at `threshold`) and the mean loss over every sample
+        of `batches`, an iterable of (ids [n, S] int64, labels [n, 1] f32), 1 <= n <= batch, on the host (pinned, for
+        overlap) or on the device.  Returns python floats for BinaryMetrics.NAMES and "loss"; the state is fresh per
+        call.  Every batch runs the eval step: the train step's forward (its p is bit for bit the p_raw a train step
+        from the same state computes) on the static buffers, padded with id -1 rows to the batch size, and the metrics
+        and the summed loss of its first n rows.  Nothing the train step updates changes, hash mode inserts and counts
+        no id (an unseen id reads as padding), and a captured train graph stays valid.  Full batches replay a CUDA
+        graph of the eval step captured on first use; a partial one runs the same launches eagerly."""
+        ev = self._eval_state(num_thresholds, threshold)
+        ev["metrics"].reset_states()
+        count, loss_sum = 0, 0.0
+        for n, loss in self._pipelined("eval", batches, self._check_eval_batch, self._eval_run, ev["loss"]):
+            count += n
+            loss_sum += n * loss                # the batch's fp32 mean times its rows
+        totals = torch.tensor([loss_sum, count], dtype=torch.float64, device=self.dev)
+        self._eval_reduce(ev, totals)
+        out = ev["metrics"].result()
+        loss_sum, count = totals.tolist()
+        out["loss"] = loss_sum / count if count > 0 else 0.0
+        return out
+
+    def _check_eval_batch(self, ids, labels) -> int:
+        """n of an (ids [n, S], labels [n, 1]) eval batch; ValueError unless 1 <= n <= batch and the labels are [n, 1]."""
+        B, S = self.ids.shape
+        if ids.dim() != 2 or ids.shape[1] != S or not 1 <= ids.shape[0] <= B:
+            raise ValueError(f"ids of shape {tuple(ids.shape)}: evaluate takes [n, sum(bag_size)] = [n, {S}] with "
+                             f"1 <= n <= batch = {B}")
+        n = int(ids.shape[0])
+        if tuple(labels.shape) != (n, 1):
+            raise ValueError(f"labels of shape {tuple(labels.shape)} for {n} rows of ids: evaluate takes [n, 1]")
+        return n
+
+    def _eval_state(self, num_thresholds, threshold):
+        """The eval step's own buffers: the metric state (BinaryMetrics), the batch loss, scratch for what the forward
+        kernels also write (bags: 1 / count; the separate head pass: dZ and its partial sums) and the graph.  Kept
+        while num_thresholds and threshold stay the same."""
+        key = (int(num_thresholds), float(threshold))
+        ev = getattr(self, "_ev", None)
+        if ev is not None and ev["key"] == key:
+            return ev
+        from .api.metrics import BinaryMetrics
+        B, F = self.cfg.batch, self.cfg.num_fields
+        ev = {"key": key, "metrics": BinaryMetrics(num_thresholds, threshold, self.dev),
+              "loss": torch.zeros(1, device=self.dev), "graph": None}
+        if self.fused and self.bag:
+            ev["inv_cnt"] = torch.empty(B * F, device=self.dev)
+        if not self.fuse_tower:
+            ev["dZ"] = torch.empty_like(self.dZ)
+            ev["head_ws"] = ops.logit_head_workspace(B, self.zw, self.dev)
+        self._ev = ev
+        return ev
+
+    def _eval_run(self, n):
+        """One eval step over the static buffers; a full batch replays the eval graph, captured after its first eager
+        launch (no state to restore: the eval step changes none)."""
+        ev = self._ev
+        full = n == self.cfg.batch
+        if full and ev["graph"] is not None:
+            ev["graph"].replay()
+            return
+        self._launch_eval(n)
+        if full:
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                self._launch_eval(n)
+            ev["graph"] = g
+
+    def _launch_eval(self, n):
+        """The eval step on torch's current stream: the train step's forward (same kernels, same arithmetic; no saved
+        activations, sort keys or gradients) into p_raw, then the metrics and the summed loss of rows [0, n)."""
+        c = self.cfg
+        F, d, U, B = c.num_fields, c.embed_dim, c.unit_num, c.batch
+        st, T, P = ops._stream(), ops._DT[self.act_dtype], self.P
+        ev = self._ev
+        if self.fused:
+            self.store.lookup(self.ids, self.slot_fields, insert=False, out=self.ids_rows)
+            tabs, world, lbase_t, _ = self._lookup_args()
+            lk_ids, _, lk_rows = self.lookup
+            if self.bag:
+                cabi.call("rs_interacting_fwd_gather_bag", self.table.data_ptr(), self.table_ld, lk_ids.data_ptr(),
+                          self.slot_off.data_ptr(), lbase_t.data_ptr(), lk_rows.data_ptr(), self.X.data_ptr(), d, 0,
+                          None, ev["inv_cnt"].data_ptr(), T, P["Wqkvr"].data_ptr(), P["bqkvr"].data_ptr(),
+                          P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps, self.Z[:, self.n_deep:].data_ptr(), U,
+                          self.zw, None, B, F, self.S, d, U, c.head_num, c.layer_num, int(c.use_res), st)
+            else:
+                cabi.call("rs_interacting_fwd_gather", tabs, self.table_ld, world, lk_ids.data_ptr(), lbase_t.data_ptr(),
+                          lk_rows.data_ptr(), self.X.data_ptr(), d, 0, None, T, P["Wqkvr"].data_ptr(),
+                          P["bqkvr"].data_ptr(), P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps,
+                          self.Z[:, self.n_deep:].data_ptr(), U, self.zw, None, B, F, d, U, c.head_num, c.layer_num,
+                          int(c.use_res), st)
+        else:
+            self._predict_lookup(st, T)
+            cabi.call("rs_interacting_fwd", self.X.data_ptr(), d, 0, T, P["Wqkvr"].data_ptr(), P["bqkvr"].data_ptr(),
+                      P["gamma"].data_ptr(), P["beta"].data_ptr(), c.ln_eps, self.Z[:, self.n_deep:].data_ptr(), U,
+                      self.zw, None, B, F, d, U, c.head_num, c.layer_num, int(c.use_res), int(self.bf16), st)
+        Xf = self.X.view(B, F * d)
+        if self.fuse_tower:
+            ops.tower_fwd(Xf, self.WT16["mlp_W0"], self.WT16["mlp_W1"], self.P16["mlp_W0"], self.P16["mlp_W1"],
+                          P["mlp_b0"], P["mlp_b1"], P["out_W"], P["out_b"], self.Z, self.p_raw)
+        else:
+            acts = [Xf] + self.H + [self.Z[:, :self.n_deep]]
+            for i in range(len(c.mlp_hidden)):
+                self._dense_fwd(acts[i], f"mlp_W{i}", f"mlp_b{i}", acts[i + 1])
+            # the train step's head pass; its dZ and gradient partials land in the eval step's scratch
+            ops.logit_head(self.Z, P["out_W"], P["out_b"], self.labels, ev["dZ"], None, None, p_out=self.p_raw,
+                           loss=ev["loss"], relu_cols=self.n_deep, ws=ev["head_ws"], defer_reduce=True)
+        m = ev["metrics"]
+        ops.binary_metrics_update(m.state, self.p_raw[:n], self.labels[:n], m.thresholds, m.threshold)
+        ops.bce_sigmoid_fwd_bwd(self.p_raw[:n], self.labels[:n], want_grad=False, loss=ev["loss"])
+
+    def _eval_reduce(self, ev, totals):
+        """One GPU: nothing to merge.  (Sharded: the sum of every rank's metric state and loss totals.)"""
 
     @torch.no_grad()
     def predict(self, ids: torch.Tensor) -> torch.Tensor:

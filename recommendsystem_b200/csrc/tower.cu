@@ -21,6 +21,7 @@
 //                      [384, 512) H0 (bf16), then dX chunk buffer 2
 // The Z·w dot of the interacting half runs on the tensor core: B = [w_hi; w_lo] (w = w_hi + w_lo to ~2^-17, both
 // bf16), so it keeps the fp32 weight's precision.
+// rs_tower_fwd (evaluation) is the same kernel body stopped after p_out: no H0 / Z stores, nothing of 3.-5. but p.
 #include "tc_common.cuh"
 
 namespace rs {
@@ -68,10 +69,13 @@ __device__ __forceinline__ void stg_put(uint8_t* slab, int row, int c, uint32_t 
 __device__ __forceinline__ float lo_bf(uint32_t u) { return __uint_as_float(u << 16); }
 __device__ __forceinline__ float hi_bf(uint32_t u) { return __uint_as_float(u & 0xFFFF0000u); }
 
-__global__ void __launch_bounds__(TW_THREADS, 1)
-tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict__ b0, const float* __restrict__ b1,
-                  const float* __restrict__ w, const float* __restrict__ ob, const float* __restrict__ y, float a,
-                  __nv_bfloat16* __restrict__ p_out, int B, int K0, int Ki) {
+// FWD = the forward half (steps 1-3 up to p_out; rs_tower_fwd): the same code, with the loads, products and stores
+// that only the backward needs left out, so p_out is bit-identical to the full step's
+template <bool FWD>
+__device__ __forceinline__ void tower_body(const TowerMaps& tm, const float* __restrict__ b0, const float* __restrict__ b1,
+                                           const float* __restrict__ w, const float* __restrict__ ob,
+                                           const float* __restrict__ y, float a, __nv_bfloat16* __restrict__ p_out, int B,
+                                           int K0, int Ki) {
   extern __shared__ uint8_t tw_smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tw_smem_raw) + 1023) & ~(uintptr_t)1023);
   const int kpad = tower_kpad(Ki);
@@ -129,15 +133,17 @@ tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict_
         const int s = slot(TW_SLAB);
         tma_load_2d(ring + s * TW_STAGE, &tm.w1t, &full[s], kb * 64, 0);
       }
-      for (int kb = 0; kb < TW_N1 / 64; ++kb) {
-        const int s = slot(2 * TW_SLAB);
-        tma_load_2d(ring + s * TW_STAGE, &tm.w1, &full[s], kb * 64, 0);
-      }
-      for (int ch = 0; ch < nch; ++ch)
-        for (int kb = 0; kb < TW_N0 / 64; ++kb) {
-          const int s = slot(TW_SLAB);
-          tma_load_2d(ring + s * TW_STAGE, &tm.w0, &full[s], kb * 64, ch * 128);
+      if constexpr (!FWD) {
+        for (int kb = 0; kb < TW_N1 / 64; ++kb) {
+          const int s = slot(2 * TW_SLAB);
+          tma_load_2d(ring + s * TW_STAGE, &tm.w1, &full[s], kb * 64, 0);
         }
+        for (int ch = 0; ch < nch; ++ch)
+          for (int kb = 0; kb < TW_N0 / 64; ++kb) {
+            const int s = slot(TW_SLAB);
+            tma_load_2d(ring + s * TW_STAGE, &tm.w0, &full[s], kb * 64, ch * 128);
+          }
+      }
     }
   } else if (warp == 1) {
     if (lane == 0) {
@@ -187,37 +193,39 @@ tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict_
         tc_commit(&empty[s]);
       }
       tc_commit(&bar[B_ACC1]);
-      // 4. dH1 W1^T -> [0, 256)
-      mbar_wait(&bar[B_DH1], 0);
-      tc_fence_after();
-      for (int kb = 0; kb < TW_N1 / 64; ++kb) {
-        const int s = take();
-        const uint64_t bd = make_sw128_kmajor_desc(smem_u32(ring + s * TW_STAGE));
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-          tc_mma_bf16_ts(tmem + C_ACC0, tmem + C_DH1 + kb * 32 + k * 8, bd + 2 * k, ID256, (kb | k) ? 1u : 0u);
-        tc_commit(&empty[s]);
-      }
-      tc_commit(&bar[B_ACC4]);
-      // 5. dH0 W0^T, 128 output columns per chunk, three TMEM buffers
-      mbar_wait(&bar[B_DH0], 0);
-      tc_fence_after();
-      for (int ch = 0; ch < nch; ++ch) {
-        const int buf = ch % 3, u = ch / 3;
-        const uint32_t col = buf == 0 ? 0u : buf == 1 ? 128u : 384u;
-        if (u > 0) {
-          mbar_wait(&bar[B_XE + buf], (uint32_t)(u - 1) & 1u);
-          tc_fence_after();
-        }
-        for (int kb = 0; kb < TW_N0 / 64; ++kb) {
+      if constexpr (!FWD) {
+        // 4. dH1 W1^T -> [0, 256)
+        mbar_wait(&bar[B_DH1], 0);
+        tc_fence_after();
+        for (int kb = 0; kb < TW_N1 / 64; ++kb) {
           const int s = take();
           const uint64_t bd = make_sw128_kmajor_desc(smem_u32(ring + s * TW_STAGE));
 #pragma unroll
           for (int k = 0; k < 4; ++k)
-            tc_mma_bf16_ts(tmem + col, tmem + C_DH0 + kb * 32 + k * 8, bd + 2 * k, ID128, (kb | k) ? 1u : 0u);
+            tc_mma_bf16_ts(tmem + C_ACC0, tmem + C_DH1 + kb * 32 + k * 8, bd + 2 * k, ID256, (kb | k) ? 1u : 0u);
           tc_commit(&empty[s]);
         }
-        tc_commit(&bar[B_XF + buf]);
+        tc_commit(&bar[B_ACC4]);
+        // 5. dH0 W0^T, 128 output columns per chunk, three TMEM buffers
+        mbar_wait(&bar[B_DH0], 0);
+        tc_fence_after();
+        for (int ch = 0; ch < nch; ++ch) {
+          const int buf = ch % 3, u = ch / 3;
+          const uint32_t col = buf == 0 ? 0u : buf == 1 ? 128u : 384u;
+          if (u > 0) {
+            mbar_wait(&bar[B_XE + buf], (uint32_t)(u - 1) & 1u);
+            tc_fence_after();
+          }
+          for (int kb = 0; kb < TW_N0 / 64; ++kb) {
+            const int s = take();
+            const uint64_t bd = make_sw128_kmajor_desc(smem_u32(ring + s * TW_STAGE));
+#pragma unroll
+            for (int k = 0; k < 4; ++k)
+              tc_mma_bf16_ts(tmem + col, tmem + C_DH0 + kb * 32 + k * 8, bd + 2 * k, ID128, (kb | k) ? 1u : 0u);
+            tc_commit(&empty[s]);
+          }
+          tc_commit(&bar[B_XF + buf]);
+        }
       }
     }
   } else {
@@ -267,7 +275,7 @@ tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict_
     mbar_wait(&bar[B_ACC0], 0);
     tc_fence_after();
     for (int p = 0; p < 2; ++p) {
-      uint8_t* sb = pass_begin();
+      uint8_t* sb = FWD ? nullptr : pass_begin();
 #pragma unroll
       for (int c0 = 0; c0 < 128; c0 += 32) {
         const int c = p * 128 + c0;
@@ -278,15 +286,19 @@ tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict_
           h[j] = pack_bf16x2(fmaxf(__uint_as_float(r[2 * j]) + __ldg(b0 + c + 2 * j), 0.f),
                              fmaxf(__uint_as_float(r[2 * j + 1]) + __ldg(b0 + c + 2 * j + 1), 0.f));
         tc_st_32x16(tl + C_H0 + c / 2, h);
+        if constexpr (!FWD) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
-          stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q, h[4 * q], h[4 * q + 1], h[4 * q + 2], h[4 * q + 3]);
+          for (int q = 0; q < 4; ++q)
+            stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q, h[4 * q], h[4 * q + 1], h[4 * q + 2], h[4 * q + 3]);
+        }
       }
-      pass_end();
-      if (et == 0) {
-        tma_store_2d(&tm.h0, sb, p * 128, m0);
-        tma_store_2d(&tm.h0, sb + TW_SLAB, p * 128 + 64, m0);
-        bulk_commit();
+      if constexpr (!FWD) {
+        pass_end();
+        if (et == 0) {
+          tma_store_2d(&tm.h0, sb, p * 128, m0);
+          tma_store_2d(&tm.h0, sb + TW_SLAB, p * 128 + 64, m0);
+          bulk_commit();
+        }
       }
     }
     tc_wait_st();
@@ -310,7 +322,7 @@ tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict_
     float dot = 0.f;
     uint32_t mask[TW_N1 / 32];
     {
-      uint8_t* sb = pass_begin();
+      uint8_t* sb = FWD ? nullptr : pass_begin();
 #pragma unroll
       for (int c0 = 0; c0 < TW_N1; c0 += 32) {
         uint32_t r[32], h[16], m = 0;
@@ -326,132 +338,138 @@ tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict_
           m |= (q1 > 0.f ? 1u : 0u) << (2 * j + 1);
         }
         mask[c0 / 32] = m;
+        if constexpr (!FWD) {
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
-          stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q, h[4 * q], h[4 * q + 1], h[4 * q + 2], h[4 * q + 3]);
+          for (int q = 0; q < 4; ++q)
+            stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q, h[4 * q], h[4 * q + 1], h[4 * q + 2], h[4 * q + 3]);
+        }
       }
-      pass_end();
-      if (et == 0) {
-        tma_store_2d(&tm.z, sb, 0, m0);
-        tma_store_2d(&tm.z, sb + TW_SLAB, 64, m0);
-        bulk_commit();
+      if constexpr (!FWD) {
+        pass_end();
+        if (et == 0) {
+          tma_store_2d(&tm.z, sb, 0, m0);
+          tma_store_2d(&tm.z, sb + TW_SLAB, 64, m0);
+          bulk_commit();
+        }
       }
     }
     const bool live = grow < B;
     const float pr = 1.f / (1.f + expf(-(dot + zi_dot + __ldg(ob))));
     const float prs = __bfloat162float(__float2bfloat16_rn(pr));   // the stored activation
     const float pc = fminf(fmaxf(prs, 1e-6f), 1.0f);
-    const float yy = live ? y[grow] : 0.f;
+    const float yy = !FWD && live ? y[grow] : 0.f;           // FWD: y is NULL (dz is not computed)
     const float dp = (-yy / (pc + 1e-6f) + (a - yy) / (1.0f - pc + 1e-6f)) * (1.f / (float)B);
     const float dz = (live && prs >= 1e-6f && prs <= 1.0f) ? dp * prs * (1.f - prs) : 0.f;
     if (live) p_out[grow] = __float2bfloat16_rn(pr);
-    // dH1 = dz w[:N1] relu'(H1) -> dZ[:, :N1] + TMEM
-    {
-      uint8_t* sb = pass_begin();
+    if constexpr (!FWD) {
+      // dH1 = dz w[:N1] relu'(H1) -> dZ[:, :N1] + TMEM
+      {
+        uint8_t* sb = pass_begin();
 #pragma unroll
-      for (int c0 = 0; c0 < TW_N1; c0 += 32) {
-        uint32_t g[16];
+        for (int c0 = 0; c0 < TW_N1; c0 += 32) {
+          uint32_t g[16];
 #pragma unroll
-        for (int j = 0; j < 16; ++j)
-          g[j] = pack_bf16x2((mask[c0 / 32] >> (2 * j)) & 1u ? dz * w_s[c0 + 2 * j] : 0.f,
-                             (mask[c0 / 32] >> (2 * j + 1)) & 1u ? dz * w_s[c0 + 2 * j + 1] : 0.f);
-        tc_st_32x16(tl + C_DH1 + c0 / 2, g);
+          for (int j = 0; j < 16; ++j)
+            g[j] = pack_bf16x2((mask[c0 / 32] >> (2 * j)) & 1u ? dz * w_s[c0 + 2 * j] : 0.f,
+                               (mask[c0 / 32] >> (2 * j + 1)) & 1u ? dz * w_s[c0 + 2 * j + 1] : 0.f);
+          tc_st_32x16(tl + C_DH1 + c0 / 2, g);
 #pragma unroll
-        for (int q = 0; q < 4; ++q)
-          stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q, g[4 * q], g[4 * q + 1], g[4 * q + 2], g[4 * q + 3]);
+          for (int q = 0; q < 4; ++q)
+            stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q, g[4 * q], g[4 * q + 1], g[4 * q + 2], g[4 * q + 3]);
+        }
+        pass_end();
+        if (et == 0) {
+          tma_store_2d(&tm.dz, sb, 0, m0);
+          tma_store_2d(&tm.dz, sb + TW_SLAB, 64, m0);
+          bulk_commit();
+        }
       }
-      pass_end();
-      if (et == 0) {
-        tma_store_2d(&tm.dz, sb, 0, m0);
-        tma_store_2d(&tm.dz, sb + TW_SLAB, 64, m0);
-        bulk_commit();
-      }
-    }
-    tc_wait_st();
-    tc_fence_before();
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&bar[B_DH1]);
-    // dZ[:, N1:] = dz w[N1:] (what the InteractingLayer backward reads), while the MMAs of 4. run
-    for (int s0 = 0; s0 < nki; s0 += 2) {
-      uint8_t* sb = pass_begin();
-      const int ns = min(2, nki - s0);
-      for (int sl = 0; sl < ns; ++sl) {
-        const float* wc = w_s + TW_N1 + (s0 + sl) * 64;
-#pragma unroll
-        for (int q = 0; q < 8; ++q)
-          stg_put(sb + sl * TW_SLAB, row, q, pack_bf16x2(dz * wc[q * 8 + 0], dz * wc[q * 8 + 1]),
-                  pack_bf16x2(dz * wc[q * 8 + 2], dz * wc[q * 8 + 3]), pack_bf16x2(dz * wc[q * 8 + 4], dz * wc[q * 8 + 5]),
-                  pack_bf16x2(dz * wc[q * 8 + 6], dz * wc[q * 8 + 7]));
-      }
-      pass_end();
-      if (et == 0) {
-        for (int sl = 0; sl < ns; ++sl) tma_store_2d(&tm.dz, sb + sl * TW_SLAB, TW_N1 + (s0 + sl) * 64, m0);
-        bulk_commit();
-      }
-    }
-
-    // ---- 4. dH0 = acc relu'(H0) -> global + TMEM (bf16)
-    mbar_wait(&bar[B_ACC4], 0);
-    tc_fence_after();
-    for (int p = 0; p < 2; ++p) {
-      uint8_t* sb = pass_begin();
-#pragma unroll
-      for (int c0 = 0; c0 < 128; c0 += 32) {
-        const int c = p * 128 + c0;
-        uint32_t r[32], hm[16], g[16];
-        tc_ld_32x16(tl + C_H0 + c / 2, hm);
-        tc_ld_32x32(tl + C_ACC0 + c, r);              // waits for both loads
-#pragma unroll
-        for (int j = 0; j < 16; ++j)
-          g[j] = pack_bf16x2(lo_bf(hm[j]) > 0.f ? __uint_as_float(r[2 * j]) : 0.f,
-                             hi_bf(hm[j]) > 0.f ? __uint_as_float(r[2 * j + 1]) : 0.f);
-        tc_st_32x16(tl + C_DH0 + c / 2, g);
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q, g[4 * q], g[4 * q + 1], g[4 * q + 2], g[4 * q + 3]);
-      }
-      pass_end();
-      if (et == 0) {
-        tma_store_2d(&tm.dh0, sb, p * 128, m0);
-        tma_store_2d(&tm.dh0, sb + TW_SLAB, p * 128 + 64, m0);
-        bulk_commit();
-      }
-    }
-    tc_wait_st();
-    tc_fence_before();
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&bar[B_DH0]);
-
-    // ---- 5. dX chunks -> global
-    for (int ch = 0; ch < nch; ++ch) {
-      const int buf = ch % 3;
-      const uint32_t col = buf == 0 ? 0u : buf == 1 ? 128u : 384u;
-      mbar_wait(&bar[B_XF + buf], (uint32_t)(ch / 3) & 1u);
-      tc_fence_after();
-      uint8_t* sb = pass_begin();
-#pragma unroll
-      for (int c0 = 0; c0 < 128; c0 += 32) {
-        uint32_t r[32];
-        tc_ld_32x32(tl + col + c0, r);
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q,
-                  pack_bf16x2(__uint_as_float(r[8 * q + 0]), __uint_as_float(r[8 * q + 1])),
-                  pack_bf16x2(__uint_as_float(r[8 * q + 2]), __uint_as_float(r[8 * q + 3])),
-                  pack_bf16x2(__uint_as_float(r[8 * q + 4]), __uint_as_float(r[8 * q + 5])),
-                  pack_bf16x2(__uint_as_float(r[8 * q + 6]), __uint_as_float(r[8 * q + 7])));
-      }
+      tc_wait_st();
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(&bar[B_XE + buf]);
-      pass_end();
-      if (et == 0) {
-        tma_store_2d(&tm.dx, sb, ch * 128, m0);
-        if (ch * 128 + 64 < K0) tma_store_2d(&tm.dx, sb + TW_SLAB, ch * 128 + 64, m0);
-        bulk_commit();
+      if (lane == 0) mbar_arrive(&bar[B_DH1]);
+      // dZ[:, N1:] = dz w[N1:] (what the InteractingLayer backward reads), while the MMAs of 4. run
+      for (int s0 = 0; s0 < nki; s0 += 2) {
+        uint8_t* sb = pass_begin();
+        const int ns = min(2, nki - s0);
+        for (int sl = 0; sl < ns; ++sl) {
+          const float* wc = w_s + TW_N1 + (s0 + sl) * 64;
+#pragma unroll
+          for (int q = 0; q < 8; ++q)
+            stg_put(sb + sl * TW_SLAB, row, q, pack_bf16x2(dz * wc[q * 8 + 0], dz * wc[q * 8 + 1]),
+                    pack_bf16x2(dz * wc[q * 8 + 2], dz * wc[q * 8 + 3]), pack_bf16x2(dz * wc[q * 8 + 4], dz * wc[q * 8 + 5]),
+                    pack_bf16x2(dz * wc[q * 8 + 6], dz * wc[q * 8 + 7]));
+        }
+        pass_end();
+        if (et == 0) {
+          for (int sl = 0; sl < ns; ++sl) tma_store_2d(&tm.dz, sb + sl * TW_SLAB, TW_N1 + (s0 + sl) * 64, m0);
+          bulk_commit();
+        }
       }
+
+      // ---- 4. dH0 = acc relu'(H0) -> global + TMEM (bf16)
+      mbar_wait(&bar[B_ACC4], 0);
+      tc_fence_after();
+      for (int p = 0; p < 2; ++p) {
+        uint8_t* sb = pass_begin();
+#pragma unroll
+        for (int c0 = 0; c0 < 128; c0 += 32) {
+          const int c = p * 128 + c0;
+          uint32_t r[32], hm[16], g[16];
+          tc_ld_32x16(tl + C_H0 + c / 2, hm);
+          tc_ld_32x32(tl + C_ACC0 + c, r);              // waits for both loads
+#pragma unroll
+          for (int j = 0; j < 16; ++j)
+            g[j] = pack_bf16x2(lo_bf(hm[j]) > 0.f ? __uint_as_float(r[2 * j]) : 0.f,
+                               hi_bf(hm[j]) > 0.f ? __uint_as_float(r[2 * j + 1]) : 0.f);
+          tc_st_32x16(tl + C_DH0 + c / 2, g);
+#pragma unroll
+          for (int q = 0; q < 4; ++q)
+            stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q, g[4 * q], g[4 * q + 1], g[4 * q + 2], g[4 * q + 3]);
+        }
+        pass_end();
+        if (et == 0) {
+          tma_store_2d(&tm.dh0, sb, p * 128, m0);
+          tma_store_2d(&tm.dh0, sb + TW_SLAB, p * 128 + 64, m0);
+          bulk_commit();
+        }
+      }
+      tc_wait_st();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&bar[B_DH0]);
+
+      // ---- 5. dX chunks -> global
+      for (int ch = 0; ch < nch; ++ch) {
+        const int buf = ch % 3;
+        const uint32_t col = buf == 0 ? 0u : buf == 1 ? 128u : 384u;
+        mbar_wait(&bar[B_XF + buf], (uint32_t)(ch / 3) & 1u);
+        tc_fence_after();
+        uint8_t* sb = pass_begin();
+#pragma unroll
+        for (int c0 = 0; c0 < 128; c0 += 32) {
+          uint32_t r[32];
+          tc_ld_32x32(tl + col + c0, r);
+#pragma unroll
+          for (int q = 0; q < 4; ++q)
+            stg_put(sb + (c0 >> 6) * TW_SLAB, row, ((c0 & 63) >> 3) + q,
+                    pack_bf16x2(__uint_as_float(r[8 * q + 0]), __uint_as_float(r[8 * q + 1])),
+                    pack_bf16x2(__uint_as_float(r[8 * q + 2]), __uint_as_float(r[8 * q + 3])),
+                    pack_bf16x2(__uint_as_float(r[8 * q + 4]), __uint_as_float(r[8 * q + 5])),
+                    pack_bf16x2(__uint_as_float(r[8 * q + 6]), __uint_as_float(r[8 * q + 7])));
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&bar[B_XE + buf]);
+        pass_end();
+        if (et == 0) {
+          tma_store_2d(&tm.dx, sb, ch * 128, m0);
+          if (ch * 128 + 64 < K0) tma_store_2d(&tm.dx, sb + TW_SLAB, ch * 128 + 64, m0);
+          bulk_commit();
+        }
+      }
+      if (et == 0) bulk_wait_all();
     }
-    if (et == 0) bulk_wait_all();
   }
   tc_fence_before();
   __syncthreads();
@@ -459,6 +477,21 @@ tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict_
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(512));
   }
+}
+
+__global__ void __launch_bounds__(TW_THREADS, 1)
+tower_step_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict__ b0, const float* __restrict__ b1,
+                  const float* __restrict__ w, const float* __restrict__ ob, const float* __restrict__ y, float a,
+                  __nv_bfloat16* __restrict__ p_out, int B, int K0, int Ki) {
+  tower_body<false>(tm, b0, b1, w, ob, y, a, p_out, B, K0, Ki);
+}
+
+// steps 1-3 up to p_out; reads tm.x, tm.w0t, tm.z and tm.w1t only
+__global__ void __launch_bounds__(TW_THREADS, 1)
+tower_fwd_kernel(const __grid_constant__ TowerMaps tm, const float* __restrict__ b0, const float* __restrict__ b1,
+                 const float* __restrict__ w, const float* __restrict__ ob, __nv_bfloat16* __restrict__ p_out, int B,
+                 int K0, int Ki) {
+  tower_body<true>(tm, b0, b1, w, ob, nullptr, 0.f, p_out, B, K0, Ki);
 }
 
 }  // namespace rs
@@ -494,6 +527,30 @@ int rs_tower_step(const void* X, const void* W0T, const void* W1T, const void* W
   tower_step_kernel<<<(unsigned)cdiv(B, TW_BM), TW_THREADS, smem, as_stream(stream)>>>(
       m, b0, b1, w, ob, y, a, (__nv_bfloat16*)p_out, B, K0, Ki);
   return check_launch("tower_step");
+}
+
+int rs_tower_fwd(const void* X, const void* W0T, const void* W1T, const void* W0, const void* W1, const float* b0,
+                 const float* b1, const float* w, const float* ob, const void* Z, void* p_out, int B, int K0, int N0,
+                 int N1, int Ki, void* stream) {
+  (void)W0;
+  (void)W1;
+  RS_REQUIRE(B > 0 && rs_tower_supported(K0, N0, N1, Ki),
+             "tower_fwd: B=%d K0=%d N0=%d N1=%d Ki=%d (N0 = %d, N1 = %d, K0 %% 16 == 0, Ki %% 16 == 0, Ki <= ~700)", B, K0,
+             N0, N1, Ki, TW_N0, TW_N1);
+  const void* ptrs[] = {X, W0T, W1T, Z};
+  for (const void* p : ptrs) RS_REQUIRE(p != nullptr && (uintptr_t)p % 16 == 0, "tower_fwd: operands must be 16-byte aligned");
+  RS_REQUIRE(b0 && b1 && w && ob && p_out, "tower_fwd: null pointer");
+  const int zw = N1 + Ki;
+  TowerMaps m;
+  int e;
+  if ((e = make_map(&m.x, X, B, K0, K0, TW_BM)) || (e = make_map(&m.w0t, W0T, N0, K0, K0, 256)) ||
+      (e = make_map(&m.w1t, W1T, N1, N0, N0, TW_BM)) || (e = make_map(&m.z, Z, B, zw, zw, TW_BM)))
+    return e;
+  const int smem = (int)tower_smem_bytes(Ki);
+  RS_CUDA(cudaFuncSetAttribute(tower_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  tower_fwd_kernel<<<(unsigned)cdiv(B, TW_BM), TW_THREADS, smem, as_stream(stream)>>>(m, b0, b1, w, ob,
+                                                                                      (__nv_bfloat16*)p_out, B, K0, Ki);
+  return check_launch("tower_fwd");
 }
 
 }  // extern "C"

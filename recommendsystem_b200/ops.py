@@ -447,6 +447,19 @@ def tower_step(X, W0T, W1T, W0, W1, b0, b1, w, ob, y, Z, p_out, dZ, H0, dH0, dX,
          _ptr(y), a, _ptr(Z), _ptr(p_out), _ptr(dZ), _ptr(H0), _ptr(dH0), _ptr(dX), B, K0, N0, N1, Ki, _stream())
 
 
+def tower_fwd(X, W0T, W1T, W0, W1, b0, b1, w, ob, Z, p_out):
+    """The forward half of tower_step (rs_tower_fwd): p_out from X [B, K0] and Z[:, N1:], bit-identical to the p_out
+    tower_step writes; nothing else is written."""
+    B, K0 = X.shape
+    N0, N1 = W0T.shape[0], W1T.shape[0]
+    Ki = Z.shape[1] - N1
+    for t in (X, W0T, W1T, W0, W1, Z):
+        _need(t.dtype == torch.bfloat16 and t.is_contiguous(), "tower_fwd: contiguous bf16 operands")
+    _need(p_out.dtype == torch.bfloat16 and p_out.numel() == B, "tower_fwd: p_out must be bf16 [B]")
+    call("rs_tower_fwd", _ptr(X), _ptr(W0T), _ptr(W1T), _ptr(W0), _ptr(W1), _ptr(b0), _ptr(b1), _ptr(w), _ptr(ob),
+         _ptr(Z), _ptr(p_out), B, K0, N0, N1, Ki, _stream())
+
+
 def colsum(x, out=None):
     _need(x.dim() == 2 and x.stride(1) == 1, "colsum: 2-D row-major view")
     M, N = x.shape
@@ -477,9 +490,9 @@ def add2d(a, b, out):
     return out
 
 
-def bce_sigmoid_fwd_bwd(p_raw, y, a=1.0, want_grad=True):
+def bce_sigmoid_fwd_bwd(p_raw, y, a=1.0, want_grad=True, loss=None):
     B, k = p_raw.shape
-    loss = torch.empty(1, dtype=torch.float32, device=p_raw.device)
+    loss = torch.empty(1, dtype=torch.float32, device=p_raw.device) if loss is None else loss
     dz = torch.empty_like(p_raw) if want_grad else None
     call("rs_bce_sigmoid_fwd_bwd", _ptr(p_raw), _dt(p_raw), _ptr(y), a, _ptr(loss), _ptr(dz), B, k, _stream())
     return loss, dz

@@ -321,6 +321,28 @@ class ShardedAutoIntTrainer(AutoIntTrainer):
         """The peer gather, never the local shard with global row numbers."""
         self.buckets.gather(self.ids, self.X)
 
+    def evaluate(self, batches, num_thresholds: int = 200, threshold: float = 0.5) -> dict:
+        """AutoIntTrainer.evaluate over this rank's `batches`, collective: every rank calls it with its own stream (the
+        number of batches, zero included, may differ) and every rank returns the metrics and mean loss of all of them.
+
+        The eval step reads rows straight from the owners' shards (the fused loader over the peer table pointers, or
+        the peer gather) and needs no routing, id exchange or barrier: this rank's last train step ended behind the
+        update barrier (every owner's update of that step is complete), and no owner updates a row again before its
+        next train step's push barrier, which every rank enters only after the eval launches queued before it."""
+        return super().evaluate(batches, num_thresholds, threshold)
+
+    def _eval_reduce(self, ev, totals):
+        """One all-reduce (sum) of every rank's metric state and [loss sum, count].  The integer words travel as
+        float64, exact below 2^53; NCCL hands every rank the same sums, so every rank returns the same dict."""
+        T = ev["metrics"].num_thresholds
+        state = ev["metrics"].state
+        n_int = 2 * T + 4                    # integer words; the last two hold float64 bit patterns
+        buf = torch.cat([state[:n_int].double(), state[n_int:].view(torch.float64), totals])
+        dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=self.ex.group)
+        state[:n_int].copy_(buf[:n_int].to(torch.int64))
+        state[n_int:].view(torch.float64).copy_(buf[n_int:n_int + 2])
+        totals.copy_(buf[n_int + 2:])
+
     def check_overflow(self):
         """Raise if any routing bucket ever exceeded its capacity (ids too skewed for `capacity_factor`)."""
         self.peers.check_overflow()
